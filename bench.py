@@ -30,6 +30,7 @@ host threads; the C oracle port if cv2 is unavailable) on the same workload, met
 Launch: python bench.py --gpus N --steps K --warmup W      (N > 1: under torchrun, one rank per GPU)
 """
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -114,6 +115,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(self.gpu), f"--query-gpu={self.Q}",
                                           "--format=csv,noheader,nounits", "-lms", "10"],
                                          stdout=open(self.path, "w"), stderr=subprocess.DEVNULL)
+            atexit.register(lambda p=self.proc: p.poll() is None and p.kill())     # a run that fails leaves no sampler behind
         except Exception:
             self.proc = None
 
@@ -156,6 +158,29 @@ class ClockSampler:
         if sm:
             out = {"sm_mhz": statistics.median(sm), "sm_max_mhz": max(mx), "reasons": sorted(reasons), "samples": len(sm)}
         return out
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, res, inlier_xy, inlier_offsets):
+    """--dump-outputs: what a caller received from the last timed step, as <name>.npy in float64 (float32 for the points).
+    The per-pair fields come from the headline loop (resident scenes, calls in flight); the inlier scene points and their
+    per-pair offsets from the e2e loop, whose last step ran the same scene batch.  Above DUMP_LIMIT bytes in all, the points
+    are replaced by a fixed sample of their rows (seed 0), whose indices are written as inlier_xy_rows."""
+    arrays = {name: np.ascontiguousarray(res[name], np.float64) for name in res.dtype.names}
+    arrays["inlier_offsets"] = inlier_offsets.astype(np.float64)
+    arrays["inlier_xy"] = np.ascontiguousarray(inlier_xy, np.float32)
+    budget = DUMP_LIMIT - 4096 - sum(a.nbytes for k, a in arrays.items() if k != "inlier_xy")     # 4096: the .npy headers
+    n = len(inlier_xy)
+    if arrays["inlier_xy"].nbytes > budget:
+        keep = budget // (8 + 8)                                 # a sampled row costs its point and its float64 index
+        rows = np.sort(np.random.default_rng(0).choice(n, size=keep, replace=False))
+        arrays["inlier_xy"] = arrays["inlier_xy"][rows]
+        arrays["inlier_xy_rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def bind_to_gpu_numa_node(props):
@@ -500,6 +525,7 @@ def run_cvgraft(args):
 
     # ---- phase 3 (headline `value`): the same thread keeps DEPTH calls in flight (cvg_detect_scenes_submit / cvg_job_wait)
     accepted = 0
+    last = {}                                          # what the last step of a loop handed back to its caller
 
     def loop_pipe(steps):
         nonlocal accepted
@@ -509,7 +535,8 @@ def run_cvgraft(args):
             if len(jobs) > DEPTH - 1:
                 accepted += int((jobs.pop(0).wait()[0]["status"] == 0).sum())
         for j in jobs:
-            accepted += int((j.wait()[0]["status"] == 0).sum())
+            last["pipe"] = j.wait()[0]
+            accepted += int((last["pipe"]["status"] == 0).sum())
 
     tw0 = time.time()                                  # clock samples: from the warm-up on (the timed region is short)
     loop_pipe(max(args.warmup, DEPTH))
@@ -546,6 +573,7 @@ def run_cvgraft(args):
             for sc0, j0 in inflight:
                 res, xy, off = j0.wait(); sc0.free()
                 d2h_seen.append(res.nbytes + xy.nbytes + off.nbytes)
+                last["e2e"] = (res, xy, off)
         return loop
 
     loop_e2e = loop_e2e_with(lambda j: ctx.upload_scenes_async(pinned[j][0], pinned[j][1], pinned[j][2]))
@@ -556,6 +584,8 @@ def run_cvgraft(args):
     d2h = int(statistics.mean(d2h_seen))
     e2e_value = world * B * args.steps / (ms_e2e * 1e-3)
     clocks.mark(tw0, time.time())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["pipe"], *last["e2e"][1:])
     clk = clocks.stop()
 
     # ---- same loop with uint8 descriptor rows in host memory (cv::SIFT can emit CV_8U; SURVEY 8f-3): extra key only
@@ -775,7 +805,11 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the extra keys (e2e_u8, real_dataset): launch-list runs")
     ap.add_argument("--desc", default="sift", choices=["sift", "float"],
                     help="descriptor generator: integer-valued SIFT-like rows (default) or non-integer float rows")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step returned (per-pair results, inlier points) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "cvgraft" else args.warmup
     if args.impl == "reference":
         run_reference(args)

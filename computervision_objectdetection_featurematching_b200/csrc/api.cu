@@ -75,15 +75,6 @@ static cudaError_t h2d_small(cvg_ctx* c, void* dst, const void* src, size_t byte
     return cudaGetLastError();
 }
 
-__global__ void fault_trap_kernel(int* dbg)
-{
-    if (threadIdx.x == 0) { dbg[0] = 99; dbg[1] = (int)blockIdx.x; dbg[2] = 0; }
-    __threadfence_system();
-    __trap();
-}
-
-static int sync_and_check(cvg_ctx* c);
-
 extern "C" {
 
 const char* cvg_last_error(void) { return g_err; }
@@ -269,15 +260,8 @@ int cvg_last_hyp_stats(const cvg_ctx* c0, float* hyp_ms, int* hyp_launches, uint
 int cvg_selftest(cvg_ctx* c0, int which, uint64_t* mismatches)
 {
     cvg_ctx* c = cvg_primary(c0);
-    if (!c || !mismatches || (which != 0 && which != 99)) return set_err(CVG_ERR_INVALID, "cvg_selftest: bad argument");
+    if (!c || !mismatches || which != 0) return set_err(CVG_ERR_INVALID, "cvg_selftest: bad argument");
     CU_CHECK(cudaSetDevice(c->device));
-    if (which == 99) {
-        // fault injection for the tests of the error path: what a protocol bug in a kernel ends in (mbar_wait -> __trap)
-        *mismatches = 0;
-        fault_trap_kernel<<<1, 32, 0, c->stream>>>(c->d_flags + 8);
-        c->launches++;
-        return sync_and_check(c);
-    }
     CU_CHECK(cudaMemsetAsync(c->d_scored, 0, 8, c->stream));
     c->launches += launch_selftest_rcp(c->d_scored, c->stream);
     unsigned long long n = 0;

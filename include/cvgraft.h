@@ -304,7 +304,7 @@ int  cvg_last_score_ms(const cvg_ctx* ctx, float* score_ms);
  * — cudaDeviceReset, which also voids every other CUDA user's state in the process — and cvg_create again.  Whether the
  * driver hands the device back to the SAME process is up to the system: on this pool's B200 boxes it answers "device busy or
  * unavailable" (cvg_device_reset then returns CVG_ERR_CUDA and says so) and the process has to be restarted; a new process
- * gets the GPU at once.  cvg_selftest(ctx, 99, &n) injects such a fault on purpose (tests/test_zz_gpu_fault.py). */
+ * gets the GPU at once. */
 int  cvg_device_reset(int device);
 /* Device self tests.  which = 0: the reciprocal the scoring kernel writes out by hand (MUFU.RCP + one Newton step) against
  * __frcp_rn and against 1.f / x on EVERY float with 2^-126 <= |x| < 2^126; *mismatches must come back 0. */

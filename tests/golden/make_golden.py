@@ -10,6 +10,7 @@ cv2 4.13.0 (opencv-python-headless 4.13.0.92) — in the build container.  The r
 Run:  python tests/golden/make_golden.py          (needs /root/reference/data and cv2)
 Outputs (committed): features_small.npz, golden_pairs.npz, golden_synth.npz, golden_sat.npz
       python tests/golden/make_golden.py sat      (only golden_sat.npz; needs cv2 alone)
+      python tests/golden/make_golden.py rect     (only golden_rect.npz; needs cv2 alone)
 """
 import os
 import sys
@@ -239,6 +240,27 @@ def make_golden_synth():
     np.savez_compressed(path, **out)
     return path
 
+
+def rect_cases():
+    """Point sets of the cv::boundingRect cases (tests/test_host_consumer.py): 500 sets, some of them on integer coordinates."""
+    rng = np.random.default_rng(0)
+    for _ in range(500):
+        p = rng.uniform(-50, 700, size=(int(rng.integers(1, 40)), 2)).astype(np.float32)
+        if rng.random() < 0.3:
+            p = np.round(p)
+        yield p
+
+
+def make_golden_rect():
+    path = os.path.join(HERE, "golden_rect.npz")
+    np.savez_compressed(path, rect=np.array([cv2.boundingRect(p) for p in rect_cases()], np.int32),
+                        cv2_version=np.array(cv2.__version__))
+    return path
+
+
+if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "rect":
+    print(make_golden_rect())
+    sys.exit(0)
 
 if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "sat":
     print(make_golden_sat())

@@ -63,15 +63,16 @@ def py_consume(pts):
 
 
 def test_bounding_rect_matches_cv2(host):
-    cv2 = pytest.importorskip("cv2")
+    """Against cv2.boundingRect of the same point sets (tests/golden/golden_rect.npz, make_golden.py rect_cases)."""
+    want = np.load(os.path.join(ROOT, "tests", "golden", "golden_rect.npz"))["rect"]
     rng = np.random.default_rng(0)
-    for _ in range(500):
+    for k in range(500):
         p = rng.uniform(-50, 700, size=(int(rng.integers(1, 40)), 2)).astype(np.float32)
         if rng.random() < 0.3:
             p = np.round(p)
         out = np.zeros(4, np.int32)
         host.cvh_bounding_rect(_p(p), len(p), _p(out))
-        assert tuple(out) == cv2.boundingRect(p)
+        assert tuple(out) == tuple(want[k]), k
 
 
 def test_cluster_box_merge_filter(host):
