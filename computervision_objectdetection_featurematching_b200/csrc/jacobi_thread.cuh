@@ -3,12 +3,15 @@
 //
 // jacobi_warp.cuh spends ~360 warp instructions per rotation (90 per matrix with four matrices per warp), most of
 // them the rotation's scalar chain replicated across lanes.  Here a thread owns a matrix, so a warp retires 32
-// rotations with ~850 instructions (~27 per matrix).  What made the generic serial routine (homography_math.cuh,
-// jacobi<9,S>) slow is removed: indR/indC live in two registers as packed nibbles (no local memory), every loop has
-// static bounds with predicated bodies (no divergence inside a rotation), the refreshed row/column maxima are taken
-// from the values the rotation has just produced (no re-reads), and the pivot search is a tournament that keeps the
-// serial rule "first maximum wins".  The matrix state is 126 doubles per thread (strict upper triangle of A, V, W)
-// in shared memory, element-major (element e of thread t at e*S + t), so divergent element indices never conflict.
+// rotations with one pass of the rotation loop: 771 SASS instructions (tools/jacobi_sass_digest.py; ~220 of them are
+// the five divisions and two square roots of the c/s chain).  What made the generic serial routine
+// (homography_math.cuh, jacobi<9,S>) slow is removed: indR/indC live in two registers as packed nibbles (no local
+// memory), every loop has static bounds with predicated bodies (no divergence inside a rotation), the two lines of a
+// rotation come from a table of element indices (jt_lines) and need no predicate on any load or store, the refreshed
+// row/column maxima are taken from the values the rotation has just produced (no re-reads), and the pivot search is a
+// tournament that keeps the serial rule "first maximum wins".  The matrix state is 126 doubles per thread (strict
+// upper triangle of A, V, W) plus one spare slot that stays 0, in shared memory, element-major (element e of thread t
+// at e*S + t), so divergent element indices never conflict.
 // Every element sees exactly the arithmetic of the serial code (same operands, same order, no FMA): results are
 // bit-identical to jacobi<9> on finite input.  (With NaN in the matrix the pivot choice may differ, as in
 // jacobi_warp.cuh.)  Compiles for the host too (tests/hostmath).
@@ -20,7 +23,7 @@ namespace cvg {
 constexpr int JT_A = 0;                 // 36 doubles: A[i][j], i < j, at JT_A + tri(i, j)
 constexpr int JT_V = 36;                // 81 doubles: V row-major
 constexpr int JT_W = 117;               //  9 doubles
-constexpr int JT_SPARE = 126;            //  1 double: target of the predicated-off rotations
+constexpr int JT_SPARE = 126;            //  1 double, always 0: the diagonal of jt_lines
 constexpr int JT_DOUBLES = 127;
 
 // first element of row i in the packed strict upper triangle: 0, 8, 15, 21, 26, 30, 33, 35
@@ -28,6 +31,35 @@ CVG_HD constexpr int jt_off(int i) { return i * (17 - i) / 2; }
 // OFFM(i) = jt_off(i) - i - 1: tri(i, j) = OFFM(i) + j for i < j
 CVG_HD constexpr int jt_offm(int i) { return jt_off(i) - i - 1; }
 CVG_HD int jt_offm_dyn(int i) { return i * (17 - i) / 2 - i - 1; }
+
+// Line x of A: jt_lines.e[x][i] = the element index of A(x, i) = A(i, x) for i != x, JT_SPARE for i == x.  A rotation
+// reads its two lines from this table instead of choosing between the row and the column form per element.  The table
+// sits in global memory (432 B, served by L1): lanes of a warp index it with different x, which __constant__ serialises.
+struct alignas(16) JtLines { int e[9][12]; };
+CVG_HD constexpr JtLines jt_make_lines()
+{
+    JtLines t{};
+    for (int x = 0; x < 9; x++)
+        for (int i = 0; i < 9; i++)
+            t.e[x][i] = i == x ? JT_SPARE : JT_A + (i < x ? jt_offm(i) + x : jt_offm(x) + i);
+    return t;
+}
+#if defined(__CUDACC__)
+__device__ const JtLines jt_lines_dev = jt_make_lines();
+#endif
+constexpr JtLines jt_lines_host = jt_make_lines();
+
+CVG_HD void jt_line(int x, int (&e)[9])
+{
+#if defined(__CUDA_ARCH__)
+    const int4* q = reinterpret_cast<const int4*>(jt_lines_dev.e[x]);
+    const int4 a = __ldg(q), b = __ldg(q + 1);
+    e[0] = a.x; e[1] = a.y; e[2] = a.z; e[3] = a.w; e[4] = b.x; e[5] = b.y; e[6] = b.z; e[7] = b.w;
+    e[8] = __ldg(&jt_lines_dev.e[x][8]);
+#else
+    for (int i = 0; i < 9; i++) e[i] = jt_lines_host.e[x][i];
+#endif
+}
 
 CVG_HD int jt_nib(uint32_t r, int i) { return (int)((r >> (4 * i)) & 15u); }
 CVG_HD uint32_t jt_set(uint32_t r, int i, int v) { return (r & ~(15u << (4 * i))) | ((uint32_t)v << (4 * i)); }
@@ -44,8 +76,8 @@ CVG_HD double jt_hypot(double a, double b)
     return hi * sqrt(1 + q * q);
 }
 
-// (val, key) tournament step: the right entry wins only when strictly larger — "first maximum wins"
-#define CVG_JT_PICK(va, ka, vb, kb) do { if ((va) < (vb)) { (va) = (vb); (ka) = (kb); } } while (0)
+// (val, key) tournament step on magnitudes: the right entry wins only when strictly larger — "first maximum wins"
+#define CVG_JT_PICK(va, ka, vb, kb) do { if (fabs(va) < fabs(vb)) { (va) = (vb); (ka) = (kb); } } while (0)
 
 // HomographyEstimatorCallback::runKernel for one 4-point sample, by one thread.  m: this thread's JT_DOUBLES
 // elements with stride S.  `live` = the thread has a sample.  Returns false for "no model".  `any_active` must
@@ -91,6 +123,7 @@ CVG_HD bool run_kernel4_thread(const float* ms1, const float* ms2, double* H, do
         }
         #pragma unroll
         for (int e = 0; e < 81; e++) m[(JT_V + e) * S] = (e / 9 == e % 9) ? 1.0 : 0.0;
+        m[JT_SPARE * S] = 0;
         // ---- initial indR / indC (first maximum wins) ----
         #pragma unroll
         for (int k = 0; k < 8; k++) {
@@ -117,19 +150,20 @@ CVG_HD bool run_kernel4_thread(const float* ms1, const float* ms2, double* H, do
     bool done = !ok;
     for (int iters = 0; iters < 9 * 9 * 30; iters++) {
         int k = 0, l = 1;
-        double p = 0;
+        double p = 0, *pp = m;
         if (!done) {
-            // pivot candidates in the serial scan order: rows 0..7 (k = i, l = indR[i]), then columns 1..8
+            // pivot candidates in the serial scan order: rows 0..7 (k = i, l = indR[i]), then columns 1..8; signed,
+            // so that the winner is the pivot p itself
             double v[16]; int key[16];
             #pragma unroll
             for (int i = 0; i < 8; i++) {
-                v[i] = fabs(m[(JT_A + jt_offm(i) + jt_nib(R, i)) * S]);
+                v[i] = m[(JT_A + jt_offm(i) + jt_nib(R, i)) * S];
                 key[i] = i;
             }
             #pragma unroll
             for (int i = 1; i < 9; i++) {
                 const int ci = jt_nib(C, i - 1);
-                v[7 + i] = fabs(m[(JT_A + jt_offm_dyn(ci) + i) * S]);
+                v[7 + i] = m[(JT_A + jt_offm_dyn(ci) + i) * S];
                 key[7 + i] = 7 + i;
             }
             #pragma unroll
@@ -139,7 +173,8 @@ CVG_HD bool run_kernel4_thread(const float* ms1, const float* ms2, double* H, do
             const int kk = key[0];
             if (kk < 8) { k = kk; l = jt_nib(R, kk); }
             else        { l = kk - 7; k = jt_nib(C, kk - 8); }
-            p = m[(JT_A + jt_offm_dyn(k) + l) * S];
+            pp = m + (JT_A + jt_offm_dyn(k) + l) * S;
+            p = v[0];
             if (fabs(p) <= DBL_EPSILON) done = true;
         }
         if (!any_active(!done)) break;
@@ -151,44 +186,44 @@ CVG_HD bool run_kernel4_thread(const float* ms1, const float* ms2, double* H, do
             const double c = t / s;
             s = p / s; t = (p / t) * p;
             if (y < 0) { s = -s; t = -t; }
-            // element (i, x), i < x, sits at mA[jt_offm(i) * S + x * S]; element (x, i), i > x, at mA[(jt_offm(x) + i) * S]:
-            // with the four bases below every access is base + compile-time offset, chosen by a predicate
-            double* const mA = m + JT_A * S;
-            double* const spare = m + JT_SPARE * S;
-            double* const mk_lt = mA + k * S;                     // + jt_offm(i) * S   for i < k
-            double* const mk_gt = mA + jt_offm_dyn(k) * S;        // + i * S            for i > k
-            double* const ml_lt = mA + l * S;
-            double* const ml_gt = mA + jt_offm_dyn(l) * S;
-            mk_gt[l * S] = 0;
+            // A: element pairs (line of k, line of l) for every index i.  The pairs at i == k and i == l are
+            // (spare, A[k][l]) and (A[k][l], spare): both slots hold 0 and c > 0, so they rotate to +0 and stay 0 — the
+            // serial code's A[k][l] = 0 — with no predicate on any load or store.  Every load comes before every store:
+            // the compiler cannot tell these dynamic addresses apart and would keep a load after an earlier store.
+            int ek[9], el[9];
+            jt_line(k, ek);
+            jt_line(l, el);
+            *pp = 0;
             m[(JT_W + k) * S] = wk - t;
             m[(JT_W + l) * S] = wl + t;
-            // A: element pairs (line of k, line of l) for every other index i; magnitudes kept for the refresh
-            double mvRk = -1, mvCk = -1, mvRl = -1, mvCl = -1;
-            int mRk = 0, mCk = 0, mRl = 0, mCl = 0;
+            double a0[9], b0[9];
+            #pragma unroll
+            for (int i = 0; i < 9; i++) { a0[i] = m[ek[i] * S]; b0[i] = m[el[i] * S]; }
+            // refreshed maxima, serial scans in ascending i: column of idx (i < idx), then row of idx (i > idx).  The
+            // scans keep the signed value and compare magnitudes (the |.| folds into the compare).  A column scan starts
+            // at its first element, i = 0 (unused when idx == 0).  A row scan starts at (0, idx + 1) instead of at its
+            // first element, which is equivalent under "strictly larger wins" and lets it take i == idx, whose value is
+            // 0.  A[k][l] = 0 belongs to row k and to column l, as in the serial code.  Static bounds: k <= 7, l >= 1.
+            double na[9], nb[9];
             #pragma unroll
             for (int i = 0; i < 9; i++) {
-                // branch-free on purpose (one basic block per rotation lets the scheduler overlap the independent
-                // V update with these dependent chains): for i == k and i == l the pair is redirected to the thread's
-                // spare slot, where garbage is rotated and never read back
-                const bool act = (i != k) & (i != l);
-                double* pa = (i < k) ? (mk_lt + jt_offm(i < 8 ? i : 0) * S) : (mk_gt + i * S);
-                double* pb = (i < l) ? (ml_lt + jt_offm(i < 8 ? i : 0) * S) : (ml_gt + i * S);
-                pa = act ? pa : spare; pb = act ? pb : spare;
-                const double a0 = *pa, b0 = *pb;
-                const double na = a0 * c - b0 * s, nb = a0 * s + b0 * c;
-                *pa = na; *pb = nb;
-                // |A| on the line of k resp. l at the other index i; A[k][l] = 0 belongs to row k and to column l;
-                // i == idx is no element (-1 never wins a scan, nor does it need a first-element special case)
-                const double ma = act ? fabs(na) : ((i == l) ? 0.0 : -1.0);
-                const double mb = act ? fabs(nb) : ((i == k) ? 0.0 : -1.0);
-                // serial scans in ascending i: columns (i < idx), then rows (i > idx)
+                na[i] = a0[i] * c - b0[i] * s; nb[i] = a0[i] * s + b0[i] * c;
+                m[ek[i] * S] = na[i];
+                m[el[i] * S] = nb[i];
+            }
+            double mvCk = na[0], mvRk = 0, mvCl = nb[0], mvRl = 0;
+            int mCk = 0, mRk = k + 1, mCl = 0, mRl = l + 1;
+            #pragma unroll
+            for (int i = 1; i < 9; i++) {
                 const bool ck = i < k, cl = i < l;
-                const bool tCk = ck & (mvCk < ma), tRk = (!ck) & (mvRk < ma);
-                const bool tCl = cl & (mvCl < mb), tRl = (!cl) & (mvRl < mb);
-                mvCk = tCk ? ma : mvCk; mCk = tCk ? i : mCk;
-                mvRk = tRk ? ma : mvRk; mRk = tRk ? i : mRk;
-                mvCl = tCl ? mb : mvCl; mCl = tCl ? i : mCl;
-                mvRl = tRl ? mb : mvRl; mRl = tRl ? i : mRl;
+                const bool tCk = i < 7 && ck && fabs(mvCk) < fabs(na[i]);
+                const bool tRk = !ck && fabs(mvRk) < fabs(na[i]);
+                const bool tCl = cl && fabs(mvCl) < fabs(nb[i]);
+                const bool tRl = i > 1 && !cl && fabs(mvRl) < fabs(nb[i]);
+                mvCk = tCk ? na[i] : mvCk; mCk = tCk ? i : mCk;
+                mvRk = tRk ? na[i] : mvRk; mRk = tRk ? i : mRk;
+                mvCl = tCl ? nb[i] : mvCl; mCl = tCl ? i : mCl;
+                mvRl = tRl ? nb[i] : mvRl; mRl = tRl ? i : mRl;
             }
             {
                 double* const vk = m + (JT_V + 9 * k) * S;

@@ -774,7 +774,7 @@ ransac_hyp_g8_kernel(RansacWork w, int round_base)
 }
 
 // One hypothesis per THREAD with the register/predication-friendly Jacobi of jacobi_thread.cuh: the variant for
-// rounds that fill the chip (>= a few thousand hypotheses).  A warp retires 32 rotations with ~850 instructions
+// rounds that fill the chip (>= a few thousand hypotheses).  A warp retires 32 rotations with 771 instructions
 // where the 8-lane-group kernel needs ~2900.  224 threads x 126 doubles of matrix state = 220.5 KB of shared
 // memory, one CTA per SM.  Hypotheses are numbered flat over (set, iteration) so CTAs stay full whatever the
 // round length; lanes of one warp almost always share a set, so the scoring loop's float4 loads are warp-uniform
