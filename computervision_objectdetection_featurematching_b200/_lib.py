@@ -35,6 +35,8 @@ SYMBOLS = {
     "cvg_detect_scenes_submit": (C.c_int, [_P, _P, _P, _P, C.POINTER(DetectParams), _P, _P, _P, C.POINTER(_P)]),
     "cvg_job_wait": (C.c_int, [_P, _P]),
     "cvg_match_knn2_sharded": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_float, _P, _P, _P]),
+    "cvg_find_homography_sharded": (C.c_int, [_P, _P, _P, C.c_int, C.POINTER(RansacParams), _P, _P, C.POINTER(C.c_int), _P, _P]),
+    "cvg_last_exchange": (C.c_int, [_P, C.POINTER(C.c_int), C.POINTER(C.c_float)]),
     "cvg_last_match_guard_rows": (C.c_int, [_P]),
     "cvg_destroy": (None, [_P]),
     "cvg_last_error": (C.c_char_p, []),

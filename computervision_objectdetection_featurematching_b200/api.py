@@ -362,6 +362,31 @@ class Context:
                                                     _ptr(idx), _ptr(dist), _ptr(acc)))
         return idx, dist, acc
 
+    def find_homography_sharded(self, src, dst, threshold=5.0, max_iters=2000, confidence=0.995, flags=0,
+                                want_ransac_mask=False):
+        """find_homography for one point set with the hypotheses of every round split over the GPUs of a multi-device
+        context (one all-gather of inlier counts per round).  -> the dict find_homography_batch returns for one set:
+        H 3x3, mask [n], found (bool), iters (int), and ransac_mask [n] when asked for.  Raises for n < 4 like OpenCV."""
+        s = _f32(src, 2); d = _f32(dst, 2)
+        n = s.shape[0]
+        if d.shape[0] != n:
+            raise ValueError("src and dst must have the same number of points")
+        H = np.zeros(9); mask = np.zeros(max(n, 1), np.uint8); found = C.c_int(0); iters = np.zeros(1, np.int32)
+        rmask = np.zeros(max(n, 1), np.uint8) if want_ransac_mask else None
+        p = ransac_params(threshold, max_iters, confidence, flags)
+        self._check(self.lib.cvg_find_homography_sharded(self.handle, _ptr(s), _ptr(d), n, C.byref(p), _ptr(H), _ptr(mask),
+                                                         C.byref(found), _ptr(iters), _ptr(rmask)))
+        out = {"H": H.reshape(3, 3), "mask": mask[:n], "found": bool(found.value), "iters": int(iters[0])}
+        if want_ransac_mask:
+            out["ransac_mask"] = rmask[:n]
+        return out
+
+    def last_exchange(self):
+        """(exchange steps, their device ms on the first GPU) of the last find_homography_sharded call."""
+        k, t = C.c_int(0), C.c_float(0)
+        self._check(self.lib.cvg_last_exchange(self.handle, C.byref(k), C.byref(t)))
+        return k.value, t.value
+
     # ---- device-pointer building blocks (multi-GPU train-tile shards) ---------------------------
     def dev_match_top2(self, query_ptr, n_query, train_ptr, n_train, index_base, dist_ptr, idx_ptr, stream=None):
         self._check(self.lib.cvg_dev_match_top2(self.handle, stream, query_ptr, n_query, train_ptr, n_train,

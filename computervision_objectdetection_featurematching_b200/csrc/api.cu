@@ -301,7 +301,7 @@ constexpr int NIT_REQ_CAP = 16384;                              // (n, good) pai
 // The raw cv::RNG stream of the fixed seed as a device table.  An accepted 4-point sample costs 4 draws plus the
 // draws of the attempts checkSubset rejected before it (5-8 attempts on outlier-heavy sets), so the table is sized
 // at 48 draws per iteration; a call that still runs out grows it (min_len) and repeats the verify stage.
-static int ensure_rng(cvg_ctx* c, int max_iters, int64_t min_len = 0)
+int ensure_rng(cvg_ctx* c, int max_iters, int64_t min_len)
 {
     int64_t want = std::max<int64_t>(1 << 20, (int64_t)max_iters * 48 + (1 << 16));
     want = std::max(want, min_len);
@@ -528,16 +528,15 @@ __global__ void combine_flags_kernel(int* f, const int* train_flag, int extra_ki
     f[2] = (k & 6) ? 2 : ((k & 1) ? 1 : 0);
 }
 
-// Verify stage on a device correspondence pool.
-static int run_ransac(cvg_ctx* c, const float4* d_pts, const int64_t* d_starts, const int32_t* d_counts_n,
-                      int n_sets, int max_n, int64_t pool_rows, const cvg_ransac_params* p, bool want_rmask)
+// Scratch, flags and parameters of the verify stage on a device correspondence pool, ready for launch_ransac or its phases.
+int eng_ransac_work(cvg_ctx* c, const float4* d_pts, const int64_t* d_starts, const int32_t* d_counts_n, int n_sets,
+                    int max_n, int64_t pool_rows, const cvg_ransac_params* p, bool want_rmask, int counts_slack, RansacWork* out)
 {
-    if (n_sets <= 0) return CVG_OK;
     int rc = ensure_rng(c, p->max_iters);
     if (rc) return rc;
     const int mi = std::max(p->max_iters, 1);
     CU_CHECK(c->sample_pos.ensure((size_t)n_sets * mi * 4));
-    CU_CHECK(c->counts.ensure((size_t)n_sets * mi * 4));
+    CU_CHECK(c->counts.ensure(((size_t)n_sets * mi + counts_slack) * 4));
     static const bool split_score = !(getenv("CVG_FUSED_SCORE") && atoi(getenv("CVG_FUSED_SCORE")));   // A/B: 1 = score inside the solve kernel
     if (split_score) CU_CHECK(c->hypH.ensure((size_t)n_sets * mi * 32));
     CU_CHECK(c->n_samples.ensure((size_t)n_sets * 4));
@@ -603,14 +602,26 @@ static int run_ransac(cvg_ctx* c, const float4* d_pts, const int64_t* d_starts, 
     }
     w.scored_pts = c->timing ? c->d_scored : nullptr;
     if (c->timing) CU_CHECK(cudaMemsetAsync(c->d_scored, 0, 8, c->stream));
+    *out = w;
+    return CVG_OK;
+}
+
+// Verify stage on a device correspondence pool.
+static int run_ransac(cvg_ctx* c, const float4* d_pts, const int64_t* d_starts, const int32_t* d_counts_n,
+                      int n_sets, int max_n, int64_t pool_rows, const cvg_ransac_params* p, bool want_rmask)
+{
+    if (n_sets <= 0) return CVG_OK;
+    RansacWork w;
+    const int rc = eng_ransac_work(c, d_pts, d_starts, d_counts_n, n_sets, max_n, pool_rows, p, want_rmask, 0, &w);
+    if (rc) return rc;
     c->launches += launch_ransac(w, c->stream, c->timing ? c->hyp_ev : nullptr, &c->hyp_rounds);
     CU_CHECK(cudaGetLastError());
     return CVG_OK;
 }
 
-// The device asked about (n, good) pairs (err_flag bit 1): evaluate them with this host's libm — the functions OpenCV itself
-// calls — and put them in the engine's table; the caller then repeats the verify stage.  Stream is idle (caller synchronised).
-static int answer_nit_requests(cvg_ctx* c)
+// The device asked about (n, good) pairs (err_flag bit 1): evaluate the ones `tab` lacks with this host's libm — the
+// functions OpenCV itself calls — and append them.  Stream is idle (caller synchronised).
+int nit_add_requests(cvg_ctx* c, std::vector<NitEntry>& tab, size_t* added_out)
 {
     int n_req = 0;
     CU_CHECK(cudaMemcpy(&n_req, c->d_flags + 19, 4, cudaMemcpyDeviceToHost));
@@ -620,19 +631,37 @@ static int answer_nit_requests(cvg_ctx* c)
     size_t added = 0;
     for (const int2& r : req) {
         bool have = false;
-        for (const NitEntry& e : c->nit_host) if (e.n == r.x && e.good == r.y) { have = true; break; }
+        for (const NitEntry& e : tab) if (e.n == r.x && e.good == r.y) { have = true; break; }
         if (have || r.x <= 0) continue;
         double ep = (double)(r.x - r.y) / r.x;                       // ptsetreg.cpp: (double)(count - goodCount) / count
         ep = ep > 0. ? ep : 0.; ep = ep < 1. ? ep : 1.;
         const double d0 = 1. - pow(1. - ep, 4);                      // modelPoints = 4
         NitEntry e; e.n = r.x; e.good = r.y; e.zero = d0 < DBL_MIN ? 1 : 0; e.denom_log = e.zero ? -1. : log(d0); e.pad = 0;
-        c->nit_host.push_back(e); added++;
+        tab.push_back(e); added++;
     }
+    *added_out = added;
+    return CVG_OK;
+}
+
+// the engine's host table of verified entries to its device copy, read by the next verify stage
+int nit_upload(cvg_ctx* c)
+{
+    if (c->nit_host.empty()) return CVG_OK;
+    CU_CHECK(c->nit.ensure(c->nit_host.size() * sizeof(NitEntry)));
+    CU_CHECK(cudaMemcpyAsync(c->nit.p, c->nit_host.data(), c->nit_host.size() * sizeof(NitEntry), cudaMemcpyHostToDevice, c->stream));
+    CU_CHECK(cudaStreamSynchronize(c->stream));
+    return CVG_OK;
+}
+
+// answer the engine's own requests, then the caller repeats the verify stage
+static int answer_nit_requests(cvg_ctx* c)
+{
+    size_t added = 0;
+    const int rc = nit_add_requests(c, c->nit_host, &added);
+    if (rc) return rc;
     if (!added) return set_err(CVG_ERR_LIMIT, "RANSACUpdateNumIters: the device keeps asking about entries it already has");
     if (c->nit_host.size() > (1u << 20)) return set_err(CVG_ERR_LIMIT, "RANSACUpdateNumIters: verification table overflow");
-    CU_CHECK(c->nit.ensure(c->nit_host.size() * sizeof(NitEntry)));
-    CU_CHECK(cudaMemcpy(c->nit.p, c->nit_host.data(), c->nit_host.size() * sizeof(NitEntry), cudaMemcpyHostToDevice));
-    return CVG_OK;
+    return nit_upload(c);
 }
 
 int check_params(const cvg_ransac_params* p)
@@ -643,7 +672,7 @@ int check_params(const cvg_ransac_params* p)
     return CVG_OK;
 }
 
-static int sync_and_check(cvg_ctx* c)
+int sync_and_check(cvg_ctx* c)
 {
     // The worker thread of a lane that serves a pipelined job sleeps on a blocking-sync event instead of spinning in
     // cudaStreamSynchronize: a context keeps up to 8 jobs in flight, and on a box with 8 GPUs their spinning threads would

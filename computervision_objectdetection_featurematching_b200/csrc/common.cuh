@@ -163,6 +163,15 @@ int launch_selftest_rcp(unsigned long long* d_mismatches, cudaStream_t st);
 // returns the number of kernel launches; hyp_events (optional, 48 events): [2r], [2r+1] bracket the solve kernel of round r,
 // [32 + r] follows its score kernel
 int  launch_ransac(const RansacWork& w, cudaStream_t st, cudaEvent_t* hyp_events = nullptr, int* n_hyp_rounds = nullptr);
+// The phases launch_ransac loops over (the hypothesis-range sharded driver of multi.cu runs them too, with an exchange of
+// the counts between hyp and select).  Each returns its number of kernel launches.
+int  ransac_round_len(const RansacWork& w);                                    // iterations per round on one device
+int  launch_ransac_sample(const RansacWork& w, int rb, int len, cudaStream_t st);   // samples of iterations [rb, rb + len)
+// solve + score iterations [hb, hb + hlen); ev (optional, 3 events): before the solve kernel, after it, after the score
+// kernel; *hyp_complete is cleared when the kernel used does not leave its models in hyp_H
+int  launch_ransac_hyp(const RansacWork& w, int hb, int hlen, cudaStream_t st, const cudaEvent_t* ev, bool* hyp_complete);
+int  launch_ransac_select(const RansacWork& w, int rb, int len, cudaStream_t st);   // serial scan of round [rb, rb + len)
+int  launch_ransac_finish(const RansacWork& w, bool hyp_complete, cudaStream_t st);
 
 // detect glue (ransac.cu)
 struct GateWork {

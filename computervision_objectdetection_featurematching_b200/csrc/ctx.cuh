@@ -229,4 +229,13 @@ int  eng_detect_range(cvg_ctx* c, const cvg_models* m, cvg_scenes* sc, int s0, i
                       std::vector<int32_t>* cnt);
 int  check_detect_params(const cvg_detect_params* p);
 int  check_params(const cvg_ransac_params* p);
+int  sync_and_check(cvg_ctx* c);                        // waits for the engine's stream; names the device on a fault
+// verify stage building blocks (the hypothesis-range sharded driver of multi.cu runs one engine per device through them)
+int  ensure_rng(cvg_ctx* c, int max_iters, int64_t min_len = 0);   // the engine's cv::RNG draw table: >= max_iters * 48 and min_len
+// scratch, flags and parameters of a verify stage over n_sets sets of the pool; counts gets counts_slack extra entries
+int  eng_ransac_work(cvg_ctx* c, const float4* d_pts, const int64_t* d_starts, const int32_t* d_counts_n, int n_sets,
+                     int max_n, int64_t pool_rows, const cvg_ransac_params* p, bool want_rmask, int counts_slack,
+                     cvg::RansacWork* out);
+int  nit_add_requests(cvg_ctx* c, std::vector<cvg::NitEntry>& tab, size_t* added);   // the engine's niters requests into tab
+int  nit_upload(cvg_ctx* c);                            // c->nit_host to the device (stream-ordered, synchronised)
 

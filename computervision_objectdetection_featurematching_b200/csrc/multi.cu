@@ -56,6 +56,10 @@ struct MultiState {
     std::vector<cudaEvent_t> ev;
     unsigned next_dev = 0;
     const char* exchange = "none";
+    // hypothesis-range sharded RANSAC: exchange steps of the last call and their device time on the first GPU; the first
+    // GPU's timing events, five per round (solve start, solve end, score end, exchange start, exchange end)
+    int n_exchanges = 0; float exchange_ms = 0.f;
+    std::vector<cudaEvent_t> tev;
 };
 
 struct ChunkTask { int s0 = 0, s1 = 0; Done done; std::vector<float> pool; std::vector<int32_t> cnt; int match_path = 0; };
@@ -266,6 +270,7 @@ static void multi_destroy(cvg_ctx* c)
         for (std::vector<DevBuf>* v : { &ms->loc_d, &ms->loc_i, &ms->all_d, &ms->all_i, &ms->qbuf, &ms->tbuf, &ms->out_idx, &ms->out_dist, &ms->out_acc })
             if (d < v->size()) (*v)[d].release();
         if (d < ms->ev.size() && ms->ev[d]) cudaEventDestroy(ms->ev[d]);
+        if (d == 0) for (cudaEvent_t e : ms->tev) cudaEventDestroy(e);
         if (ms->subs[d]) { destroy_lanes(ms->subs[d]); eng_destroy(ms->subs[d]); }
     }
     delete ms;
@@ -602,6 +607,269 @@ int cvg_match_knn2_sharded(cvg_ctx* c, const float* query, int n_query, const fl
         CU_CHECK(cudaSetDevice(ms->subs[(size_t)d]->device));
         CU_CHECK(cudaStreamSynchronize(ms->subs[(size_t)d]->stream));
     }
+    return CVG_OK;
+}
+
+// ---- hypothesis-range sharded RANSAC: SURVEY 8e, BASELINE config 5 ------------------------------------------------------
+// Every device holds the whole scan state of the one point set (points, draw table, samples, counts, best so far, adaptive
+// niters) and runs the sampler and the serial select scan itself; only the solve + score kernels are split.  Round
+// [rb, rb + len) is cut into G slices of S = ceil(len / G) iterations, device d solves and scores [rb + d*S, rb +
+// min((d+1)*S, len)), and one exchange per round gives every device all counts of the round: an in-place ncclAllGather of S
+// ints per device, or event-ordered peer copies.  The select kernels then scan exactly the counts one device would have
+// computed, so the winner, the adaptive stop and the niters requests are the same everywhere.  The first device's finish
+// kernel re-solves the winner from its own samples (bit-identical to the hypothesis kernels): no model crosses devices.
+static int sharded_rounds(MultiState* ms, const std::vector<RansacWork>& w, int round_len, bool timing, int* at)
+{
+    const int G = (int)ms->subs.size();
+    const int mi = w[0].max_iters;
+    cvg_ctx* e0 = ms->subs[0];
+    const int n_rounds = (mi + round_len - 1) / round_len;
+    *at = 0;
+    CU_CHECK(cudaSetDevice(e0->device));
+    while (timing && (int)ms->tev.size() < 5 * n_rounds) {
+        cudaEvent_t e;
+        CU_CHECK(cudaEventCreate(&e));
+        ms->tev.push_back(e);
+    }
+    if (timing) CU_CHECK(cudaEventRecord(e0->ev[0], e0->stream));
+    bool hyp_complete = true;                                  // unused: the finish kernel re-solves the winner
+    for (int rb = 0, round = 0; rb < mi; rb += round_len, round++) {
+        const int len = std::min(round_len, mi - rb);
+        const int S = (len + G - 1) / G;
+        const cudaEvent_t* ev = timing ? ms->tev.data() + 5 * round : nullptr;
+        for (int d = 0; d < G; d++) {
+            cvg_ctx* e = ms->subs[(size_t)d];
+            *at = d;
+            CU_CHECK(cudaSetDevice(e->device));
+            e->launches += launch_ransac_sample(w[(size_t)d], rb, len, e->stream);
+            const int a = std::min(d * S, len), b = std::min((d + 1) * S, len);
+            if (b > a) e->launches += launch_ransac_hyp(w[(size_t)d], rb + a, b - a, e->stream, d == 0 ? ev : nullptr, &hyp_complete);
+            CU_CHECK(cudaGetLastError());
+        }
+        // ---- the exchange step: every device receives the round's G*S counts at counts[rb ...) ------------------------
+        if (!ms->comms.empty()) {
+            *at = 0;
+            CU_CHECK(cudaSetDevice(e0->device));
+            if (ev) CU_CHECK(cudaEventRecord(ev[3], e0->stream));
+            NcclApi& na = nccl_api();
+            int r = na.GroupStart();
+            for (int d = 0; d < G && r == 0; d++) {
+                int32_t* cnt = w[(size_t)d].counts + rb;               // in place: rank d sends its own slice
+                r = na.AllGather(cnt + (size_t)d * S, cnt, (size_t)S * 4, NCCL_CHAR, ms->comms[(size_t)d], ms->subs[(size_t)d]->stream);
+            }
+            const int r2 = na.GroupEnd();
+            if (r == 0) r = r2;
+            if (r != 0) return cvg_set_err(CVG_ERR_CUDA, "ncclAllGather failed: %s", na.GetErrorString ? na.GetErrorString(r) : "?");
+            CU_CHECK(cudaSetDevice(e0->device));
+            if (ev) CU_CHECK(cudaEventRecord(ev[4], e0->stream));
+        } else {
+            for (int d = 0; d < G; d++) {
+                *at = d;
+                CU_CHECK(cudaSetDevice(ms->subs[(size_t)d]->device));
+                CU_CHECK(cudaEventRecord(ms->ev[(size_t)d], ms->subs[(size_t)d]->stream));
+            }
+            for (int t = 0; t < G; t++) {
+                cvg_ctx* et = ms->subs[(size_t)t];
+                *at = t;
+                CU_CHECK(cudaSetDevice(et->device));
+                if (ev && t == 0) CU_CHECK(cudaEventRecord(ev[3], et->stream));
+                for (int s = 0; s < G; s++) {
+                    const int a = std::min(s * S, len), b = std::min((s + 1) * S, len);
+                    if (s == t || b <= a) continue;
+                    CU_CHECK(cudaStreamWaitEvent(et->stream, ms->ev[(size_t)s], 0));
+                    CU_CHECK(cudaMemcpyPeerAsync(w[(size_t)t].counts + rb + a, et->device, w[(size_t)s].counts + rb + a,
+                                                 ms->subs[(size_t)s]->device, (size_t)(b - a) * 4, et->stream));
+                }
+                if (ev && t == 0) CU_CHECK(cudaEventRecord(ev[4], et->stream));
+            }
+        }
+        ms->n_exchanges++;
+        for (int d = 0; d < G; d++) {
+            cvg_ctx* e = ms->subs[(size_t)d];
+            *at = d;
+            CU_CHECK(cudaSetDevice(e->device));
+            e->launches += launch_ransac_select(w[(size_t)d], rb, len, e->stream);
+            CU_CHECK(cudaGetLastError());
+        }
+    }
+    *at = 0;
+    CU_CHECK(cudaSetDevice(e0->device));
+    e0->launches += launch_ransac_finish(w[0], false, e0->stream);
+    if (timing) CU_CHECK(cudaEventRecord(e0->ev[1], e0->stream));
+    CU_CHECK(cudaGetLastError());
+    if (timing) {
+        e0->t_hyp = 0; e0->t_score = 0; ms->exchange_ms = 0;
+        for (int r = 0; r < n_rounds; r++) {
+            const cudaEvent_t* ev = ms->tev.data() + 5 * r;
+            float t = 0;
+            CU_CHECK(cudaEventSynchronize(ev[4]));
+            CU_CHECK(cudaEventElapsedTime(&t, ev[0], ev[1])); e0->t_hyp += t;
+            CU_CHECK(cudaEventElapsedTime(&t, ev[1], ev[2])); e0->t_score += t;
+            CU_CHECK(cudaEventElapsedTime(&t, ev[3], ev[4])); ms->exchange_ms += t;
+        }
+        e0->hyp_rounds = n_rounds; e0->hyp_launches = n_rounds;
+    }
+    return CVG_OK;
+}
+
+int cvg_find_homography_sharded(cvg_ctx* c, const float* src_xy, const float* dst_xy, int n, const cvg_ransac_params* p,
+                                double H[9], uint8_t* mask, int* found, int32_t* iters, uint8_t* ransac_mask)
+{
+    if (!c || !c->multi) return cvg_set_err(CVG_ERR_INVALID, "cvg_find_homography_sharded needs a context made by cvg_create_multi");
+    if (n < 4) return cvg_set_err(CVG_ERR_TOO_FEW_POINTS, "findHomography needs at least 4 correspondences (got %d)", n);
+    int rc = check_params(p);
+    if (rc) return rc;
+    if (!src_xy || !dst_xy) return cvg_set_err(CVG_ERR_INVALID, "cvg_find_homography_sharded: bad point arrays");
+    MultiState* ms = c->multi;
+    const int G = (int)ms->subs.size();
+    cvg_ctx* e0 = ms->subs[0];
+    const int mi = std::max(p->max_iters, 1);
+    const bool timing = e0->timing != 0;
+    ms->n_exchanges = 0; ms->exchange_ms = 0.f;
+    int at = 0;                                                // the device the failing step ran on
+    const int64_t start0 = 0; const int32_t n32 = n;
+    std::vector<NitEntry> tab;                                 // the niters entries every device gets
+    std::vector<int32_t> sflags((size_t)G), words((size_t)G);
+    // every device's table to `tab`, where it differs (each engine keeps its entries unique: equal size = same set)
+    auto share_table = [&]() -> int {
+        for (int d = 0; d < G; d++) {
+            cvg_ctx* e = ms->subs[(size_t)d];
+            if (e->nit_host.size() == tab.size()) continue;
+            at = d;
+            CU_CHECK(cudaSetDevice(e->device));
+            e->nit_host = tab;
+            const int r = nit_upload(e);
+            if (r) return r;
+        }
+        return CVG_OK;
+    };
+    rc = [&]() -> int {
+        // points on every device, each device's draw table as long as the longest (the chunked sampler's layout and the
+        // samples follow from the table's length), and one niters table: the union of the devices' tables
+        int64_t rng_len = 0;
+        for (int d = 0; d < G; d++) {
+            cvg_ctx* e = ms->subs[(size_t)d];
+            at = d;
+            CU_CHECK(cudaSetDevice(e->device));
+            CU_CHECK(e->src.ensure((size_t)n * 8)); CU_CHECK(e->dst.ensure((size_t)n * 8)); CU_CHECK(e->pts.ensure((size_t)n * 16));
+            CU_CHECK(e->starts.ensure(8)); CU_CHECK(e->counts_n.ensure(4));
+            CU_CHECK(cudaMemcpyAsync(e->src.p, src_xy, (size_t)n * 8, cudaMemcpyHostToDevice, e->stream));
+            CU_CHECK(cudaMemcpyAsync(e->dst.p, dst_xy, (size_t)n * 8, cudaMemcpyHostToDevice, e->stream));
+            CU_CHECK(cudaMemcpyAsync(e->starts.p, &start0, 8, cudaMemcpyHostToDevice, e->stream));
+            CU_CHECK(cudaMemcpyAsync(e->counts_n.p, &n32, 4, cudaMemcpyHostToDevice, e->stream));
+            launch_pack_points(e->src.as<float>(), e->dst.as<float>(), n, e->pts.as<float4>(), e->stream);
+            e->launches++;
+            int r = ensure_rng(e, mi);
+            if (r) return r;
+            rng_len = std::max(rng_len, e->rng_len);
+            for (const NitEntry& x : e->nit_host) {
+                bool have = false;
+                for (const NitEntry& y : tab) if (x.n == y.n && x.good == y.good) { have = true; break; }
+                if (!have) tab.push_back(x);
+            }
+        }
+        for (int d = 0; d < G; d++) {
+            at = d;
+            CU_CHECK(cudaSetDevice(ms->subs[(size_t)d]->device));
+            const int r = ensure_rng(ms->subs[(size_t)d], mi, rng_len);
+            if (r) return r;
+        }
+        return share_table();
+    }();
+    for (int attempt = 0; rc == CVG_OK; attempt++) {
+        std::vector<RansacWork> w((size_t)G);
+        rc = [&]() -> int {
+            for (int d = 0; d < G; d++) {
+                cvg_ctx* e = ms->subs[(size_t)d];
+                at = d;
+                CU_CHECK(cudaSetDevice(e->device));
+                // counts: the exchange writes G*S <= len + G - 1 entries from rb on
+                const int r = eng_ransac_work(e, e->pts.as<float4>(), e->starts.as<int64_t>(), e->counts_n.as<int32_t>(), 1, n, n, p,
+                                              ransac_mask != nullptr, G, &w[(size_t)d]);
+                if (r) return r;
+            }
+            // adaptive stop: every device's slice of a round is the round one device would run; else one round
+            int round_len = ransac_round_len(w[0]);
+            if (!(p->flags & CVG_RANSAC_NO_EARLY_STOP)) round_len = (int)std::min<int64_t>((int64_t)G * round_len, mi);
+            ms->n_exchanges = 0;
+            int r = sharded_rounds(ms, w, round_len, timing, &at);
+            if (r) return r;
+            at = 0;
+            CU_CHECK(cudaSetDevice(e0->device));
+            if (H) CU_CHECK(cudaMemcpyAsync(H, e0->H.p, 72, cudaMemcpyDeviceToHost, e0->stream));
+            if (mask) CU_CHECK(cudaMemcpyAsync(mask, e0->mask.p, (size_t)n, cudaMemcpyDeviceToHost, e0->stream));
+            if (ransac_mask) CU_CHECK(cudaMemcpyAsync(ransac_mask, e0->rmask.p, (size_t)n, cudaMemcpyDeviceToHost, e0->stream));
+            if (found) CU_CHECK(cudaMemcpyAsync(found, e0->found.p, 4, cudaMemcpyDeviceToHost, e0->stream));
+            if (iters) CU_CHECK(cudaMemcpyAsync(iters, e0->iters_run.p, 4, cudaMemcpyDeviceToHost, e0->stream));
+            for (int d = G - 1; d >= 0; d--) {
+                cvg_ctx* e = ms->subs[(size_t)d];
+                at = d;
+                CU_CHECK(cudaSetDevice(e->device));
+                CU_CHECK(cudaMemcpyAsync(&sflags[(size_t)d], e->sflags.p, 4, cudaMemcpyDeviceToHost, e->stream));
+                CU_CHECK(cudaMemcpyAsync(&words[(size_t)d], e->d_flags + 4, 4, cudaMemcpyDeviceToHost, e->stream));
+                r = sync_and_check(e);
+                if (r) return r;
+            }
+            return CVG_OK;
+        }();
+        if (rc) break;
+        // retry decisions on the union of the devices' flags
+        bool short_tab = false; int want_nit = 0;
+        for (int d = 0; d < G; d++) { short_tab = short_tab || (sflags[(size_t)d] & 1); want_nit |= words[(size_t)d] & 2; }
+        if (!short_tab && want_nit) {                          // niters entries to verify on the host, then again
+            if (attempt >= 12) return cvg_set_err(CVG_ERR_LIMIT, "RANSACUpdateNumIters verification did not converge");
+            size_t added = 0;
+            rc = [&]() -> int {
+                for (int d = 0; d < G; d++) {
+                    if (!(words[(size_t)d] & 2)) continue;
+                    at = d;
+                    CU_CHECK(cudaSetDevice(ms->subs[(size_t)d]->device));
+                    size_t a = 0;
+                    const int r = nit_add_requests(ms->subs[(size_t)d], tab, &a);
+                    if (r) return r;
+                    added += a;
+                }
+                if (!added) return cvg_set_err(CVG_ERR_LIMIT, "RANSACUpdateNumIters: the device keeps asking about entries it already has");
+                if (tab.size() > (1u << 20)) return cvg_set_err(CVG_ERR_LIMIT, "RANSACUpdateNumIters: verification table overflow");
+                return share_table();
+            }();
+            continue;
+        }
+        if (!short_tab) break;
+        // a draw table ran out: every device's table grows to the same length, then the whole verify stage again
+        const int64_t old_len = e0->rng_len;
+        if (attempt >= 4) return cvg_set_err(CVG_ERR_LIMIT, "RNG draw table exhausted (pathological rejection rate)");
+        rc = [&]() -> int {
+            for (int d = 0; d < G; d++) {
+                at = d;
+                CU_CHECK(cudaSetDevice(ms->subs[(size_t)d]->device));
+                const int r = ensure_rng(ms->subs[(size_t)d], mi, old_len * 4);
+                if (r) return r;
+            }
+            return CVG_OK;
+        }();
+        if (rc == CVG_OK && e0->rng_len == old_len)            // at the size cap already
+            return cvg_set_err(CVG_ERR_LIMIT, "RNG draw table exhausted (pathological rejection rate)");
+    }
+    if (rc) {
+        const std::string msg = cvg_last_error();
+        for (cvg_ctx* e : ms->subs) { cudaSetDevice(e->device); cudaStreamSynchronize(e->stream); }
+        return cvg_set_err(rc, "cvg_find_homography_sharded, device %d: %s", ms->devices[(size_t)at], msg.c_str());
+    }
+    if (timing) {
+        cudaSetDevice(e0->device);
+        cudaEventElapsedTime(&e0->t_ransac, e0->ev[0], e0->ev[1]);
+        e0->t_match = 0; e0->t_total = e0->t_ransac;
+        cudaMemcpy(&e0->scored_pts, e0->d_scored, 8, cudaMemcpyDeviceToHost);   // the first GPU's share
+    }
+    return CVG_OK;
+}
+
+int cvg_last_exchange(const cvg_ctx* c, int* n_exchanges, float* exchange_ms)
+{
+    if (!c) return cvg_set_err(CVG_ERR_INVALID, "cvg_last_exchange: NULL context");
+    if (n_exchanges) *n_exchanges = c->multi ? c->multi->n_exchanges : 0;
+    if (exchange_ms) *exchange_ms = c->multi ? c->multi->exchange_ms : 0.f;
     return CVG_OK;
 }
 

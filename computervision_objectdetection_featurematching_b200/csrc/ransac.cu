@@ -1564,17 +1564,12 @@ int ransac_set_device_attrs(char* err, size_t errlen)
     return 0;
 }
 
-int launch_ransac(const RansacWork& w, cudaStream_t st, cudaEvent_t* hyp_events, int* n_hyp_rounds)
+int ransac_round_len(const RansacWork& w)
 {
-    if (n_hyp_rounds) *n_hyp_rounds = 0;
-    if (w.n_sets <= 0) return 0;
-    int launches = 1;
-
     // Hypotheses are solved and scored in rounds; after each round the serial selection scan advances, so rounds
     // beyond the adaptive stop (RANSACUpdateNumIters) cost one early exit per warp.  A round is a latency-bound
     // launch (~135 dependent rotations per matrix whatever the kernel), so it is made long enough to fill the chip:
     // at least 256 iterations per set, and n_sets x round_len >= one full wave of the thread-per-hypothesis kernel.
-    static const int hyp_mode = getenv("CVG_HYP_MODE") ? atoi(getenv("CVG_HYP_MODE")) : 0;   // experiments: 1 warp, 2 g8, 3 thread (generic), 4 thread
     static const int round_env = getenv("CVG_ROUND_LEN") ? atoi(getenv("CVG_ROUND_LEN")) : 0;
     const int n_sms = w.n_sms > 0 ? w.n_sms : 148;
     int round_len = w.max_iters;
@@ -1593,65 +1588,81 @@ int launch_ransac(const RansacWork& w, cudaStream_t st, cudaEvent_t* hyp_events,
         round_len = (int)std::min<int64_t>(std::max<int64_t>(256, fill), w.max_iters);
         if (round_env > 0) round_len = std::min(round_env, w.max_iters);
     }
-    const int warps_per_block = 4;
-    int round = 0;
-    bool hyp_complete = w.hyp_H != nullptr;
-    for (int rb = 0; rb < w.max_iters; rb += round_len, round++) {
-        const int len = w.max_iters - rb < round_len ? w.max_iters - rb : round_len;
-        if (rb == 0 && w.chunk_outs && w.n_chunks > 1 && (int64_t)len >= CHUNKED_MIN_ITERS) {
-            // a huge single round (the no-early-stop throughput mode): cut every set's draw stream into chunks
-            ChunkOut* outs = static_cast<ChunkOut*>(w.chunk_outs);
-            ransac_sample_map_kernel<<<dim3((unsigned)w.n_chunks, (unsigned)w.n_sets), SMP_THREADS, 0, st>>>(w, rb, w.n_chunks, w.chunk_maps);
-            ransac_sample_entry_kernel<<<w.n_sets, 256, 0, st>>>(w.n_chunks, w.chunk_maps, w.chunk_entries);
-            ransac_sample_chunk_kernel<<<dim3((unsigned)w.n_chunks, (unsigned)w.n_sets), SMP_THREADS, 0, st>>>(w, rb, w.n_chunks, w.chunk_entries,
-                                                                                                              outs, w.chunk_lists);
-            ransac_sample_stitch_kernel<<<(w.n_sets + 63) / 64, 64, 0, st>>>(w, rb, rb + len, w.n_chunks, outs, w.chunk_lists,
-                                                                            w.chunk_offsets, w.chunk_serial);
-            ransac_sample_scatter_kernel<<<dim3((unsigned)w.n_chunks, (unsigned)w.n_sets), 256, 0, st>>>(w, rb + len, w.n_chunks, outs,
-                                                                                                     w.chunk_lists, w.chunk_offsets);
-            ransac_sample_kernel<<<w.n_sets, SMP_THREADS, 0, st>>>(w, rb, rb + len, w.chunk_serial);   // sets the stitch rejected
-            launches += 5;
-        } else
-            ransac_sample_kernel<<<w.n_sets, SMP_THREADS, 0, st>>>(w, rb, rb + len, nullptr);
-        const bool timed = hyp_events != nullptr && round < 16;
-        if (timed) cudaEventRecord(hyp_events[2 * round], st);
-        // Measured on B200 (round 1).  13 350 real pairs (3.4 M hypotheses per round), whole verify stage: generic
-        // thread-per-hypothesis 612 ms, warp-per-hypothesis 1436 ms, four-per-warp 498 ms.  64 synthetic 8k x 8k pairs
-        // (16 384 hypotheses per round), hypothesis kernels per step: warp 4.15 ms, four-per-warp 2.41 ms.
-        // One set alone (256 hypotheses): warp 0.30 ms, generic thread 1.1 ms.
-        const int64_t hyps = (int64_t)len * w.n_sets;
-        const int mode = hyp_mode ? hyp_mode : (hyps <= 4096 ? 1 : 4);
-        if (mode == 2 || mode == 3) hyp_complete = false;      // the A/B kernels do not leave their models in hyp_H
-        if (mode == 1) {                                       // a handful of hypotheses: latency of one matrix counts
-            dim3 grid((len + HYPW_WARPS - 1) / HYPW_WARPS, w.n_sets);
-            ransac_hyp_warp_kernel<<<grid, HYPW_WARPS * 32, 0, st>>>(w, rb);
-        } else if (mode == 2) {                                // four matrices per warp
-            dim3 grid((len + HYPG_WARPS * 4 - 1) / (HYPG_WARPS * 4), w.n_sets);
-            ransac_hyp_g8_kernel<<<grid, HYPG_WARPS * 32, HYPG_SMEM, st>>>(w, rb);
-        } else if (mode == 3) {                                // generic serial routine, one thread per hypothesis
-            dim3 grid((len + HYP_THREADS - 1) / HYP_THREADS, w.n_sets);
-            ransac_hyp_kernel<<<grid, HYP_THREADS, HYP_SMEM, st>>>(w, rb);
-        } else {                                               // the chip is full: one thread per hypothesis
-            const int64_t blocks = (hyps + HYPT_THREADS - 1) / HYPT_THREADS;
-            ransac_hyp_t_kernel<<<(unsigned)blocks, HYPT_THREADS, HYPT_SMEM, st>>>(w, rb, len);
-        }
-        if (timed) { cudaEventRecord(hyp_events[2 * round + 1], st); *n_hyp_rounds = round + 1; }
-        if (mode == 4 && w.hyp_H) {
-            // slices of the correspondences so that the launch holds >= ~6 CTAs per SM (or one slice per 512 points)
-            const int tiles = (len + SCORE_THREADS - 1) / SCORE_THREADS;
-            const int64_t ctas = (int64_t)tiles * w.n_sets;
-            int n_slices = (int)std::min<int64_t>(std::max<int64_t>(1, ((int64_t)n_sms * 6 + ctas - 1) / ctas), std::max(1, w.max_n / 512));
-            n_slices = std::max(1, std::min(n_slices, 64));
-            ransac_score_kernel<<<dim3((unsigned)ctas, 1, (unsigned)n_slices), SCORE_THREADS, 0, st>>>(w, rb, len, n_slices, tiles);
-            launches += 1;
-        }
-        if (timed) cudaEventRecord(hyp_events[32 + round], st);
-        if (w.flags & CVG_RANSAC_NO_EARLY_STOP)
-            ransac_select_all_kernel<<<w.n_sets, SELP_THREADS, 0, st>>>(w, rb, len);
-        else
-            ransac_select_kernel<<<(w.n_sets + warps_per_block - 1) / warps_per_block, warps_per_block * 32, 0, st>>>(w, rb, len);
-        launches += 3;
+    return round_len;
+}
+
+int launch_ransac_sample(const RansacWork& w, int rb, int len, cudaStream_t st)
+{
+    if (rb == 0 && w.chunk_outs && w.n_chunks > 1 && (int64_t)len >= CHUNKED_MIN_ITERS) {
+        // a huge single round (the no-early-stop throughput mode): cut every set's draw stream into chunks
+        ChunkOut* outs = static_cast<ChunkOut*>(w.chunk_outs);
+        ransac_sample_map_kernel<<<dim3((unsigned)w.n_chunks, (unsigned)w.n_sets), SMP_THREADS, 0, st>>>(w, rb, w.n_chunks, w.chunk_maps);
+        ransac_sample_entry_kernel<<<w.n_sets, 256, 0, st>>>(w.n_chunks, w.chunk_maps, w.chunk_entries);
+        ransac_sample_chunk_kernel<<<dim3((unsigned)w.n_chunks, (unsigned)w.n_sets), SMP_THREADS, 0, st>>>(w, rb, w.n_chunks, w.chunk_entries,
+                                                                                                          outs, w.chunk_lists);
+        ransac_sample_stitch_kernel<<<(w.n_sets + 63) / 64, 64, 0, st>>>(w, rb, rb + len, w.n_chunks, outs, w.chunk_lists,
+                                                                        w.chunk_offsets, w.chunk_serial);
+        ransac_sample_scatter_kernel<<<dim3((unsigned)w.n_chunks, (unsigned)w.n_sets), 256, 0, st>>>(w, rb + len, w.n_chunks, outs,
+                                                                                                 w.chunk_lists, w.chunk_offsets);
+        ransac_sample_kernel<<<w.n_sets, SMP_THREADS, 0, st>>>(w, rb, rb + len, w.chunk_serial);   // sets the stitch rejected
+        return 6;
     }
+    ransac_sample_kernel<<<w.n_sets, SMP_THREADS, 0, st>>>(w, rb, rb + len, nullptr);
+    return 1;
+}
+
+int launch_ransac_hyp(const RansacWork& w, int hb, int hlen, cudaStream_t st, const cudaEvent_t* ev, bool* hyp_complete)
+{
+    static const int hyp_mode = getenv("CVG_HYP_MODE") ? atoi(getenv("CVG_HYP_MODE")) : 0;   // experiments: 1 warp, 2 g8, 3 thread (generic), 4 thread
+    const int n_sms = w.n_sms > 0 ? w.n_sms : 148;
+    int launches = 1;
+    if (ev) cudaEventRecord(ev[0], st);
+    // Measured on B200 (round 1).  13 350 real pairs (3.4 M hypotheses per round), whole verify stage: generic
+    // thread-per-hypothesis 612 ms, warp-per-hypothesis 1436 ms, four-per-warp 498 ms.  64 synthetic 8k x 8k pairs
+    // (16 384 hypotheses per round), hypothesis kernels per step: warp 4.15 ms, four-per-warp 2.41 ms.
+    // One set alone (256 hypotheses): warp 0.30 ms, generic thread 1.1 ms.
+    const int64_t hyps = (int64_t)hlen * w.n_sets;
+    const int mode = hyp_mode ? hyp_mode : (hyps <= 4096 ? 1 : 4);
+    if (mode == 2 || mode == 3) *hyp_complete = false;     // the A/B kernels do not leave their models in hyp_H
+    if (mode == 1) {                                       // a handful of hypotheses: latency of one matrix counts
+        dim3 grid((hlen + HYPW_WARPS - 1) / HYPW_WARPS, w.n_sets);
+        ransac_hyp_warp_kernel<<<grid, HYPW_WARPS * 32, 0, st>>>(w, hb);
+    } else if (mode == 2) {                                // four matrices per warp
+        dim3 grid((hlen + HYPG_WARPS * 4 - 1) / (HYPG_WARPS * 4), w.n_sets);
+        ransac_hyp_g8_kernel<<<grid, HYPG_WARPS * 32, HYPG_SMEM, st>>>(w, hb);
+    } else if (mode == 3) {                                // generic serial routine, one thread per hypothesis
+        dim3 grid((hlen + HYP_THREADS - 1) / HYP_THREADS, w.n_sets);
+        ransac_hyp_kernel<<<grid, HYP_THREADS, HYP_SMEM, st>>>(w, hb);
+    } else {                                               // the chip is full: one thread per hypothesis
+        const int64_t blocks = (hyps + HYPT_THREADS - 1) / HYPT_THREADS;
+        ransac_hyp_t_kernel<<<(unsigned)blocks, HYPT_THREADS, HYPT_SMEM, st>>>(w, hb, hlen);
+    }
+    if (ev) cudaEventRecord(ev[1], st);
+    if (mode == 4 && w.hyp_H) {
+        // slices of the correspondences so that the launch holds >= ~6 CTAs per SM (or one slice per 512 points)
+        const int tiles = (hlen + SCORE_THREADS - 1) / SCORE_THREADS;
+        const int64_t ctas = (int64_t)tiles * w.n_sets;
+        int n_slices = (int)std::min<int64_t>(std::max<int64_t>(1, ((int64_t)n_sms * 6 + ctas - 1) / ctas), std::max(1, w.max_n / 512));
+        n_slices = std::max(1, std::min(n_slices, 64));
+        ransac_score_kernel<<<dim3((unsigned)ctas, 1, (unsigned)n_slices), SCORE_THREADS, 0, st>>>(w, hb, hlen, n_slices, tiles);
+        launches += 1;
+    }
+    if (ev) cudaEventRecord(ev[2], st);
+    return launches;
+}
+
+int launch_ransac_select(const RansacWork& w, int rb, int len, cudaStream_t st)
+{
+    const int warps_per_block = 4;
+    if (w.flags & CVG_RANSAC_NO_EARLY_STOP)
+        ransac_select_all_kernel<<<w.n_sets, SELP_THREADS, 0, st>>>(w, rb, len);
+    else
+        ransac_select_kernel<<<(w.n_sets + warps_per_block - 1) / warps_per_block, warps_per_block * 32, 0, st>>>(w, rb, len);
+    return 1;
+}
+
+int launch_ransac_finish(const RansacWork& w, bool hyp_complete, cudaStream_t st)
+{
     // Sets of a few dozen correspondences (the real dataset: 445 sets per call, n <= 127) take the exact path, which is
     // warp 0's serial eigen-solves plus 56 single-thread sums: with 64 threads per CTA four CTAs fit an SM (206 registers)
     // and the call's sets run in one wave instead of two.  Every loop of the kernel strides by blockDim.x.
@@ -1659,6 +1670,27 @@ int launch_ransac(const RansacWork& w, cudaStream_t st, cudaEvent_t* hyp_events,
     RansacWork wf = w;
     wf.hyp_H_complete = hyp_complete ? 1 : 0;
     ransac_finish_kernel<<<w.n_sets, finish_threads, 0, st>>>(wf);
+    return 1;
+}
+
+int launch_ransac(const RansacWork& w, cudaStream_t st, cudaEvent_t* hyp_events, int* n_hyp_rounds)
+{
+    if (n_hyp_rounds) *n_hyp_rounds = 0;
+    if (w.n_sets <= 0) return 0;
+    const int round_len = ransac_round_len(w);
+    int launches = 0, round = 0;
+    bool hyp_complete = w.hyp_H != nullptr;
+    for (int rb = 0; rb < w.max_iters; rb += round_len, round++) {
+        const int len = w.max_iters - rb < round_len ? w.max_iters - rb : round_len;
+        launches += launch_ransac_sample(w, rb, len, st);
+        const bool timed = hyp_events != nullptr && round < 16;
+        const cudaEvent_t ev[3] = { timed ? hyp_events[2 * round] : nullptr, timed ? hyp_events[2 * round + 1] : nullptr,
+                                    timed ? hyp_events[32 + round] : nullptr };
+        launches += launch_ransac_hyp(w, rb, len, st, timed ? ev : nullptr, &hyp_complete);
+        if (timed) *n_hyp_rounds = round + 1;
+        launches += launch_ransac_select(w, rb, len, st);
+    }
+    launches += launch_ransac_finish(w, hyp_complete, st);
     return launches;
 }
 

@@ -117,8 +117,10 @@ int  cvg_create(cvg_ctx** out, int device, unsigned flags);
  * scenes to the GPUs by cost (batches of fewer than 2 x n_devices scenes stay whole and take the GPUs in turn);
  * cvg_detect_scenes* / _submit run every device's share concurrently and return results in the caller's order —
  * pair sharding of the loop nest of src/TestsDetector.cpp:38,58,99 under src/Output.cpp:23-57, no data-path
- * collective; cvg_match_knn2_sharded is the train-tile sharded match with its one all-gather.  The other entry
- * points (cvg_match_knn2, cvg_find_homography, cvg_detect_pairs, cvg_dev_*) run on the first listed GPU.
+ * collective; cvg_match_knn2_sharded is the train-tile sharded match with its one all-gather, and
+ * cvg_find_homography_sharded splits the hypotheses of one RANSAC over the GPUs with one all-gather of counts per
+ * round.  The other entry points (cvg_match_knn2, cvg_find_homography, cvg_find_homography_batch, cvg_detect_pairs,
+ * cvg_dev_*) run on the first listed GPU.
  * A device may be listed more than once (logical shards on one GPU, used by the single-GPU tests); NCCL refuses
  * such a communicator, so the exchange then runs as device-to-device copies (cvg_exchange_kind: "memcpy"). */
 int  cvg_create_multi(cvg_ctx** out, const int* devices, int n_devices, unsigned flags);
@@ -245,6 +247,24 @@ int  cvg_job_wait(cvg_ctx* ctx, cvg_job* job);
  * any number of shards.  Same outputs as cvg_match_knn2_raw; replaces src/TestsDetector.cpp:59-72. */
 int  cvg_match_knn2_sharded(cvg_ctx* ctx, const float* query, int n_query, const float* train, int n_train,
                             float ratio, int32_t* idx, float* dist, uint8_t* accept);
+
+/* findHomography(src, dst, RANSAC, p->threshold, mask, p->max_iters, p->confidence) for ONE point set, with the
+ * hypotheses of every round split over the GPUs of a cvg_create_multi context.  Outputs are those of
+ * cvg_find_homography_batch for a single set, bit for bit, for any parameters and flags (adaptive stop included).
+ * Every GPU samples the whole round and runs the serial selection scan itself; GPU g solves and scores iterations
+ * [g*S, (g+1)*S) of each round (S = ceil(round length / n_devices)), then one all-gather of the round's inlier counts,
+ * 4 B per hypothesis, gives every GPU all of them.  Rounds: one of max_iters with CVG_RANSAC_NO_EARLY_STOP, else
+ * n_devices times the round one GPU would run.  The first GPU refines the winner.  iters / ransac_mask may be NULL.
+ * n < 4 -> CVG_ERR_TOO_FEW_POINTS; a context made by cvg_create -> CVG_ERR_INVALID (cvg_create_multi with one
+ * device is valid and runs the whole range on it).  With timing on, cvg_last_timing / cvg_last_hyp_stats /
+ * cvg_last_score_ms report the first GPU's verify stage, solve and score kernels (scored points: its share). */
+int  cvg_find_homography_sharded(cvg_ctx* ctx, const float* src_xy, const float* dst_xy, int n,
+                                 const cvg_ransac_params* p, double H[9], uint8_t* mask, int* found,
+                                 int32_t* iters, uint8_t* ransac_mask);
+/* The last sharded verify call on this context: how many exchange steps it ran (one per round), and their summed
+ * device time on the first GPU in ms (0 unless cvg_set_timing is on; it includes waiting for the slowest GPU's
+ * slice).  Both are 0 before the first such call. */
+int  cvg_last_exchange(const cvg_ctx* ctx, int* n_exchanges, float* exchange_ms);
 
 /* ---- device-pointer building blocks (multi-GPU train-tile sharding, BASELINE config 5) --------
  * All pointers are DEVICE memory of the context's GPU; `stream` is a cudaStream_t (NULL = default).
