@@ -260,10 +260,11 @@ int cvg_last_hyp_stats(const cvg_ctx* c0, float* hyp_ms, int* hyp_launches, uint
 int cvg_selftest(cvg_ctx* c0, int which, uint64_t* mismatches)
 {
     cvg_ctx* c = cvg_primary(c0);
-    if (!c || !mismatches || which != 0) return set_err(CVG_ERR_INVALID, "cvg_selftest: bad argument");
+    if (!c || !mismatches || which < 0 || which > 1) return set_err(CVG_ERR_INVALID, "cvg_selftest: bad argument");
     CU_CHECK(cudaSetDevice(c->device));
     CU_CHECK(cudaMemsetAsync(c->d_scored, 0, 8, c->stream));
-    c->launches += launch_selftest_rcp(c->d_scored, c->stream);
+    c->launches += which == 0 ? launch_selftest_rcp(c->d_scored, c->stream)
+                              : launch_selftest_jacobi(c->d_scored, 5 * 2048, c->stream);
     unsigned long long n = 0;
     CU_CHECK(cudaMemcpyAsync(&n, c->d_scored, 8, cudaMemcpyDeviceToHost, c->stream));
     CU_CHECK(cudaStreamSynchronize(c->stream));

@@ -160,6 +160,7 @@ int64_t ransac_chunk_scratch_bytes(int n_sets, int n_chunks, size_t* outs, size_
                                    size_t* maps, size_t* entries);
 int ransac_chunks_for_table(int64_t rng_len);
 int launch_selftest_rcp(unsigned long long* d_mismatches, cudaStream_t st);
+int launch_selftest_jacobi(unsigned long long* d_mismatches, int n_mats, cudaStream_t st);
 // returns the number of kernel launches; hyp_events (optional, 48 events): [2r], [2r+1] bracket the solve kernel of round r,
 // [32 + r] follows its score kernel
 int  launch_ransac(const RansacWork& w, cudaStream_t st, cudaEvent_t* hyp_events = nullptr, int* n_hyp_rounds = nullptr);

@@ -2,9 +2,10 @@
 //
 // cv::eigen's Jacobi (SURVEY App. D.2) is a serial chain of ~135 rotations per 9x9 matrix; a single
 // thread spends ~6000 cycles per rotation on dependent shared-memory accesses.  Here one warp runs one
-// matrix: the pivot search is a 16-lane argmax, the 16 element-pair rotations and the four indR/indC
-// refreshes run one per lane (group), and only the rotation's scalar chain (two hypot, three divisions)
-// stays serial.  Every element sees exactly the arithmetic of the serial code (same operands, same
+// matrix: the 16 element-pairs of a rotation are rotated one per lane, the pivot search and the four
+// indR/indC refreshes run redundantly in every lane as register tournaments over broadcast loads, and
+// the rotation's scalar chain (two hypot, three divisions) is the only serial part.  Every element sees
+// exactly the arithmetic of the serial code (same operands, same
 // order, no FMA), and every argmax keeps the serial rule "first maximum wins", so results are
 // bit-identical to jacobi<9>.  All 32 lanes must call; A, W, V live in warp-private shared memory.
 // (Matrices containing NaN may pick different pivots than the serial scan; finite data cannot.)
@@ -28,63 +29,104 @@ __device__ __forceinline__ double shfl_xor_d(double v, int m)
     return __hiloint2double(hi, lo);
 }
 
-// argmax over the lanes of a group of `width` lanes (power of two, aligned): largest val, ties -> smallest
-// key.  Lanes that do not take part pass val = -1 (all real candidates are >= 0).  Result valid in every
-// lane of the group.
-template <int WIDTH>
-__device__ __forceinline__ void group_argmax_first(double& val, int& key)
+// (Measured and rejected, against the earlier 16-lane shuffle argmax of the pivot: two redux.sync integer maxima over the
+// hi / lo words of the non-negative doubles plus a ballot instead of the shuffle rounds — verify stage 2.65 -> 3.14 ms per
+// 64 pairs, real dataset 365 -> 399 ms.)
+
+// One step of a "first maximum wins" tournament: (v1, i1) comes later in the serial scan order than (v0, i0) and wins only
+// if it is strictly larger, as `if (mv < val)` does.  A tree of these over candidates in scan order picks the serial scan's
+// answer (for finite values).
+__device__ __forceinline__ void later_wins_if_larger(double& v0, int& i0, double v1, int i1)
 {
-    #pragma unroll
-    for (int m = WIDTH / 2; m > 0; m >>= 1) {
-        const double ov = shfl_xor_d(val, m);
-        const int ok = __shfl_xor_sync(0xffffffffu, key, m);
-        if (ov > val || (ov == val && ok < key)) { val = ov; key = ok; }
-    }
+    const bool take = v0 < v1;
+    v0 = take ? v1 : v0;
+    i0 = take ? i1 : i0;
 }
 
-// (Measured and rejected: the same argmax with two redux.sync integer maxima over the hi / lo words of the non-negative
-// doubles plus a ballot instead of the shuffle rounds — verify stage 2.65 -> 3.14 ms per 64 pairs, real dataset 365 -> 399 ms.)
+// Serial row scan of jacobi<9> (indR[idx], idx < 8): argmax of |A[idx][i]| over i = idx+1 .. 8, first maximum wins.  Reads
+// all of row idx (in bounds for any idx <= 8) and disqualifies i <= idx with -1, which loses to every real candidate.
+__device__ __forceinline__ int row_argmax9(const double* A, int idx)
+{
+    double v[8]; int m[8];
+    #pragma unroll
+    for (int i = 1; i < 9; i++) { const double a = fabs(A[9 * idx + i]); v[i - 1] = i > idx ? a : -1.0; m[i - 1] = i; }
+    #pragma unroll
+    for (int w = 1; w < 8; w *= 2)
+        #pragma unroll
+        for (int q = 0; q < 8; q += 2 * w) later_wins_if_larger(v[q], m[q], v[q + w], m[q + w]);
+    return m[0];
+}
+
+// Serial column scan of jacobi<9> (indC[idx], idx >= 1): argmax of |A[i][idx]| over i = 0 .. idx-1, first maximum wins.
+// The disqualified i >= idx come last in the order, so -1 never wins there either.
+__device__ __forceinline__ int col_argmax9(const double* A, int idx)
+{
+    double v[8]; int m[8];
+    #pragma unroll
+    for (int i = 0; i < 8; i++) { const double a = fabs(A[9 * i + idx]); v[i] = i < idx ? a : -1.0; m[i] = i; }
+    #pragma unroll
+    for (int w = 1; w < 8; w *= 2)
+        #pragma unroll
+        for (int q = 0; q < 8; q += 2 * w) later_wins_if_larger(v[q], m[q], v[q + w], m[q + w]);
+    return m[0];
+}
+
+// cv_hypot without branches: the larger magnitude divides the smaller, as in whichever branch cv_hypot takes, so the result
+// is the same double.  Both magnitudes zero: the quotient is NaN and is not selected.
+__device__ __forceinline__ double cv_hypot_sel(double a, double b)
+{
+    a = fabs(a); b = fabs(b);
+    const bool a_big = a > b;
+    const double hi = a_big ? a : b, lo = a_big ? b : a;
+    const double r = lo / hi;
+    const double h = hi * sqrt(1 + r * r);
+    return hi > 0 ? h : 0.0;
+}
+
 // A: 81 doubles (upper triangle significant, destroyed), W: 9, V: 81 — all in shared memory.
-__device__ __noinline__ void jacobi9_warp(double* A, double* W, double* V)
+// Every lane runs the pivot search and the four refreshed scans itself, on broadcast loads of the same shared-memory
+// values, so none of them waits on a shuffle: indR / indC live in every lane as nibbles (R: indR[i] at bits 4i, i < 8;
+// C: indC[i] at bits 4(i-1), 1 <= i < 9), and every lane arrives at the same k, l.  The serial scans' order and their
+// strict comparisons are kept, so the pivots and the bits are jacobi<9>'s.
+// Returns the number of rotations.
+__device__ __noinline__ int jacobi9_warp(double* A, double* W, double* V)
 {
     const int lane = threadIdx.x & 31;
     const double eps = DBL_EPSILON;
     for (int e = lane; e < 81; e += 32) V[e] = (e / 9 == e % 9) ? 1.0 : 0.0;
     if (lane < 9) W[lane] = A[10 * lane];
-    // lane k keeps indR[k] (k < 8) and indC[k] (1 <= k < 9)
-    int myR = 0, myC = 0;
-    if (lane < 8) {
-        int m = lane + 1; double mv = fabs(A[9 * lane + m]);
-        for (int i = lane + 2; i < 9; i++) { const double val = fabs(A[9 * lane + i]); if (mv < val) { mv = val; m = i; } }
-        myR = m;
-    }
-    if (lane > 0 && lane < 9) {
-        int m = 0; double mv = fabs(A[lane]);
-        for (int i = 1; i < lane; i++) { const double val = fabs(A[9 * i + lane]); if (mv < val) { mv = val; m = i; } }
-        myC = m;
+    uint32_t R = 0, C = 0;
+    #pragma unroll
+    for (int i = 0; i < 8; i++) {
+        R |= (uint32_t)row_argmax9(A, i) << (4 * i);
+        C |= (uint32_t)col_argmax9(A, i + 1) << (4 * i);
     }
     __syncwarp();
-    for (int iters = 0; iters < 9 * 9 * 30; iters++) {
+    int iters = 0;
+    for (; iters < 9 * 9 * 30; iters++) {
         // ---- pivot: candidates in the serial scan order: rows 0..7 (k=i, l=indR[i]), then columns 1..8 (k=indC[i], l=i)
-        int ck = 0, cl = 0;
-        double cval = -1.0;
-        {
-            const int ci = __shfl_sync(0xffffffffu, myC, lane >= 8 ? lane - 7 : 0);    // indC[lane-7] for lanes 8..15
-            if (lane < 8) { ck = lane; cl = myR; }
-            else if (lane < 16) { ck = ci; cl = lane - 7; }
-            if (lane < 16) cval = fabs(A[9 * ck + cl]);
+        double cv[16]; int ci[16];
+        #pragma unroll
+        for (int i = 0; i < 8; i++) {
+            cv[i] = fabs(A[9 * i + ((R >> (4 * i)) & 15)]);
+            cv[8 + i] = fabs(A[9 * ((C >> (4 * i)) & 15) + (i + 1)]);
+            ci[i] = i; ci[8 + i] = 8 + i;
         }
-        int key = lane;
-        group_argmax_first<16>(cval, key);                         // lanes 0..15 agree; lanes 16..31 hold garbage
-        key = __shfl_sync(0xffffffffu, key, 0);
-        const int k = __shfl_sync(0xffffffffu, ck, key), l = __shfl_sync(0xffffffffu, cl, key);
+        #pragma unroll
+        for (int w = 1; w < 16; w *= 2)
+            #pragma unroll
+            for (int q = 0; q < 16; q += 2 * w) later_wins_if_larger(cv[q], ci[q], cv[q + w], ci[q + w]);
+        const int key = ci[0];
+        const int k = key < 8 ? key : (int)((C >> (4 * (key - 8))) & 15);
+        const int l = key < 8 ? (int)((R >> (4 * key)) & 15) : key - 7;
         const double p = A[9 * k + l];
         if (fabs(p) <= eps) break;
         const double y = (W[l] - W[k]) * 0.5;
-        double t = fabs(y) + cv_hypot(p, y);
-        double s = cv_hypot(p, t);
+        double t = fabs(y) + cv_hypot_sel(p, y);
+        double s = cv_hypot_sel(p, t);
+        const double pt = p / t;
         const double c = t / s;
-        s = p / s; t = (p / t) * p;
+        s = p / s; t = pt * p;
         if (y < 0) { s = -s; t = -t; }
         __syncwarp();
         if (lane == 0) { A[9 * k + l] = 0; W[k] -= t; W[l] += t; }
@@ -107,24 +149,14 @@ __device__ __noinline__ void jacobi9_warp(double* A, double* W, double* V)
             }
         }
         __syncwarp();
-        // ---- refresh indR[k], indR[l], indC[k], indC[l]: four 8-lane groups
+        // ---- refresh indR[k], indR[l], indC[k], indC[l] (k < l, so k < 8 and l >= 1 always)
         {
-            const int g = lane >> 3, j = lane & 7;
-            const int idx = (g & 1) ? l : k;
-            double val = -1.0; int cand = 0;
-            if (g < 2) {                       // row scan: i = idx+1 .. 8, value |A[idx][i]|
-                const int i = idx + 1 + j;
-                if (i < 9) { val = fabs(A[9 * idx + i]); cand = i; }
-            } else {                           // column scan: i = 0 .. idx-1, value |A[i][idx]|
-                const int i = j;
-                if (i < idx) { val = fabs(A[9 * i + idx]); cand = i; }
-            }
-            int kk = val >= 0 ? cand : 99;
-            group_argmax_first<8>(val, kk);
-            const int r0 = __shfl_sync(0xffffffffu, kk, 0), r1 = __shfl_sync(0xffffffffu, kk, 8);
-            const int r2 = __shfl_sync(0xffffffffu, kk, 16), r3 = __shfl_sync(0xffffffffu, kk, 24);
-            if (lane == k) { if (k < 8) myR = r0; if (k > 0) myC = r2; }
-            if (lane == l) { if (l < 8) myR = r1; if (l > 0) myC = r3; }
+            const uint32_t rk = row_argmax9(A, k), rl = row_argmax9(A, l);
+            const uint32_t ck = col_argmax9(A, k), cl = col_argmax9(A, l);
+            R = (R & ~(15u << (4 * k))) | (rk << (4 * k));
+            if (l < 8) R = (R & ~(15u << (4 * l))) | (rl << (4 * l));
+            if (k > 0) C = (C & ~(15u << (4 * (k - 1)))) | (ck << (4 * (k - 1)));
+            C = (C & ~(15u << (4 * (l - 1)))) | (cl << (4 * (l - 1)));
         }
     }
     __syncwarp();
@@ -146,16 +178,18 @@ __device__ __noinline__ void jacobi9_warp(double* A, double* W, double* V)
         }
         __syncwarp();
     }
+    return iters;
 }
 
 // cv::solve(A, b, x, DECOMP_EIG) for 9x9 (see solve_eig<9>): A, b read-only (any memory), x out (9, shared);
-// a, v: 81-double shared scratch, w: 9-double shared scratch.  Result visible to the warp after return.
-__device__ __forceinline__ void solve_eig9_warp(const double* A, const double* b, double* x, double* a, double* v, double* w)
+// a, v: 81-double shared scratch, w: 9-double shared scratch.  Result visible to the warp after return.  Returns the
+// number of rotations.
+__device__ __forceinline__ int solve_eig9_warp(const double* A, const double* b, double* x, double* a, double* v, double* w)
 {
     const int lane = threadIdx.x & 31;
     for (int e = lane; e < 81; e += 32) a[e] = A[e];
     __syncwarp();
-    jacobi9_warp(a, w, v);
+    const int rotations = jacobi9_warp(a, w, v);
     if (lane == 0) {
         double threshold = 0;
         for (int i = 0; i < 9; i++) x[i] = 0;
@@ -172,15 +206,19 @@ __device__ __forceinline__ void solve_eig9_warp(const double* A, const double* b
         }
     }
     __syncwarp();
+    return rotations;
 }
 
-// max |diag(cv::invert(A, DECOMP_EIG))| for 9x9 (see invert_eig_max_diag<9>); result in every lane
-__device__ __forceinline__ double invert_eig_max_diag9_warp(const double* A, double* a, double* v, double* w)
+// max |diag(cv::invert(A, DECOMP_EIG))| for 9x9 (see invert_eig_max_diag<9>); result in every lane.  *rotations (if given):
+// the number of rotations.
+__device__ __forceinline__ double invert_eig_max_diag9_warp(const double* A, double* a, double* v, double* w,
+                                                           int* rotations = nullptr)
 {
     const int lane = threadIdx.x & 31;
     for (int e = lane; e < 81; e += 32) a[e] = A[e];
     __syncwarp();
-    jacobi9_warp(a, w, v);
+    const int rot = jacobi9_warp(a, w, v);
+    if (rotations) *rotations = rot;
     double maxval = DBL_EPSILON;
     if (lane == 0) {
         double dg[9];

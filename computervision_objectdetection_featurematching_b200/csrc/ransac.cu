@@ -1206,21 +1206,23 @@ __device__ double lm_eval_exact(const float4* __restrict__ pts, const int32_t* _
 }
 
 // lm_step / lm_update with the 9x9 eigen-solves run cooperatively by warp 0 (all 32 lanes call)
-__device__ void lm_step_warp(LmState& st, FinishShared& sh)
+// (both return the number of rotations of their eigen-solve in *rotations, 0 for none)
+__device__ void lm_step_warp(LmState& st, FinishShared& sh, int* rotations)
 {
     const int lane = threadIdx.x & 31;
     double* Ap = sh.part;                                  // 81 doubles of scratch
     for (int e = lane; e < 81; e += 32) Ap[e] = st.A[e] + ((e / 9 == e % 9) ? st.lambda * st.D[e / 9] : 0.0);
     __syncwarp();
-    solve_eig9_warp(Ap, st.v, st.d, sh.scratch_a, sh.scratch_v, sh.scratch_w);
+    *rotations = solve_eig9_warp(Ap, st.v, st.d, sh.scratch_a, sh.scratch_v, sh.scratch_w);
     if (lane < 9) st.xd[lane] = st.x[lane] - st.d[lane];
     __syncwarp();
 }
 
-__device__ bool lm_update_warp(LmState& st, double Sd, FinishShared& sh)
+__device__ bool lm_update_warp(LmState& st, double Sd, FinishShared& sh, int* rotations)
 {
     const double Rlo = 0.25, Rhi = 0.75;
     const int lane = threadIdx.x & 31;
+    *rotations = 0;
     double temp_d[9];
     for (int i = 0; i < 9; i++) {
         const double s = dot4acc(st.A + i * 9, st.d, 9);
@@ -1238,7 +1240,7 @@ __device__ bool lm_update_warp(LmState& st, double Sd, FinishShared& sh)
         nu = nu > 2. ? nu : 2.;
         nu = nu < 10. ? nu : 10.;
         if (lambda == 0) {
-            const double maxval = invert_eig_max_diag9_warp(st.A, sh.scratch_a, sh.scratch_v, sh.scratch_w);
+            const double maxval = invert_eig_max_diag9_warp(st.A, sh.scratch_a, sh.scratch_v, sh.scratch_w, rotations);
             lambda = lc = 1. / maxval;
             nu *= 0.5;
         }
@@ -1251,6 +1253,27 @@ __device__ bool lm_update_warp(LmState& st, double Sd, FinishShared& sh)
 }
 
 // ---- 4. finish kernel -----------------------------------------------------------------------------
+// Phase probe (-DFIN_PROF, off in the product build): thread 0 of every set's CTA logs each phase as it ends, after the
+// phase's barrier, into g_fin_prof: (phase id | rotations << 8, SM cycles since the previous mark).  Entry 0 is the whole
+// set: (FP_TOTAL | n_inl << 8, nanoseconds of %globaltimer).  cvg_finish_profile (below) copies the log to the host.
+#ifdef FIN_PROF
+enum FinPhase { FP_TOTAL = 0, FP_COMPACT, FP_DLT_SUMS, FP_DLT_LTL, FP_REFIT_EIG, FP_EVAL_J, FP_LM_SOLVE, FP_EVAL_XD,
+                FP_LM_UPDATE, FP_LM_PROCEED, FP_MASK };
+constexpr int FP_SETS = 256, FP_EVENTS = 96;
+__device__ long long g_fin_prof[FP_SETS][FP_EVENTS][2];
+__device__ int g_fin_prof_n[FP_SETS];
+#define FPROF_BEGIN long long fp_t = clock64(), fp_ns = 0; int fp_n = 1; \
+    if (tid == 0) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(fp_ns));
+#define FPROF(phase, rot) if (tid == 0 && set < FP_SETS && fp_n < FP_EVENTS) { \
+        const long long t_ = clock64(); g_fin_prof[set][fp_n][0] = (phase) | ((long long)(rot) << 8); \
+        g_fin_prof[set][fp_n][1] = t_ - fp_t; fp_n++; fp_t = t_; }
+#define FPROF_END(n_inl) if (tid == 0 && set < FP_SETS) { long long ns_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns_)); \
+        g_fin_prof[set][0][0] = FP_TOTAL | ((long long)(n_inl) << 8); g_fin_prof[set][0][1] = ns_ - fp_ns; g_fin_prof_n[set] = fp_n; }
+#else
+#define FPROF_BEGIN
+#define FPROF(phase, rot)
+#define FPROF_END(n_inl)
+#endif
 __global__ void __launch_bounds__(RS_THREADS)
 ransac_finish_kernel(RansacWork w)
 {
@@ -1312,6 +1335,7 @@ ransac_finish_kernel(RansacWork w)
     } else if (tid < 32) solve_winner();
     if (tid == 0) sh.base_cnt = 0;
     __syncthreads();
+    FPROF_BEGIN
     float Hf[8];
     #pragma unroll
     for (int i = 0; i < 8; i++) Hf[i] = sh.Hf[i];
@@ -1336,6 +1360,7 @@ ransac_finish_kernel(RansacWork w)
         __syncthreads();
     }
     const int n_inl = sh.base_cnt;
+    FPROF(FP_COMPACT, 0)
     if (w.flags & CVG_RANSAC_NO_REFINE) {
         if (tid < 9) Hout[tid] = sh.H[tid];
         if (tid == 0) w.found[set] = 1;
@@ -1384,6 +1409,7 @@ ransac_finish_kernel(RansacWork w)
             block_sum<4>(s, sh.part, sh.out);
             smx = s[0]; smy = s[1]; sMx = s[2]; sMy = s[3];
         }
+        FPROF(FP_DLT_SUMS, 0)
         const bool dlt_ok = !(fabs(smx) < DBL_EPSILON || fabs(smy) < DBL_EPSILON ||
                               fabs(sMx) < DBL_EPSILON || fabs(sMy) < DBL_EPSILON);
         if (!dlt_ok && have_model) {                         // block-uniform: LM starts from the RANSAC model in fp64
@@ -1433,8 +1459,10 @@ ransac_finish_kernel(RansacWork w)
                 }
             }
             __syncthreads();
+            FPROF(FP_DLT_LTL, 0)
+            int rot = 0;
             if (tid < 32) {
-                jacobi9_warp(LtL, sh.scratch_w, sh.scratch_v);
+                rot = jacobi9_warp(LtL, sh.scratch_w, sh.scratch_v);
                 if (tid == 0) {
                     const double invHnorm[9] = { 1. / smx, 0, cmx, 0, 1. / smy, cmy, 0, 0, 1 };
                     const double Hnorm2[9] = { sMx, 0, -cMx * sMx, 0, sMy, -cMy * sMy, 0, 0, 1 };
@@ -1447,6 +1475,7 @@ ransac_finish_kernel(RansacWork w)
                 }
             }
             __syncthreads();
+            FPROF(FP_REFIT_EIG, rot)
         }
         // ---- B.8: LMSolver (9 parameters, 10 iterations); reductions by the block, eigen-solves by warp 0 ----
         LmState& st = sh.lm;
@@ -1463,17 +1492,22 @@ ransac_finish_kernel(RansacWork w)
                 lm_begin(st);
             }
             __syncthreads();
+            FPROF(FP_EVAL_J, 0)
         }
         for (;;) {
-            if (tid < 32) lm_step_warp(st, sh);
+            int rot = 0;
+            if (tid < 32) lm_step_warp(st, sh, &rot);
             __syncthreads();
+            FPROF(FP_LM_SOLVE, rot)
             const double Sd = exact ? lm_eval_exact(pts, sel, n_inl, st.xd, false, nullptr, nullptr, nullptr, sh)
                                     : lm_eval_block(pts, sel, n_inl, st.xd, nullptr, nullptr, nullptr, sh);
+            FPROF(FP_EVAL_XD, 0)
             if (tid < 32) {
-                const bool acc = lm_update_warp(st, Sd, sh);
+                const bool acc = lm_update_warp(st, Sd, sh, &rot);
                 if (tid == 0) sh.flag = acc ? 1 : 0;
             }
             __syncthreads();
+            FPROF(FP_LM_UPDATE, rot)
             if (sh.flag) {
                 if (tid < 9) st.x[tid] = st.xd[tid];
                 __syncthreads();
@@ -1486,9 +1520,11 @@ ransac_finish_kernel(RansacWork w)
                     st.S = S; st.rmax = rmax;
                 }
                 __syncthreads();
+                FPROF(FP_EVAL_J, 0)
             }
             if (tid == 0) sh.flag = lm_proceed(st, 10) ? 1 : 0;
             __syncthreads();
+            FPROF(FP_LM_PROCEED, 0)
             if (!sh.flag) break;
         }
         if (tid == 0) {
@@ -1503,6 +1539,8 @@ ransac_finish_kernel(RansacWork w)
             const float4 q = pts[i];
             mask[i] = reproj_err(Hf, q.x, q.y, q.z, q.w) <= w.thr2 ? 1 : 0;
         }
+        FPROF(FP_MASK, 0)
+        FPROF_END(n_inl)
     } else {
         for (int i = tid; i < n; i += (int)blockDim.x) mask[i] = 0;
         if (have_model) {                                    // never reached with a winner of >= 4 inliers; keep H defined
@@ -1513,6 +1551,19 @@ ransac_finish_kernel(RansacWork w)
     if (tid < 9) Hout[tid] = sh.H[tid];
     if (tid == 0) w.found[set] = 1;
 }
+
+#ifdef FIN_PROF
+// Copies the phase log of the last finish launches (sets 0 .. n_sets-1, FP_EVENTS entries of two int64 each per set, then
+// one int32 entry count per set) to the host and clears the counts.  Exported only by a -DFIN_PROF build.
+extern "C" int cvg_finish_profile(long long* log, int* counts, int n_sets)
+{
+    if (n_sets < 0 || n_sets > FP_SETS) return -1;
+    if (cudaMemcpyFromSymbol(log, g_fin_prof, sizeof(long long) * 2 * FP_EVENTS * n_sets) != cudaSuccess) return -1;
+    if (cudaMemcpyFromSymbol(counts, g_fin_prof_n, sizeof(int) * n_sets) != cudaSuccess) return -1;
+    static int zero[FP_SETS];
+    return cudaMemcpyToSymbol(g_fin_prof_n, zero, sizeof(zero)) == cudaSuccess ? FP_EVENTS : -1;
+}
+#endif
 
 // layout of the chunked sampler's scratch inside one allocation; returns the total size
 int64_t ransac_chunk_scratch_bytes(int n_sets, int n_chunks, size_t* outs, size_t* lists, size_t* offsets, size_t* serial,
@@ -1552,6 +1603,120 @@ __global__ void selftest_rcp_kernel(unsigned long long* mismatches)
 int launch_selftest_rcp(unsigned long long* d_mismatches, cudaStream_t st)
 {
     selftest_rcp_kernel<<<148 * 16, 256, 0, st>>>(d_mismatches);
+    return 1;
+}
+
+// ---- self test 1: the warp-cooperative 9x9 routines (jacobi_warp.cuh) == the serial ones (homography_math.cuh) ----------
+// One warp per matrix; lane 0 builds the matrix from its index (no host data) and runs the serial routine on the device.
+// Every output double is compared bit for bit: W and V of jacobi, x of solve, the returned maximum of invert.
+struct StRng {
+    uint64_t s;
+    __device__ uint64_t next()
+    {
+        uint64_t z = (s += 0x9E3779B97F4A7C15ull);
+        z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+        z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+        return z ^ (z >> 31);
+    }
+    __device__ double unif() { return (double)(next() >> 11) * 0x1.0p-53; }     // [0, 1)
+    __device__ int below(int n) { return (int)(next() % (uint64_t)n); }
+};
+
+// LtL of a normalised DLT over n correspondences (a near-affine map with 30 % outliers), as the refit builds it
+__device__ void selftest_dlt(StRng& r, int n, double* LtL)
+{
+    const uint64_t seed = r.next();
+    auto point = [&](int i, float& Mx, float& My, float& mx, float& my) {
+        StRng q{ seed + (uint64_t)i * 0x2545F4914F6CDD1Dull };
+        Mx = (float)(640 * q.unif()); My = (float)(480 * q.unif());
+        if (q.unif() < 0.3) { mx = (float)(640 * q.unif()); my = (float)(480 * q.unif()); }
+        else { mx = (float)(0.9 * Mx + 0.05 * My + 20 + q.unif() - 0.5); my = (float)(-0.04 * Mx + 1.1 * My - 7 + q.unif() - 0.5); }
+    };
+    double cMx = 0, cMy = 0, cmx = 0, cmy = 0, sMx = 0, sMy = 0, smx = 0, smy = 0;
+    float Mx, My, mx, my;
+    for (int i = 0; i < n; i++) { point(i, Mx, My, mx, my); cmx += mx; cmy += my; cMx += Mx; cMy += My; }
+    cmx /= n; cmy /= n; cMx /= n; cMy /= n;
+    for (int i = 0; i < n; i++) {
+        point(i, Mx, My, mx, my);
+        smx += fabs(mx - cmx); smy += fabs(my - cmy); sMx += fabs(Mx - cMx); sMy += fabs(My - cMy);
+    }
+    smx = n / smx; smy = n / smy; sMx = n / sMx; sMy = n / sMy;
+    for (int e = 0; e < 81; e++) LtL[e] = 0;
+    for (int i = 0; i < n; i++) { point(i, Mx, My, mx, my); dlt_accumulate_point(LtL, Mx, My, mx, my, cMx, cMy, cmx, cmy, sMx, sMy, smx, smy); }
+}
+
+__device__ void selftest_matrix(int idx, double* M, double* b)
+{
+    StRng r{ 0x5EEDull * 1000003ull + (uint64_t)idx };
+    switch (idx % 5) {
+    case 0: selftest_dlt(r, 4, M); break;                                    // a 4-point sample
+    case 1: selftest_dlt(r, 5 + r.below(3996), M); break;                    // a refit over 5 .. 4000 inliers
+    case 2: {                                                                // LM: J^T J + lambda * diag(J^T J)
+        for (int e = 0; e < 81; e++) M[e] = 0;
+        const int rows = 10 + r.below(400);
+        for (int q = 0; q < rows; q++) {
+            double J[9];
+            for (int j = 0; j < 9; j++) J[j] = (2 * r.unif() - 1) * (j < 6 ? 1.0 : 1e-3);
+            for (int j = 0; j < 9; j++) for (int k = j; k < 9; k++) M[j * 9 + k] += J[j] * J[k];
+        }
+        const double lambda = pow(10.0, -6 + 8 * r.unif());
+        for (int j = 0; j < 9; j++) M[j * 10] = M[j * 10] + lambda * M[j * 10];
+        break;
+    }
+    case 3: {                                                                // small integers: tied pivot candidates
+        for (int j = 0; j < 9; j++) for (int k = j; k < 9; k++) M[j * 9 + k] = (double)(r.below(5) - 2) * (j == k ? -2 : 1);
+        break;
+    }
+    default: {                                                               // zeros in the upper triangle
+        const double pz = r.unif();
+        for (int j = 0; j < 9; j++)
+            for (int k = j; k < 9; k++) M[j * 9 + k] = (k > j && r.unif() < pz) ? 0.0 : 2 * r.unif() - 1;
+        break;
+    }
+    }
+    for (int j = 0; j < 9; j++) for (int k = 0; k < j; k++) M[j * 9 + k] = M[k * 9 + j];
+    for (int j = 0; j < 9; j++) b[j] = 2 * r.unif() - 1;
+}
+
+constexpr int STJ_WARPS = 4;
+constexpr int STJ_DOUBLES = 81 * 5 + 9 * 4;
+__global__ void __launch_bounds__(STJ_WARPS * 32) selftest_jacobi_kernel(unsigned long long* mismatches, int n_mats)
+{
+    __shared__ double sm[STJ_WARPS][STJ_DOUBLES];
+    const int lane = threadIdx.x & 31;
+    double* M = sm[threadIdx.x >> 5];
+    double* a = M + 81; double* v = a + 81; double* sa = v + 81; double* sv = sa + 81;
+    double* w = sv + 81; double* b = w + 9; double* x = b + 9; double* xs = x + 9;
+    unsigned long long bad = 0;
+    for (int m = blockIdx.x * STJ_WARPS + (threadIdx.x >> 5); m < n_mats; m += gridDim.x * STJ_WARPS) {
+        if (lane == 0) selftest_matrix(m, M, b);
+        __syncwarp();
+        for (int e = lane; e < 81; e += 32) a[e] = M[e];
+        __syncwarp();
+        jacobi9_warp(a, w, v);
+        if (lane == 0) {
+            double ws[9];
+            for (int e = 0; e < 81; e++) sa[e] = M[e];
+            jacobi<9>(sa, ws, sv);
+            for (int i = 0; i < 9; i++) bad += __double_as_longlong(w[i]) != __double_as_longlong(ws[i]);
+            for (int e = 0; e < 81; e++) bad += __double_as_longlong(v[e]) != __double_as_longlong(sv[e]);
+        }
+        __syncwarp();
+        solve_eig9_warp(M, b, x, a, v, w);
+        if (lane == 0) {
+            solve_eig<9>(M, b, xs, sa, sv);
+            for (int i = 0; i < 9; i++) bad += __double_as_longlong(x[i]) != __double_as_longlong(xs[i]);
+        }
+        __syncwarp();
+        const double mv = invert_eig_max_diag9_warp(M, a, v, w);
+        if (lane == 0) bad += __double_as_longlong(mv) != __double_as_longlong(invert_eig_max_diag<9>(M, sa, sv));
+        __syncwarp();
+    }
+    if (lane == 0 && bad) atomicAdd(mismatches, bad);
+}
+int launch_selftest_jacobi(unsigned long long* d_mismatches, int n_mats, cudaStream_t st)
+{
+    selftest_jacobi_kernel<<<(n_mats + STJ_WARPS - 1) / STJ_WARPS, STJ_WARPS * 32, 0, st>>>(d_mismatches, n_mats);
     return 1;
 }
 
