@@ -12,6 +12,11 @@ class RansacParams(C.Structure):
                 ("confidence", C.c_double), ("max_iters", C.c_int32), ("reserved", C.c_int32)]
 
 
+class AffineParams(C.Structure):
+    _fields_ = [("size", C.c_uint32), ("flags", C.c_uint32), ("threshold", C.c_double),
+                ("confidence", C.c_double), ("max_iters", C.c_int32), ("refine_iters", C.c_int32)]
+
+
 class DetectParams(C.Structure):
     _fields_ = [("size", C.c_uint32), ("ratio", C.c_float), ("min_inliers", C.c_int32), ("det_lo", C.c_float),
                 ("det_hi", C.c_float), ("reserved", C.c_int32), ("ransac", RansacParams)]
@@ -27,6 +32,7 @@ _P = C.c_void_p
 SYMBOLS = {
     "cvg_ransac_params_default": (None, [C.POINTER(RansacParams)]),
     "cvg_detect_params_default": (None, [C.POINTER(DetectParams)]),
+    "cvg_affine_params_default": (None, [C.POINTER(AffineParams)]),
     "cvg_create": (C.c_int, [C.POINTER(_P), C.c_int, C.c_uint]),
     "cvg_create_multi": (C.c_int, [C.POINTER(_P), C.POINTER(C.c_int), C.c_int, C.c_uint]),
     "cvg_num_devices": (C.c_int, [_P]),
@@ -51,6 +57,8 @@ SYMBOLS = {
     "cvg_match_knn2_raw": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_float, _P, _P, _P]),
     "cvg_find_homography": (C.c_int, [_P, _P, _P, C.c_int, C.POINTER(RansacParams), _P, _P, C.POINTER(C.c_int), _P]),
     "cvg_find_homography_batch": (C.c_int, [_P, _P, _P, _P, C.c_int, C.POINTER(RansacParams), _P, _P, _P, _P, _P]),
+    "cvg_estimate_affine2d": (C.c_int, [_P, _P, _P, C.c_int, C.POINTER(AffineParams), _P, _P, C.POINTER(C.c_int)]),
+    "cvg_estimate_affine2d_batch": (C.c_int, [_P, _P, _P, _P, C.c_int, C.POINTER(AffineParams), _P, _P, _P, _P]),
     "cvg_detect_pairs": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_float, C.POINTER(DetectParams), _P, _P, _P]),
     "cvg_scenes_upload": (C.c_int, [_P, _P, _P, _P, C.c_int, C.POINTER(_P)]),
     "cvg_scenes_free": (None, [_P, _P]),

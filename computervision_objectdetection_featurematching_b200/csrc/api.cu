@@ -86,6 +86,12 @@ void cvg_ransac_params_default(cvg_ransac_params* p)
     p->size = sizeof *p; p->flags = 0; p->threshold = 5.0; p->confidence = 0.995; p->max_iters = 2000;
 }
 
+void cvg_affine_params_default(cvg_affine_params* p)
+{
+    memset(p, 0, sizeof *p);
+    p->size = sizeof *p; p->flags = 0; p->threshold = 3.0; p->confidence = 0.99; p->max_iters = 2000; p->refine_iters = 10;
+}
+
 void cvg_detect_params_default(cvg_detect_params* p)
 {
     memset(p, 0, sizeof *p);
@@ -531,7 +537,8 @@ __global__ void combine_flags_kernel(int* f, const int* train_flag, int extra_ki
 
 // Scratch, flags and parameters of the verify stage on a device correspondence pool, ready for launch_ransac or its phases.
 int eng_ransac_work(cvg_ctx* c, const float4* d_pts, const int64_t* d_starts, const int32_t* d_counts_n, int n_sets,
-                    int max_n, int64_t pool_rows, const cvg_ransac_params* p, bool want_rmask, int counts_slack, RansacWork* out)
+                    int max_n, int64_t pool_rows, const cvg_ransac_params* p, bool want_rmask, int counts_slack, RansacWork* out,
+                    int model_points)
 {
     int rc = ensure_rng(c, p->max_iters);
     if (rc) return rc;
@@ -556,7 +563,10 @@ int eng_ransac_work(cvg_ctx* c, const float4* d_pts, const int64_t* d_starts, co
     w.pts = d_pts; w.starts = d_starts; w.counts_n = d_counts_n; w.n_sets = n_sets; w.max_n = max_n;
     w.n_sms = c->n_sms; w.wave_div = std::max(1, c->wave_div);
     w.max_iters = mi;
-    const double thr = p->threshold > 0 ? p->threshold : 3.0;        // defaultRANSACReprojThreshold
+    w.model_points = model_points;
+    c->nit_mp = model_points;
+    // findHomography replaces a threshold <= 0 by defaultRANSACReprojThreshold; estimateAffine2D squares what it is given
+    const double thr = (p->threshold > 0 || model_points != 4) ? p->threshold : 3.0;
     w.thr2 = (float)(thr * thr);
     w.conf = p->confidence; w.flags = p->flags;
     w.rng_tab = c->d_rng; w.rng_len = c->rng_len;
@@ -572,7 +582,8 @@ int eng_ransac_work(cvg_ctx* c, const float4* d_pts, const int64_t* d_starts, co
     w.chunk_outs = nullptr; w.chunk_lists = nullptr; w.chunk_offsets = nullptr; w.chunk_serial = nullptr; w.n_chunks = 0;
     w.chunk_maps = nullptr; w.chunk_entries = nullptr; w.chunk_serial_count = nullptr;
     c->last_chunked = false;
-    if ((p->flags & CVG_RANSAC_NO_EARLY_STOP) && mi >= 32768 && n_sets <= 65535) {     // sets ride on gridDim.y of the chunk kernels
+    // (4-point draws only; estimateAffine2D calls run on the round sampler)
+    if (model_points == 4 && (p->flags & CVG_RANSAC_NO_EARLY_STOP) && mi >= 32768 && n_sets <= 65535) {     // sets ride on gridDim.y of the chunk kernels
         // one huge round: the draw stream of every set is walked by many CTAs at once (ransac_sample_chunk_kernel)
         const int n_chunks = ransac_chunks_for_table(c->rng_len);
         size_t o_outs, o_lists, o_off, o_ser, o_maps, o_ent;
@@ -632,12 +643,12 @@ int nit_add_requests(cvg_ctx* c, std::vector<NitEntry>& tab, size_t* added_out)
     size_t added = 0;
     for (const int2& r : req) {
         bool have = false;
-        for (const NitEntry& e : tab) if (e.n == r.x && e.good == r.y) { have = true; break; }
+        for (const NitEntry& e : tab) if (e.n == r.x && e.good == r.y && e.mp == c->nit_mp) { have = true; break; }
         if (have || r.x <= 0) continue;
         double ep = (double)(r.x - r.y) / r.x;                       // ptsetreg.cpp: (double)(count - goodCount) / count
         ep = ep > 0. ? ep : 0.; ep = ep < 1. ? ep : 1.;
-        const double d0 = 1. - pow(1. - ep, 4);                      // modelPoints = 4
-        NitEntry e; e.n = r.x; e.good = r.y; e.zero = d0 < DBL_MIN ? 1 : 0; e.denom_log = e.zero ? -1. : log(d0); e.pad = 0;
+        const double d0 = 1. - pow(1. - ep, c->nit_mp);              // pow(1 - ep, modelPoints)
+        NitEntry e; e.n = r.x; e.good = r.y; e.zero = d0 < DBL_MIN ? 1 : 0; e.denom_log = e.zero ? -1. : log(d0); e.mp = c->nit_mp;
         tab.push_back(e); added++;
     }
     *added_out = added;
@@ -855,14 +866,13 @@ int cvg_match_knn2_raw(cvg_ctx* c, const float* query, int n_query, const float*
 }
 
 // ---- verify stage ---------------------------------------------------------------------------------
-int cvg_find_homography_batch(cvg_ctx* c, const float* src_xy, const float* dst_xy, const int64_t* offsets,
-                              int n_sets, const cvg_ransac_params* p, double* H, uint8_t* mask, int32_t* found,
-                              int32_t* iters, uint8_t* ransac_mask)
+// One batched verify call: pack the sets, run the stage (findHomography for model_points 4, estimateAffine2D for 3), copy
+// the results back; repeat it with a longer cv::RNG draw table when a set ran out of draws, or after the host answered the
+// device's RANSACUpdateNumIters requests.  M gets m_doubles per set (9: H, 6: the 2x3 affine matrix).
+static int verify_batch(cvg_ctx* c, const float* src_xy, const float* dst_xy, const int64_t* offsets, int n_sets,
+                        const cvg_ransac_params* p, int model_points, int refine_iters, double* M, int m_doubles,
+                        uint8_t* mask, int32_t* found, int32_t* iters, uint8_t* ransac_mask)
 {
-    c = cvg_primary(c);
-    if (!c || !offsets || n_sets < 0) return set_err(CVG_ERR_INVALID, "cvg_find_homography_batch: bad argument");
-    int rc = check_params(p);
-    if (rc) return rc;
     if (n_sets == 0) return CVG_OK;
     CU_CHECK(cudaSetDevice(c->device));
     const int64_t total = offsets[n_sets];
@@ -886,13 +896,21 @@ int cvg_find_homography_batch(cvg_ctx* c, const float* src_xy, const float* dst_
     launch_pack_points(c->src.as<float>(), c->dst.as<float>(), total, c->pts.as<float4>(), c->stream);
     c->launches++;
     std::vector<int32_t> sflags(n_sets);
+    int rc;
     for (int attempt = 0;; attempt++) {
         if (c->timing) cudaEventRecord(c->ev[0], c->stream);
-        rc = run_ransac(c, c->pts.as<float4>(), c->starts.as<int64_t>(), c->counts_n.as<int32_t>(), n_sets, max_n, total, p,
-                        ransac_mask != nullptr);
+        if (model_points == 4) {
+            rc = run_ransac(c, c->pts.as<float4>(), c->starts.as<int64_t>(), c->counts_n.as<int32_t>(), n_sets, max_n, total, p,
+                            ransac_mask != nullptr);
+        } else {
+            RansacWork w;
+            rc = eng_ransac_work(c, c->pts.as<float4>(), c->starts.as<int64_t>(), c->counts_n.as<int32_t>(), n_sets, max_n, total,
+                                 p, false, 0, &w, model_points);
+            if (!rc) { c->launches += launch_affine(w, refine_iters, c->stream); CU_CHECK(cudaGetLastError()); }
+        }
         if (rc) return rc;
         if (c->timing) cudaEventRecord(c->ev[1], c->stream);
-        if (H) CU_CHECK(cudaMemcpyAsync(H, c->H.p, (size_t)n_sets * 72, cudaMemcpyDeviceToHost, c->stream));
+        if (M) CU_CHECK(cudaMemcpyAsync(M, c->H.p, (size_t)n_sets * m_doubles * 8, cudaMemcpyDeviceToHost, c->stream));
         if (mask && total > 0) CU_CHECK(cudaMemcpyAsync(mask, c->mask.p, (size_t)total, cudaMemcpyDeviceToHost, c->stream));
         if (ransac_mask && total > 0) CU_CHECK(cudaMemcpyAsync(ransac_mask, c->rmask.p, (size_t)total, cudaMemcpyDeviceToHost, c->stream));
         if (found) CU_CHECK(cudaMemcpyAsync(found, c->found.p, (size_t)n_sets * 4, cudaMemcpyDeviceToHost, c->stream));
@@ -920,6 +938,17 @@ int cvg_find_homography_batch(cvg_ctx* c, const float* src_xy, const float* dst_
     return CVG_OK;
 }
 
+int cvg_find_homography_batch(cvg_ctx* c, const float* src_xy, const float* dst_xy, const int64_t* offsets,
+                              int n_sets, const cvg_ransac_params* p, double* H, uint8_t* mask, int32_t* found,
+                              int32_t* iters, uint8_t* ransac_mask)
+{
+    c = cvg_primary(c);
+    if (!c || !offsets || n_sets < 0) return set_err(CVG_ERR_INVALID, "cvg_find_homography_batch: bad argument");
+    const int rc = check_params(p);
+    if (rc) return rc;
+    return verify_batch(c, src_xy, dst_xy, offsets, n_sets, p, 4, 0, H, 9, mask, found, iters, ransac_mask);
+}
+
 int cvg_find_homography(cvg_ctx* c, const float* src_xy, const float* dst_xy, int n, const cvg_ransac_params* p,
                         double H[9], uint8_t* mask, int* found, uint8_t* ransac_mask)
 {
@@ -927,6 +956,33 @@ int cvg_find_homography(cvg_ctx* c, const float* src_xy, const float* dst_xy, in
     const int64_t offs[2] = { 0, n };
     int32_t f = 0;
     int rc = cvg_find_homography_batch(c, src_xy, dst_xy, offs, 1, p, H, mask, &f, nullptr, ransac_mask);
+    if (found) *found = f;
+    return rc;
+}
+
+int cvg_estimate_affine2d_batch(cvg_ctx* c, const float* src_xy, const float* dst_xy, const int64_t* offsets, int n_sets,
+                                const cvg_affine_params* p, double* M, uint8_t* mask, int32_t* found, int32_t* iters)
+{
+    c = cvg_primary(c);
+    if (!c || !offsets || n_sets < 0) return set_err(CVG_ERR_INVALID, "cvg_estimate_affine2d_batch: bad argument");
+    if (!p || p->size != sizeof(cvg_affine_params)) return set_err(CVG_ERR_INVALID, "cvg_affine_params: bad size field");
+    if (p->flags & ~CVG_RANSAC_NO_EARLY_STOP) return set_err(CVG_ERR_INVALID, "cvg_affine_params: unknown flags 0x%x", p->flags);
+    if (p->refine_iters < 0 || p->refine_iters > 1000) return set_err(CVG_ERR_LIMIT, "refine_iters out of range [0, 1000]");
+    cvg_ransac_params rp;
+    cvg_ransac_params_default(&rp);
+    rp.flags = p->flags; rp.threshold = p->threshold; rp.confidence = p->confidence; rp.max_iters = p->max_iters;
+    const int rc = check_params(&rp);
+    if (rc) return rc;
+    return verify_batch(c, src_xy, dst_xy, offsets, n_sets, &rp, 3, p->refine_iters, M, 6, mask, found, iters, nullptr);
+}
+
+int cvg_estimate_affine2d(cvg_ctx* c, const float* src_xy, const float* dst_xy, int n, const cvg_affine_params* p,
+                          double M[6], uint8_t* mask, int* found)
+{
+    if (n <= 0) return set_err(CVG_ERR_TOO_FEW_POINTS, "estimateAffine2D needs at least one correspondence (got %d)", n);
+    const int64_t offs[2] = { 0, n };
+    int32_t f = 0;
+    const int rc = cvg_estimate_affine2d_batch(c, src_xy, dst_xy, offs, 1, p, M, mask, &f, nullptr);
     if (found) *found = f;
     return rc;
 }

@@ -165,6 +165,7 @@ struct cvg_ctx {
     DevBuf H, mask, rmask, found, sflags, results, inl_xy, inl_cnt, scales, src, dst;
     DevBuf nit, nitreq;                                // host-verified RANSACUpdateNumIters entries, the device's requests (run_ransac)
     std::vector<cvg::NitEntry> nit_host;
+    int nit_mp = 4;                                    // model points of the last verify stage (keys its niters requests)
     BufPool pool;                                      // recycled buffers of freed scene batches
     // Small host->device parameter blocks of the fused path go through a mapped pinned staging area read by a
     // copy kernel, not through cudaMemcpyAsync: the H2D copy engine may be busy for milliseconds with the next
@@ -235,7 +236,7 @@ int  ensure_rng(cvg_ctx* c, int max_iters, int64_t min_len = 0);   // the engine
 // scratch, flags and parameters of a verify stage over n_sets sets of the pool; counts gets counts_slack extra entries
 int  eng_ransac_work(cvg_ctx* c, const float4* d_pts, const int64_t* d_starts, const int32_t* d_counts_n, int n_sets,
                      int max_n, int64_t pool_rows, const cvg_ransac_params* p, bool want_rmask, int counts_slack,
-                     cvg::RansacWork* out);
+                     cvg::RansacWork* out, int model_points = 4);
 int  nit_add_requests(cvg_ctx* c, std::vector<cvg::NitEntry>& tab, size_t* added);   // the engine's niters requests into tab
 int  nit_upload(cvg_ctx* c);                            // c->nit_host to the device (stream-ordered, synchronised)
 

@@ -764,7 +764,7 @@ int cvg_find_homography_sharded(cvg_ctx* c, const float* src_xy, const float* ds
             rng_len = std::max(rng_len, e->rng_len);
             for (const NitEntry& x : e->nit_host) {
                 bool have = false;
-                for (const NitEntry& y : tab) if (x.n == y.n && x.good == y.good) { have = true; break; }
+                for (const NitEntry& y : tab) if (x.n == y.n && x.good == y.good && x.mp == y.mp) { have = true; break; }
                 if (!have) tab.push_back(x);
             }
         }

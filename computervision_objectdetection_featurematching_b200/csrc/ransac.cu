@@ -36,21 +36,21 @@ constexpr int RS_THREADS = 128;
 constexpr int EXACT_MAX_INLIERS = 128;
 constexpr int SMEM_PTS = 1024;              // correspondences staged per shared-memory tile
 
-// ---- draw 4 distinct indices starting at table position p (getSubset's inner loop) ----------------
+// ---- draw MP distinct indices starting at table position p (getSubset's inner loop) ---------------
 // `get(pos)` returns uniform(0, n) for draw position pos, i.e. rng_tab[pos] % n, or -1 past the table.
 // returns the number of draws consumed, or -1 when the table would be overrun
-template <class Get>
-__device__ __forceinline__ int draw_subset_g(const Get& get, int64_t p, int idx[4])
+template <int MP = 4, class Get>
+__device__ __forceinline__ int draw_subset_g(const Get& get, int64_t p, int* idx)
 {
     int64_t pos = p;
     #pragma unroll
-    for (int i = 0; i < 4; i++) {
+    for (int i = 0; i < MP; i++) {
         for (;;) {
             const int v = get(pos++);
             if (v < 0) return -1;
             bool dup = false;
             #pragma unroll
-            for (int k = 0; k < 4; k++) dup |= (k < i) && (idx[k] == v);
+            for (int k = 0; k < MP; k++) dup |= (k < i) && (idx[k] == v);
             if (!dup) { idx[i] = v; break; }
         }
     }
@@ -72,12 +72,15 @@ __device__ __forceinline__ int draw_subset(const uint32_t* __restrict__ tab, int
 // A window of SW consecutive draw positions is evaluated in parallel: for every position p the attempt
 // that would start there (draws consumed, checkSubset verdict).  The serial getSubset visits the chain
 // p -> p + consumed(p); the nodes of that chain inside the window are found by pointer jumping
-// (log2(SW/4) doubling rounds: an attempt consumes >= 4 draws, so a window holds <= SW/4 chain nodes),
-// ranked by a block prefix sum, and the accepted ones become the samples of consecutive iterations —
-// the same order, rejected attempts and 10000-attempt limit as the serial loop.
+// (ceil(log2(SW/MP)) doubling rounds: an attempt of an MP-point model consumes >= MP draws, so a window holds
+// <= SW/MP chain nodes), ranked by a block prefix sum, and the accepted ones become the samples of consecutive
+// iterations — the same order, rejected attempts and 10000-attempt limit as the serial loop.
+// MP = 4: findHomography (checkSubset: collinearity + orientation); MP = 3: estimateAffine2D (collinearity only).
 constexpr int SW = 2048;                          // measured: 512 -> 2048 halves the sampler time per draw (fewer serial windows)
-constexpr int SW_ROUNDS = 9;                      // log2(SW / 4)
-static_assert((4 << SW_ROUNDS) == SW, "pointer-jumping rounds must cover SW / 4 chain nodes");
+constexpr int SW_ROUNDS = 9;                      // log2(SW / 4): the 4-point chunked sampler below
+template <int MP> __host__ __device__ constexpr int sw_rounds() { int r = 0; while ((MP << r) < SW) r++; return r; }
+static_assert(sw_rounds<4>() == SW_ROUNDS && (4 << SW_ROUNDS) == SW, "pointer-jumping rounds must cover SW / 4 chain nodes");
+static_assert(sw_rounds<3>() == 10 && (3 << sw_rounds<3>()) >= SW, "pointer-jumping rounds must cover SW / 3 chain nodes");
 constexpr int SW_TAIL = 64;                       // draws staged beyond the window for attempts that start near its end
 constexpr int SMP_THREADS = 512;                  // one window offset per thread
 constexpr int SW_PER_THREAD = SW / SMP_THREADS;
@@ -85,9 +88,11 @@ constexpr int SW_PER_THREAD = SW / SMP_THREADS;
 // Samples are produced round by round (iterations [round_base, round_end)); the stream position and the
 // running failure count persist in smp_state between rounds, and a set whose adaptive niters already
 // ended before round_base is skipped.
+template <int MP>
 __global__ void __launch_bounds__(SMP_THREADS)
 ransac_sample_kernel(RansacWork w, int round_base, int round_end, const int* __restrict__ only_if_flag)
 {
+    constexpr int ROUNDS = sw_rounds<MP>();
     const int set = blockIdx.x;
     if (only_if_flag && only_if_flag[set] == 0) return;          // chunked sampler handled this set
     const int n = w.counts_n[set];
@@ -98,10 +103,10 @@ ransac_sample_kernel(RansacWork w, int round_base, int round_end, const int* __r
             w.n_samples[set] = 0; w.status_flags[set] = 0;
             w.smp_state[2 * set] = 0; w.smp_state[2 * set + 1] = 0;
         }
-        if (n <= 4) return;                         // n < 4: nothing; n == 4: handled by finish kernel
+        if (n <= MP) return;                        // n < MP: nothing; n == MP: handled by finish kernel
     } else {
         // finished earlier (getSubset failure / table exhausted), or the adaptive stop is behind us
-        if (n <= 4 || w.smp_state[2 * set + 1] < 0 || w.n_samples[set] < round_base || round_base >= w.niters_cur[set]) return;
+        if (n <= MP || w.smp_state[2 * set + 1] < 0 || w.n_samples[set] < round_base || round_base >= w.niters_cur[set]) return;
     }
     const float4* __restrict__ pts = w.pts + w.starts[set];
     __shared__ float4 spts[SMEM_PTS];
@@ -134,17 +139,20 @@ ransac_sample_kernel(RansacWork w, int round_base, int round_end, const int* __r
         #pragma unroll 1
         for (int k = 0; k < SW_PER_THREAD; k++) {
             const int o = k * SMP_THREADS + threadIdx.x;
-            int idx[4];
-            const int cons = draw_subset_g(get, base + o, idx);
+            int idx[MP];
+            const int cons = draw_subset_g<MP>(get, base + o, idx);
             uint16_t e = 0;
             if (cons > 0 && cons < 0x7fff) {
-                float ms1[8], ms2[8];
+                float ms1[2 * MP], ms2[2 * MP];
                 #pragma unroll
-                for (int i = 0; i < 4; i++) {
+                for (int i = 0; i < MP; i++) {
                     const float4 q = staged ? spts[idx[i]] : pts[idx[i]];
                     ms1[2 * i] = q.x; ms1[2 * i + 1] = q.y; ms2[2 * i] = q.z; ms2[2 * i + 1] = q.w;
                 }
-                e = (uint16_t)(cons | (check_subset4(ms1, ms2) ? 0x8000 : 0));
+                bool ok;
+                if constexpr (MP == 4) ok = check_subset4(ms1, ms2);
+                else ok = check_subset_affine(ms1, ms2);
+                e = (uint16_t)(cons | (ok ? 0x8000 : 0));
             }
             info[o] = e;
             const int c = e & 0x7fff;
@@ -154,7 +162,7 @@ ransac_sample_kernel(RansacWork w, int round_base, int round_end, const int* __r
         __syncthreads();
         int cur = 0;
         #pragma unroll 1
-        for (int r = 0; r < SW_ROUNDS; r++) {         // reach = { next^i(0) : i < 2^(r+1) }
+        for (int r = 0; r < ROUNDS; r++) {            // reach = { next^i(0) : i < 2^(r+1) }
             #pragma unroll
             for (int k = 0; k < SW_PER_THREAD; k++) {
                 const int o = k * SMP_THREADS + threadIdx.x;
@@ -927,15 +935,16 @@ ransac_score_kernel(RansacWork w, int round_base, int round_len, int n_slices, i
 }
 
 // ---- 3. select kernel: the serial scan of RANSACPointSetRegistrator::run --------------------------
-// cv::RANSACUpdateNumIters(confidence, (double)(n - good) / n, 4, niters) for the whole warp (same arguments in every lane).
-// log(1 - confidence) comes from the host; log(1 - (1 - ep)^4) comes from the host-verified table when the pair is listed,
+// cv::RANSACUpdateNumIters(confidence, (double)(n - good) / n, mp, niters) for the whole warp (same arguments in every lane),
+// mp = w.model_points.
+// log(1 - confidence) comes from the host; log(1 - (1 - ep)^mp) comes from the host-verified table when the entry is listed,
 // else from CUDA's log / pow with a check that neither the cap comparison nor cvRound is within nit_margin of flipping
 // (then the pair is sent to the host and the call repeats the verify stage, see run_ransac in api.cu).
 __device__ int update_num_iters_checked(const RansacWork& w, int n, int good, int niters, int lane)
 {
     int found = -1;
     for (int i = lane; i < w.nit_n; i += 32)
-        if (w.nit_tab[i].n == n && w.nit_tab[i].good == good) found = i;
+        if (w.nit_tab[i].n == n && w.nit_tab[i].good == good && w.nit_tab[i].mp == w.model_points) found = i;
     #pragma unroll
     for (int o = 16; o > 0; o >>= 1) found = max(found, __shfl_xor_sync(0xffffffffu, found, o));
     double ep = (double)(n - good) / n;
@@ -944,7 +953,7 @@ __device__ int update_num_iters_checked(const RansacWork& w, int n, int good, in
     double denom; bool zero;
     if (found >= 0) { denom = w.nit_tab[found].denom_log; zero = w.nit_tab[found].zero != 0; }
     else {
-        const double d0 = 1. - pow(1. - ep, 4.0);
+        const double d0 = 1. - (w.model_points == 4 ? pow(1. - ep, 4.0) : pow(1. - ep, 3.0));
         zero = d0 < DBL_MIN;
         denom = zero ? -1. : log(d0);
     }
@@ -953,7 +962,7 @@ __device__ int update_num_iters_checked(const RansacWork& w, int n, int good, in
     else if (denom >= 0 || -num >= niters * (-denom)) result = niters;
     else result = (int)rint(num / denom);            // cvRound: round half to even
     if (found < 0 && w.nit_req) {
-        bool unsure = zero || !(denom < 0);           // never reached with good >= 4; let the host decide if it is
+        bool unsure = zero || !(denom < 0);           // never reached with good >= mp; let the host decide if it is
         if (!unsure) {
             // q >= niters: the cap wins and nothing is rounded; only a quotient within the margin of the cap, or — below the
             // cap — within the margin of a half-integer, could come out differently with the host's log / pow
@@ -980,6 +989,7 @@ __global__ void ransac_select_kernel(RansacWork w, int round_base, int round_len
     const int32_t* __restrict__ counts = w.counts + (size_t)set * w.max_iters;
     int niters = w.niters_cur[set];
     int best = w.best_count[set], best_iter = w.best_iter[set];
+    const int floor_good = w.model_points - 1;                     // good > max(best, modelPoints - 1)
     int base = round_base;
     const int end = min(round_base + round_len, n_samples);
     while (base < niters && base < end) {
@@ -987,7 +997,7 @@ __global__ void ransac_select_kernel(RansacWork w, int round_base, int round_len
         const int c = (it < end) ? counts[it] : -1;
         int start = 0;
         for (;;) {
-            const bool cand = lane >= start && it < niters && it < end && c > max(best, 3);
+            const bool cand = lane >= start && it < niters && it < end && c > max(best, floor_good);
             const unsigned bal = __ballot_sync(0xffffffffu, cand);
             if (!bal) break;
             const int f = __ffs(bal) - 1;
@@ -1004,12 +1014,12 @@ __global__ void ransac_select_kernel(RansacWork w, int round_base, int round_len
         w.best_count[set] = best;
         w.niters_cur[set] = niters;
         // value of `iter` when the reference loop exits
-        w.iters_run[set] = n <= 4 ? 0 : min(max(niters, best_iter + 1), n_samples);
+        w.iters_run[set] = n <= w.model_points ? 0 : min(max(niters, best_iter + 1), n_samples);
     }
 }
 
 // Without the adaptive stop (CVG_RANSAC_NO_EARLY_STOP) niters never changes, so the serial scan reduces to "first
-// iteration with the largest count, if it beats the running best and 3": a block-wide argmax, one CTA per set.
+// iteration with the largest count, if it beats the running best and modelPoints - 1": a block-wide argmax, one CTA per set.
 constexpr int SELP_THREADS = 256;
 __global__ void __launch_bounds__(SELP_THREADS)
 ransac_select_all_kernel(RansacWork w, int round_base, int round_len)
@@ -1035,11 +1045,11 @@ ransac_select_all_kernel(RansacWork w, int round_base, int round_len)
         int bc = w.best_count[set], bi = w.best_iter[set];
         if (best >= 0) {
             const int c = (int)(best >> 32), it = 0x7fffffff - (int)(unsigned int)best;
-            if (c > max(bc, 3)) { bc = c; bi = it; }
+            if (c > max(bc, w.model_points - 1)) { bc = c; bi = it; }
         }
         w.best_count[set] = bc; w.best_iter[set] = bi;
         const int niters = w.niters_cur[set];
-        w.iters_run[set] = n <= 4 ? 0 : min(max(niters, bi + 1), n_samples);
+        w.iters_run[set] = n <= w.model_points ? 0 : min(max(niters, bi + 1), n_samples);
     }
 }
 
@@ -1769,10 +1779,10 @@ int launch_ransac_sample(const RansacWork& w, int rb, int len, cudaStream_t st)
                                                                         w.chunk_offsets, w.chunk_serial);
         ransac_sample_scatter_kernel<<<dim3((unsigned)w.n_chunks, (unsigned)w.n_sets), 256, 0, st>>>(w, rb + len, w.n_chunks, outs,
                                                                                                  w.chunk_lists, w.chunk_offsets);
-        ransac_sample_kernel<<<w.n_sets, SMP_THREADS, 0, st>>>(w, rb, rb + len, w.chunk_serial);   // sets the stitch rejected
+        ransac_sample_kernel<4><<<w.n_sets, SMP_THREADS, 0, st>>>(w, rb, rb + len, w.chunk_serial);   // sets the stitch rejected
         return 6;
     }
-    ransac_sample_kernel<<<w.n_sets, SMP_THREADS, 0, st>>>(w, rb, rb + len, nullptr);
+    ransac_sample_kernel<4><<<w.n_sets, SMP_THREADS, 0, st>>>(w, rb, rb + len, nullptr);
     return 1;
 }
 
@@ -1857,6 +1867,300 @@ int launch_ransac(const RansacWork& w, cudaStream_t st, cudaEvent_t* hyp_events,
     }
     launches += launch_ransac_finish(w, hyp_complete, st);
     return launches;
+}
+
+// ---- cv::estimateAffine2D(RANSAC): solve + score, finish -------------------------------------------
+// The affine path shares the sampler (ransac_sample_kernel<3>), the select scan and the niters verification with
+// findHomography.  Its minimal solve is a closed form of ~40 fp64 operations, so one kernel solves and scores: a CTA is
+// SCORE_THREADS consecutive iterations of one set x one slice of its correspondences (blockIdx.z), as in
+// ransac_score_kernel; every thread re-solves its hypothesis from the sample (cheaper than a round trip through HBM) and
+// adds its slice's count to counts[] (zeroed before the launch) with an integer atomicAdd.
+__device__ __forceinline__ void affine_solve_sample(const RansacWork& w, const float4* __restrict__ pts, int n, int32_t pos,
+                                                    double M[6])
+{
+    int idx[3];
+    draw_subset_g<3>(TabGet{ w.rng_tab, w.rng_len, (uint32_t)n }, pos, idx);
+    float ms1[6], ms2[6];
+    #pragma unroll
+    for (int i = 0; i < 3; i++) {
+        const float4 q = pts[idx[i]];
+        ms1[2 * i] = q.x; ms1[2 * i + 1] = q.y; ms2[2 * i] = q.z; ms2[2 * i + 1] = q.w;
+    }
+    affine_solve(ms1, ms2, M);
+}
+
+__global__ void __launch_bounds__(SCORE_THREADS)
+ransac_affine_hyp_kernel(RansacWork w, int round_base, int round_len, int n_slices, int tiles)
+{
+    __shared__ float4 stage[SCORE_STAGE];
+    const int set = (int)(blockIdx.x / (unsigned)tiles);
+    const int r = (int)(blockIdx.x % (unsigned)tiles) * SCORE_THREADS + threadIdx.x;
+    const int iter = round_base + r;
+    const int n = w.counts_n[set];
+    const size_t slot = (size_t)set * w.max_iters + iter;
+    const bool live = r < round_len && iter < w.n_samples[set] && iter < w.niters_cur[set];
+    if (!__syncthreads_or(live)) return;
+    const float4* __restrict__ ps = w.pts + w.starts[set];
+    float F[6];
+    {
+        double M[6];
+        if (live) affine_solve_sample(w, ps, n, w.sample_pos[slot], M);
+        #pragma unroll
+        for (int i = 0; i < 6; i++) F[i] = live ? (float)M[i] : 0.f;
+    }
+    const int per = (n + n_slices - 1) / n_slices;
+    const int p0 = min(n, (int)blockIdx.z * per), p1 = min(n, p0 + per);
+    const float thr2 = w.thr2;
+    int cnt = 0;
+    for (int base = p0; base < p1; base += SCORE_STAGE) {
+        const int m = min(SCORE_STAGE, p1 - base);
+        __syncthreads();
+        for (int i = threadIdx.x; i < m; i += SCORE_THREADS) stage[i] = ps[base + i];
+        __syncthreads();
+        if (live) {
+            #pragma unroll 4
+            for (int i = 0; i < m; i++) {
+                const float4 q = stage[i];                              // same address in every lane: broadcast
+                cnt += affine_err(F, q.x, q.y, q.z, q.w) <= thr2 ? 1 : 0;   // NaN -> not an inlier
+            }
+        }
+    }
+    if (live && cnt) atomicAdd(&w.counts[slot], cnt);
+}
+
+struct AffineShared {
+    double part[(RS_THREADS / 32) * 28];
+    double out[29];
+    LmStateN<6> lm;
+    double scratch_a[36], scratch_v[36];
+    double r[2 * EXACT_MAX_INLIERS];            // exact mode: residuals of the current evaluation
+    int flag;
+    int warp_cnt[RS_THREADS / 32];
+    int base_cnt;
+};
+
+// Jacobian entry (row, j) of Affine2DRefineCallback: row 2i is (X, Y, 1, 0, 0, 0), row 2i + 1 is (0, 0, 0, X, Y, 1)
+__device__ __forceinline__ double affine_jac(int row, int j, const float4& q)
+{
+    const int c = j - 3 * (row & 1);
+    return c == 0 ? (double)q.x : c == 1 ? (double)q.y : c == 2 ? 1.0 : 0.0;
+}
+
+// At x (wantJ): S = |r|^2, max |r|, A = J^T J (6 x 6) and v = J^T r, left in st.  At xd: Sd = |r|^2 in sh.out[0].  Up to
+// EXACT_MAX_INLIERS inliers every sum is one thread's, in OpenCV's order (mulTransposed sequential over rows, gemm with
+// 4 interleaved accumulators below 100 rows, norm in the AVX2 pattern); above, per-thread partial sums and block_sum.
+__device__ void affine_lm_eval(const float4* __restrict__ pts, const int32_t* __restrict__ sel, int count, const double* h,
+                               bool wantJ, AffineShared& sh)
+{
+    const int tid = threadIdx.x;
+    double S, rm, A[21], v[6];
+    if (count <= EXACT_MAX_INLIERS) {
+        const int rows = 2 * count;
+        for (int i = tid; i < count; i += (int)blockDim.x) {
+            const float4 q = pts[sel[i]];
+            const double Mx = q.x, My = q.y;
+            sh.r[2 * i] = h[0] * Mx + h[1] * My + h[2] - q.z;
+            sh.r[2 * i + 1] = h[3] * Mx + h[4] * My + h[5] - q.w;
+        }
+        __syncthreads();
+        if (wantJ && tid < 21) {                                 // upper triangle entry (j, k) of J^T J
+            int j = 0, e = tid;
+            while (e >= 6 - j) { e -= 6 - j; j++; }
+            const int k = j + e;
+            double s = 0;
+            for (int row = 0; row < rows; row++) {
+                const float4 q = pts[sel[row >> 1]];
+                s += affine_jac(row, j, q) * affine_jac(row, k, q);
+            }
+            sh.out[tid] = s;
+        } else if (wantJ && tid >= 21 && tid < 27) {             // J^T r entry
+            const int j = tid - 21;
+            double s;
+            if (rows < 100) {
+                double s4[4] = { 0, 0, 0, 0 };
+                const int full = rows & ~3;
+                for (int row = 0; row < rows; row++)
+                    s4[row < full ? (row & 3) : 0] += affine_jac(row, j, pts[sel[row >> 1]]) * sh.r[row];
+                s = ((s4[0] + s4[1]) + s4[2]) + s4[3];
+            } else {
+                s = 0;
+                for (int row = 0; row < rows; row++) s += affine_jac(row, j, pts[sel[row >> 1]]) * sh.r[row];
+            }
+            sh.out[21 + j] = s;
+        } else if (tid == 27) {
+            NormL2SqrAcc na; na.init();
+            for (int row = 0; row < rows; row++) na.push(sh.r[row]);
+            sh.out[27] = na.finish();
+        } else if (tid == 28) {
+            double m = 0;
+            for (int row = 0; row < rows; row++) { const double q = fabs(sh.r[row]); if (q > m) m = q; }
+            sh.out[28] = m;
+        }
+        __syncthreads();
+        S = sh.out[27]; rm = sh.out[28];
+        if (wantJ) {
+            for (int e = 0; e < 21; e++) A[e] = sh.out[e];
+            for (int j = 0; j < 6; j++) v[j] = sh.out[21 + j];
+        }
+        __syncthreads();
+    } else {
+        double acc[28];
+        #pragma unroll
+        for (int k = 0; k < 28; k++) acc[k] = 0;
+        rm = 0;
+        // 64 partial sums whatever blockDim.x (64 or 128, chosen from the batch's largest set): threads 64.. add exact
+        // zeros, so a set's M does not depend on the batch it came in
+        for (int i = tid; tid < 64 && i < count; i += 64) {
+            const float4 q = pts[sel[i]];
+            const double Mx = q.x, My = q.y;
+            const double r0 = h[0] * Mx + h[1] * My + h[2] - q.z;
+            const double r1 = h[3] * Mx + h[4] * My + h[5] - q.w;
+            acc[27] += r0 * r0; acc[27] += r1 * r1;
+            rm = fmax(rm, fmax(fabs(r0), fabs(r1)));
+            if (wantJ) {
+                int e = 0;
+                #pragma unroll
+                for (int j = 0; j < 6; j++) {
+                    #pragma unroll
+                    for (int k = j; k < 6; k++) {
+                        acc[e] += affine_jac(0, j, q) * affine_jac(0, k, q); acc[e] += affine_jac(1, j, q) * affine_jac(1, k, q); e++;
+                    }
+                    acc[21 + j] += affine_jac(0, j, q) * r0; acc[21 + j] += affine_jac(1, j, q) * r1;
+                }
+            }
+        }
+        block_sum<28>(acc, sh.part, sh.out);
+        #pragma unroll
+        for (int o = 16; o > 0; o >>= 1) rm = fmax(rm, shfl_down_d(rm, o));
+        if ((tid & 31) == 0) sh.part[tid >> 5] = rm;
+        __syncthreads();
+        rm = sh.part[0];
+        for (int q = 1; q < (int)(blockDim.x >> 5); q++) rm = fmax(rm, sh.part[q]);
+        __syncthreads();
+        S = acc[27];
+        for (int e = 0; e < 21; e++) A[e] = acc[e];
+        for (int j = 0; j < 6; j++) v[j] = acc[21 + j];
+    }
+    if (tid == 0) {
+        LmStateN<6>& st = sh.lm;
+        if (wantJ) {
+            int e = 0;
+            for (int j = 0; j < 6; j++) {
+                for (int k = j; k < 6; k++) { st.A[j * 6 + k] = A[e]; st.A[k * 6 + j] = A[e]; e++; }
+                st.v[j] = v[j];
+            }
+            st.S = S; st.rmax = rm;
+        } else {
+            sh.out[0] = S;                                       // Sd, read by thread 0 after the barrier below
+        }
+    }
+    __syncthreads();
+}
+
+// One CTA per set: the winner re-solved in fp64, the returned mask from (float)M (RANSAC stage: the refine moves M, not the
+// mask), the ordered compaction of its inliers and LMSolver with Affine2DRefineCallback for refine_iters iterations.
+__global__ void __launch_bounds__(RS_THREADS)
+ransac_affine_finish_kernel(RansacWork w, int refine_iters)
+{
+    const int set = blockIdx.x;
+    const int n = w.counts_n[set];
+    const int64_t start = w.starts[set];
+    const float4* __restrict__ pts = w.pts + start;
+    uint8_t* mask = w.mask + start;
+    int32_t* sel = w.sel + start;
+    double* Mout = w.H + (size_t)set * 6;
+    __shared__ AffineShared sh;
+    LmStateN<6>& st = sh.lm;
+    const int tid = threadIdx.x;
+    if (n < 3 || (n > 3 && w.best_iter[set] < 0)) {             // cv2 returns an empty matrix
+        for (int i = tid; i < n; i += (int)blockDim.x) mask[i] = 0;
+        if (tid < 6) Mout[tid] = 0.0;
+        if (tid == 0) w.found[set] = 0;
+        return;
+    }
+    if (n == 3) {                                                // count == modelPoints: the closed form, mask 1,1,1, no refine
+        if (tid == 0) {
+            float ms1[6], ms2[6];
+            for (int i = 0; i < 3; i++) { ms1[2 * i] = pts[i].x; ms1[2 * i + 1] = pts[i].y; ms2[2 * i] = pts[i].z; ms2[2 * i + 1] = pts[i].w; }
+            double M[6];
+            affine_solve(ms1, ms2, M);
+            for (int i = 0; i < 6; i++) Mout[i] = M[i];
+            w.found[set] = 1;
+        }
+        if (tid < 3) mask[tid] = 1;
+        return;
+    }
+    if (tid == 0) {
+        affine_solve_sample(w, pts, n, w.sample_pos[(size_t)set * w.max_iters + w.best_iter[set]], st.x);
+        sh.base_cnt = 0;
+    }
+    __syncthreads();
+    float F[6];
+    #pragma unroll
+    for (int i = 0; i < 6; i++) F[i] = (float)st.x[i];
+    const int lane = tid & 31, wid = tid >> 5;
+    for (int base = 0; base < n; base += (int)blockDim.x) {       // mask + ordered compaction of the inlier indices
+        const int i = base + tid;
+        bool in = false;
+        if (i < n) {
+            const float4 q = pts[i];
+            in = affine_err(F, q.x, q.y, q.z, q.w) <= w.thr2;
+            mask[i] = in ? 1 : 0;
+        }
+        const unsigned bal = __ballot_sync(0xffffffffu, in);
+        if (lane == 0) sh.warp_cnt[wid] = __popc(bal);
+        __syncthreads();
+        int off = sh.base_cnt;
+        for (int k = 0; k < wid; k++) off += sh.warp_cnt[k];
+        if (in) sel[off + __popc(bal & ((1u << lane) - 1))] = i;
+        __syncthreads();
+        if (tid == 0) { int t = 0; for (int k = 0; k < (int)(blockDim.x >> 5); k++) t += sh.warp_cnt[k]; sh.base_cnt += t; }
+        __syncthreads();
+    }
+    const int n_inl = sh.base_cnt;
+    if (refine_iters > 0 && n_inl > 0) {
+        affine_lm_eval(pts, sel, n_inl, st.x, true, sh);
+        if (tid == 0) lm_begin(st);
+        for (;;) {
+            if (tid == 0) lm_step(st, sh.scratch_a, sh.scratch_v);
+            __syncthreads();
+            affine_lm_eval(pts, sel, n_inl, st.xd, false, sh);
+            if (tid == 0) sh.flag = lm_update(st, sh.out[0], sh.scratch_a, sh.scratch_v) ? 1 : 0;
+            __syncthreads();
+            if (sh.flag) {                                       // accepted: x = xd, A, v, S, rmax at x
+                if (tid == 0) for (int i = 0; i < 6; i++) st.x[i] = st.xd[i];
+                __syncthreads();
+                affine_lm_eval(pts, sel, n_inl, st.x, true, sh);
+            }
+            if (tid == 0) sh.flag = lm_proceed(st, refine_iters) ? 1 : 0;
+            __syncthreads();
+            if (!sh.flag) break;
+        }
+    }
+    if (tid < 6) Mout[tid] = st.x[tid];
+    if (tid == 0) w.found[set] = 1;
+}
+
+int launch_affine(const RansacWork& w, int refine_iters, cudaStream_t st)
+{
+    if (w.n_sets <= 0) return 0;
+    const int round_len = ransac_round_len(w);
+    const int n_sms = w.n_sms > 0 ? w.n_sms : 148;
+    int launches = 0;
+    for (int rb = 0; rb < w.max_iters; rb += round_len) {
+        const int len = w.max_iters - rb < round_len ? w.max_iters - rb : round_len;
+        ransac_sample_kernel<3><<<w.n_sets, SMP_THREADS, 0, st>>>(w, rb, rb + len, nullptr);
+        cudaMemset2DAsync(w.counts + rb, (size_t)w.max_iters * 4, 0, (size_t)len * 4, (size_t)w.n_sets, st);
+        // slices of the correspondences so that the launch holds >= ~6 CTAs per SM (or one slice per 512 points)
+        const int tiles = (len + SCORE_THREADS - 1) / SCORE_THREADS;
+        const int64_t ctas = (int64_t)tiles * w.n_sets;
+        int n_slices = (int)std::min<int64_t>(std::max<int64_t>(1, ((int64_t)n_sms * 6 + ctas - 1) / ctas), std::max(1, w.max_n / 512));
+        n_slices = std::max(1, std::min(n_slices, 64));
+        ransac_affine_hyp_kernel<<<dim3((unsigned)ctas, 1, (unsigned)n_slices), SCORE_THREADS, 0, st>>>(w, rb, len, n_slices, tiles);
+        launches += 2 + launch_ransac_select(w, rb, len, st);
+    }
+    ransac_affine_finish_kernel<<<w.n_sets, w.max_n <= 512 ? 64 : RS_THREADS, 0, st>>>(w, refine_iters);
+    return launches + 1;
 }
 
 // ---- gates + inlier gather: reference src/TestsDetector.cpp:74-94 ---------------------------------

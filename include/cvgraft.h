@@ -86,6 +86,17 @@ typedef struct cvg_ransac_params {
     int32_t reserved;
 } cvg_ransac_params;
 
+/* estimateAffine2D(..., RANSAC, threshold, maxIters, confidence, refineIters) — OpenCV's defaults are
+ * 3.0, 2000, 0.99, 10 (cvg_affine_params_default).  flags: CVG_RANSAC_NO_EARLY_STOP or 0. */
+typedef struct cvg_affine_params {
+    uint32_t size;                  /* = sizeof(cvg_affine_params)                                   */
+    uint32_t flags;
+    double threshold;               /* ransacReprojThreshold, compared as (float)(t*t) with the error */
+    double confidence;
+    int32_t max_iters;              /* [1, 2^24]                                                     */
+    int32_t refine_iters;           /* LM iterations on the inliers, [0, 1000]; 0 = none             */
+} cvg_affine_params;
+
 /* constants of detectObjects() — src/TestsDetector.cpp:21-25 */
 typedef struct cvg_detect_params {
     uint32_t size;                  /* = sizeof(cvg_detect_params)                                   */
@@ -108,6 +119,7 @@ typedef struct cvg_pair_result {
 
 void cvg_ransac_params_default(cvg_ransac_params* p);
 void cvg_detect_params_default(cvg_detect_params* p);
+void cvg_affine_params_default(cvg_affine_params* p);
 
 /* ---- context -------------------------------------------------------------------------------- */
 int  cvg_create(cvg_ctx** out, int device, unsigned flags);
@@ -119,8 +131,8 @@ int  cvg_create(cvg_ctx** out, int device, unsigned flags);
  * pair sharding of the loop nest of src/TestsDetector.cpp:38,58,99 under src/Output.cpp:23-57, no data-path
  * collective; cvg_match_knn2_sharded is the train-tile sharded match with its one all-gather, and
  * cvg_find_homography_sharded splits the hypotheses of one RANSAC over the GPUs with one all-gather of counts per
- * round.  The other entry points (cvg_match_knn2, cvg_find_homography, cvg_find_homography_batch, cvg_detect_pairs,
- * cvg_dev_*) run on the first listed GPU.
+ * round.  The other entry points (cvg_match_knn2, cvg_find_homography, cvg_find_homography_batch,
+ * cvg_estimate_affine2d, cvg_estimate_affine2d_batch, cvg_detect_pairs, cvg_dev_*) run on the first listed GPU.
  * A device may be listed more than once (logical shards on one GPU, used by the single-GPU tests); NCCL refuses
  * such a communicator, so the exchange then runs as device-to-device copies (cvg_exchange_kind: "memcpy"). */
 int  cvg_create_multi(cvg_ctx** out, const int* devices, int n_devices, unsigned flags);
@@ -185,6 +197,23 @@ int  cvg_find_homography_batch(cvg_ctx* ctx, const float* src_xy, const float* d
                                const int64_t* offsets, int n_sets, const cvg_ransac_params* p,
                                double* H /*[P,9]*/, uint8_t* mask, int32_t* found /*[P]*/,
                                int32_t* iters /*[P]*/, uint8_t* ransac_mask);
+
+/* cv::estimateAffine2D(src, dst, inliers, RANSAC, p->threshold, p->max_iters, p->confidence, p->refine_iters):
+ * the 2x3 affine map of src onto dst.  M gets the row-major 2x3 CV_64F result (zeros if none), mask [n] the returned
+ * inlier mask, *found = 0 iff OpenCV returns an empty matrix.  As in OpenCV the mask is that of the winning RANSAC
+ * hypothesis: the Levenberg-Marquardt refine on its inliers moves M, not the mask.  n = 3 returns the exact fit of the
+ * three points with mask 1,1,1 (OpenCV does not refine it); n = 1 or 2 returns found = 0 and a zero mask; n = 0 ->
+ * CVG_ERR_TOO_FEW_POINTS (OpenCV fails an assertion).  Flags other than CVG_RANSAC_NO_EARLY_STOP -> CVG_ERR_INVALID,
+ * refine_iters outside [0, 1000] -> CVG_ERR_LIMIT.  On a cvg_create_multi context it runs on the first GPU. */
+int  cvg_estimate_affine2d(cvg_ctx* ctx, const float* src_xy, const float* dst_xy, int n,
+                           const cvg_affine_params* p, double M[6], uint8_t* mask, int* found);
+
+/* Batched form: P independent point sets, set k = rows [offsets[k], offsets[k+1]) of src/dst, each with the semantics
+ * above (sets of fewer than 3 points report found = 0).  iters (may be NULL) [P] = RANSAC iterations. */
+int  cvg_estimate_affine2d_batch(cvg_ctx* ctx, const float* src_xy, const float* dst_xy,
+                                 const int64_t* offsets, int n_sets, const cvg_affine_params* p,
+                                 double* M /*[P,6]*/, uint8_t* mask, int32_t* found /*[P]*/,
+                                 int32_t* iters /*[P]*/);
 
 /* ---- fused path: replaces the body of the view loop, src/TestsDetector.cpp:58-95 -------------
  * All views of the resident model set against one scene (descriptors [n_train,128] + keypoints
@@ -298,7 +327,8 @@ int  cvg_last_match_fallback_rows(const cvg_ctx* ctx);
 int  cvg_last_match_guard_rows(const cvg_ctx* ctx);
 /* Verify calls with CVG_RANSAC_NO_EARLY_STOP and max_iters >= 32768 cut every set's cv::RNG draw stream into
  * chunks walked by many CTAs (same samples as the serial walk).  Returns how many sets of the last such call
- * were handed back to the one-CTA-per-set sampler, or -1 if the last verify call did not use the chunked sampler. */
+ * were handed back to the one-CTA-per-set sampler, or -1 if the last verify call did not use the chunked sampler
+ * (estimateAffine2D calls never do). */
 int  cvg_last_sampler_serial_sets(const cvg_ctx* ctx);
 /* The context's cudaStream_t (all of its GPU work is issued there); lets a harness record its own
  * CUDA events around calls. */
