@@ -59,6 +59,8 @@ SYMBOLS = {
     "cvg_find_homography_batch": (C.c_int, [_P, _P, _P, _P, C.c_int, C.POINTER(RansacParams), _P, _P, _P, _P, _P]),
     "cvg_estimate_affine2d": (C.c_int, [_P, _P, _P, C.c_int, C.POINTER(AffineParams), _P, _P, C.POINTER(C.c_int)]),
     "cvg_estimate_affine2d_batch": (C.c_int, [_P, _P, _P, _P, C.c_int, C.POINTER(AffineParams), _P, _P, _P, _P]),
+    "cvg_estimate_affine_partial2d": (C.c_int, [_P, _P, _P, C.c_int, C.POINTER(AffineParams), _P, _P, C.POINTER(C.c_int)]),
+    "cvg_estimate_affine_partial2d_batch": (C.c_int, [_P, _P, _P, _P, C.c_int, C.POINTER(AffineParams), _P, _P, _P, _P]),
     "cvg_detect_pairs": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_float, C.POINTER(DetectParams), _P, _P, _P]),
     "cvg_scenes_upload": (C.c_int, [_P, _P, _P, _P, C.c_int, C.POINTER(_P)]),
     "cvg_scenes_free": (None, [_P, _P]),

@@ -3,7 +3,8 @@
     Context.match_knn2        <- cv::BFMatcher(NORM_L2).knnMatch(q, t, 2) + ratio test
                                  reference src/TestsDetector.cpp:59-72
     Context.find_homography   <- cv::findHomography(src, dst, RANSAC, 5.0, mask)    :77-78
-    Context.estimate_affine2d <- cv::estimateAffine2D(src, dst, inliers, RANSAC)    (the other geometric check)
+    Context.estimate_affine2d <- cv::estimateAffine2D(src, dst, inliers, RANSAC)    (the other geometric checks)
+    Context.estimate_affine_partial2d <- cv::estimateAffinePartial2D(src, dst, inliers, RANSAC)
     Context.detect_pairs      <- body of the view loop of detectAtScale             :58-95
     Models                    <- ObjectModel descriptors resident in HBM            include/objectModel.hpp:11-16
 
@@ -53,7 +54,8 @@ def ransac_params(threshold=5.0, max_iters=2000, confidence=0.995, flags=0):
 
 
 def affine_params(threshold=3.0, max_iters=2000, confidence=0.99, refine_iters=10, flags=0):
-    """cv2.estimateAffine2D's ransacReprojThreshold, maxIters, confidence, refineIters (OpenCV's defaults)."""
+    """cv2.estimateAffine2D's / estimateAffinePartial2D's ransacReprojThreshold, maxIters, confidence, refineIters
+    (OpenCV's defaults)."""
     p = AffineParams()
     _lib.load().cvg_affine_params_default(C.byref(p))
     p.threshold = threshold; p.max_iters = max_iters; p.confidence = confidence; p.refine_iters = refine_iters
@@ -312,32 +314,52 @@ class Context:
             out["ransac_mask"] = rmask[:s.shape[0]]
         return out
 
-    def estimate_affine2d(self, src, dst, threshold=3.0, max_iters=2000, confidence=0.99, refine_iters=10, flags=0):
-        """cv2.estimateAffine2D(src, dst, method=cv2.RANSAC, ransacReprojThreshold=, maxIters=, confidence=, refineIters=)
-        -> (M 2x3 or None, inlier mask uint8 [n]).  Raises for n = 0 like OpenCV."""
+    def _affine(self, fn, src, dst, threshold, max_iters, confidence, refine_iters, flags):
         s = _f32(src, 2); d = _f32(dst, 2)
         n = s.shape[0]
         if d.shape[0] != n:
             raise ValueError("src and dst must have the same number of points")
         M = np.zeros(6); mask = np.zeros(max(n, 1), np.uint8); found = C.c_int(0)
         p = affine_params(threshold, max_iters, confidence, refine_iters, flags)
-        self._check(self.lib.cvg_estimate_affine2d(self.handle, _ptr(s), _ptr(d), n, C.byref(p), _ptr(M), _ptr(mask),
-                                                   C.byref(found)))
+        self._check(fn(self.handle, _ptr(s), _ptr(d), n, C.byref(p), _ptr(M), _ptr(mask), C.byref(found)))
         return (M.reshape(2, 3) if found.value else None), mask[:n]
 
-    def estimate_affine2d_batch(self, src, dst, offsets, threshold=3.0, max_iters=2000, confidence=0.99, refine_iters=10,
-                                flags=0):
-        """estimate_affine2d for every set k = rows [offsets[k], offsets[k+1]) -> dict(M [P,2,3] (zeros where none),
-        mask, found [P] bool, iters [P] RANSAC iterations)."""
+    def _affine_batch(self, fn, src, dst, offsets, threshold, max_iters, confidence, refine_iters, flags):
         s = _f32(src, 2); d = _f32(dst, 2)
         off = np.ascontiguousarray(offsets, np.int64)
         P = len(off) - 1
         M = np.zeros((max(P, 1), 6)); mask = np.zeros(max(s.shape[0], 1), np.uint8)
         found = np.zeros(max(P, 1), np.int32); iters = np.zeros(max(P, 1), np.int32)
         p = affine_params(threshold, max_iters, confidence, refine_iters, flags)
-        self._check(self.lib.cvg_estimate_affine2d_batch(self.handle, _ptr(s), _ptr(d), _ptr(off), P, C.byref(p),
-                                                         _ptr(M), _ptr(mask), _ptr(found), _ptr(iters)))
+        self._check(fn(self.handle, _ptr(s), _ptr(d), _ptr(off), P, C.byref(p), _ptr(M), _ptr(mask), _ptr(found),
+                       _ptr(iters)))
         return {"M": M[:P].reshape(P, 2, 3), "mask": mask[:s.shape[0]], "found": found[:P].astype(bool), "iters": iters[:P]}
+
+    def estimate_affine2d(self, src, dst, threshold=3.0, max_iters=2000, confidence=0.99, refine_iters=10, flags=0):
+        """cv2.estimateAffine2D(src, dst, method=cv2.RANSAC, ransacReprojThreshold=, maxIters=, confidence=, refineIters=)
+        -> (M 2x3 or None, inlier mask uint8 [n]).  Raises for n = 0 like OpenCV."""
+        return self._affine(self.lib.cvg_estimate_affine2d, src, dst, threshold, max_iters, confidence, refine_iters, flags)
+
+    def estimate_affine2d_batch(self, src, dst, offsets, threshold=3.0, max_iters=2000, confidence=0.99, refine_iters=10,
+                                flags=0):
+        """estimate_affine2d for every set k = rows [offsets[k], offsets[k+1]) -> dict(M [P,2,3] (zeros where none),
+        mask, found [P] bool, iters [P] RANSAC iterations)."""
+        return self._affine_batch(self.lib.cvg_estimate_affine2d_batch, src, dst, offsets, threshold, max_iters, confidence,
+                                  refine_iters, flags)
+
+    def estimate_affine_partial2d(self, src, dst, threshold=3.0, max_iters=2000, confidence=0.99, refine_iters=10,
+                                  flags=0):
+        """cv2.estimateAffinePartial2D(src, dst, method=cv2.RANSAC, ...): the 4-DOF similarity [[a, -b, tx], [b, a, ty]]
+        -> (M 2x3 or None, inlier mask uint8 [n]).  Raises for n = 0 like OpenCV."""
+        return self._affine(self.lib.cvg_estimate_affine_partial2d, src, dst, threshold, max_iters, confidence,
+                            refine_iters, flags)
+
+    def estimate_affine_partial2d_batch(self, src, dst, offsets, threshold=3.0, max_iters=2000, confidence=0.99,
+                                        refine_iters=10, flags=0):
+        """estimate_affine_partial2d for every set k = rows [offsets[k], offsets[k+1]), with the outputs of
+        estimate_affine2d_batch."""
+        return self._affine_batch(self.lib.cvg_estimate_affine_partial2d_batch, src, dst, offsets, threshold, max_iters,
+                                  confidence, refine_iters, flags)
 
     # ---- fused path ----------------------------------------------------------------------------
     def detect_pairs(self, models, scene_desc, scene_kpt_xy, scale=1.0, params=None, want_inliers=True):

@@ -565,7 +565,7 @@ int eng_ransac_work(cvg_ctx* c, const float4* d_pts, const int64_t* d_starts, co
     w.max_iters = mi;
     w.model_points = model_points;
     c->nit_mp = model_points;
-    // findHomography replaces a threshold <= 0 by defaultRANSACReprojThreshold; estimateAffine2D squares what it is given
+    // findHomography replaces a threshold <= 0 by defaultRANSACReprojThreshold; the affine methods square what they are given
     const double thr = (p->threshold > 0 || model_points != 4) ? p->threshold : 3.0;
     w.thr2 = (float)(thr * thr);
     w.conf = p->confidence; w.flags = p->flags;
@@ -582,7 +582,7 @@ int eng_ransac_work(cvg_ctx* c, const float4* d_pts, const int64_t* d_starts, co
     w.chunk_outs = nullptr; w.chunk_lists = nullptr; w.chunk_offsets = nullptr; w.chunk_serial = nullptr; w.n_chunks = 0;
     w.chunk_maps = nullptr; w.chunk_entries = nullptr; w.chunk_serial_count = nullptr;
     c->last_chunked = false;
-    // (4-point draws only; estimateAffine2D calls run on the round sampler)
+    // (4-point draws only; the affine methods run on the round sampler)
     if (model_points == 4 && (p->flags & CVG_RANSAC_NO_EARLY_STOP) && mi >= 32768 && n_sets <= 65535) {     // sets ride on gridDim.y of the chunk kernels
         // one huge round: the draw stream of every set is walked by many CTAs at once (ransac_sample_chunk_kernel)
         const int n_chunks = ransac_chunks_for_table(c->rng_len);
@@ -866,9 +866,9 @@ int cvg_match_knn2_raw(cvg_ctx* c, const float* query, int n_query, const float*
 }
 
 // ---- verify stage ---------------------------------------------------------------------------------
-// One batched verify call: pack the sets, run the stage (findHomography for model_points 4, estimateAffine2D for 3), copy
-// the results back; repeat it with a longer cv::RNG draw table when a set ran out of draws, or after the host answered the
-// device's RANSACUpdateNumIters requests.  M gets m_doubles per set (9: H, 6: the 2x3 affine matrix).
+// One batched verify call: pack the sets, run the stage (findHomography for model_points 4, estimateAffine2D for 3,
+// estimateAffinePartial2D for 2), copy the results back; repeat it with a longer cv::RNG draw table when a set ran out of
+// draws, or after the host answered the device's RANSACUpdateNumIters requests.  M gets m_doubles per set (9: H, 6: the 2x3 affine matrix).
 static int verify_batch(cvg_ctx* c, const float* src_xy, const float* dst_xy, const int64_t* offsets, int n_sets,
                         const cvg_ransac_params* p, int model_points, int refine_iters, double* M, int m_doubles,
                         uint8_t* mask, int32_t* found, int32_t* iters, uint8_t* ransac_mask)
@@ -960,11 +960,13 @@ int cvg_find_homography(cvg_ctx* c, const float* src_xy, const float* dst_xy, in
     return rc;
 }
 
-int cvg_estimate_affine2d_batch(cvg_ctx* c, const float* src_xy, const float* dst_xy, const int64_t* offsets, int n_sets,
-                                const cvg_affine_params* p, double* M, uint8_t* mask, int32_t* found, int32_t* iters)
+// estimateAffine2D (model_points 3) and estimateAffinePartial2D (2): the cvg_affine_params checks, then one verify call
+static int affine_batch(cvg_ctx* c, const char* fn, const float* src_xy, const float* dst_xy, const int64_t* offsets,
+                        int n_sets, const cvg_affine_params* p, int model_points, double* M, uint8_t* mask, int32_t* found,
+                        int32_t* iters)
 {
     c = cvg_primary(c);
-    if (!c || !offsets || n_sets < 0) return set_err(CVG_ERR_INVALID, "cvg_estimate_affine2d_batch: bad argument");
+    if (!c || !offsets || n_sets < 0) return set_err(CVG_ERR_INVALID, "%s: bad argument", fn);
     if (!p || p->size != sizeof(cvg_affine_params)) return set_err(CVG_ERR_INVALID, "cvg_affine_params: bad size field");
     if (p->flags & ~CVG_RANSAC_NO_EARLY_STOP) return set_err(CVG_ERR_INVALID, "cvg_affine_params: unknown flags 0x%x", p->flags);
     if (p->refine_iters < 0 || p->refine_iters > 1000) return set_err(CVG_ERR_LIMIT, "refine_iters out of range [0, 1000]");
@@ -973,7 +975,14 @@ int cvg_estimate_affine2d_batch(cvg_ctx* c, const float* src_xy, const float* ds
     rp.flags = p->flags; rp.threshold = p->threshold; rp.confidence = p->confidence; rp.max_iters = p->max_iters;
     const int rc = check_params(&rp);
     if (rc) return rc;
-    return verify_batch(c, src_xy, dst_xy, offsets, n_sets, &rp, 3, p->refine_iters, M, 6, mask, found, iters, nullptr);
+    return verify_batch(c, src_xy, dst_xy, offsets, n_sets, &rp, model_points, p->refine_iters, M, 6, mask, found, iters,
+                        nullptr);
+}
+
+int cvg_estimate_affine2d_batch(cvg_ctx* c, const float* src_xy, const float* dst_xy, const int64_t* offsets, int n_sets,
+                                const cvg_affine_params* p, double* M, uint8_t* mask, int32_t* found, int32_t* iters)
+{
+    return affine_batch(c, "cvg_estimate_affine2d_batch", src_xy, dst_xy, offsets, n_sets, p, 3, M, mask, found, iters);
 }
 
 int cvg_estimate_affine2d(cvg_ctx* c, const float* src_xy, const float* dst_xy, int n, const cvg_affine_params* p,
@@ -983,6 +992,26 @@ int cvg_estimate_affine2d(cvg_ctx* c, const float* src_xy, const float* dst_xy, 
     const int64_t offs[2] = { 0, n };
     int32_t f = 0;
     const int rc = cvg_estimate_affine2d_batch(c, src_xy, dst_xy, offs, 1, p, M, mask, &f, nullptr);
+    if (found) *found = f;
+    return rc;
+}
+
+int cvg_estimate_affine_partial2d_batch(cvg_ctx* c, const float* src_xy, const float* dst_xy, const int64_t* offsets,
+                                        int n_sets, const cvg_affine_params* p, double* M, uint8_t* mask, int32_t* found,
+                                        int32_t* iters)
+{
+    return affine_batch(c, "cvg_estimate_affine_partial2d_batch", src_xy, dst_xy, offsets, n_sets, p, 2, M, mask, found,
+                        iters);
+}
+
+int cvg_estimate_affine_partial2d(cvg_ctx* c, const float* src_xy, const float* dst_xy, int n, const cvg_affine_params* p,
+                                  double M[6], uint8_t* mask, int* found)
+{
+    if (n <= 0)
+        return set_err(CVG_ERR_TOO_FEW_POINTS, "estimateAffinePartial2D needs at least one correspondence (got %d)", n);
+    const int64_t offs[2] = { 0, n };
+    int32_t f = 0;
+    const int rc = cvg_estimate_affine_partial2d_batch(c, src_xy, dst_xy, offs, 1, p, M, mask, &f, nullptr);
     if (found) *found = f;
     return rc;
 }

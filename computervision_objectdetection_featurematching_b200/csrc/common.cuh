@@ -113,7 +113,8 @@ void launch_shift_index(const int32_t* idx_in, const float* dist_in, int n_query
 // move cvRound(num / denom) when the quotient sits within ~1e-12 of a half-integer.  The device therefore uses the HOST's
 // log(1 - confidence), flags every evaluation whose rounding or cap decision is closer than `nit_margin` to a boundary, and
 // the host answers those (n, good) pairs with its own libm values; the verify stage is then repeated with the table.
-// An entry is keyed on (model points, n, good): homography (4) and estimateAffine2D (3) calls on one engine share its table.
+// An entry is keyed on (model points, n, good): homography (4), estimateAffine2D (3) and estimateAffinePartial2D (2) calls on
+// one engine share its table.
 struct NitEntry { int32_t n; int32_t good; double denom_log; int32_t zero; int32_t mp; };   // zero: 1 - (1-ep)^mp < DBL_MIN
 struct RansacWork {
     const float4* pts;          // correspondence pool, (X, Y, x, y)
@@ -143,7 +144,7 @@ struct RansacWork {
     int hyp_H_complete;         // every round's kernel left its models in hyp_H (set by launch_ransac for the finish kernel)
     int32_t* sel;               // [total] compacted inlier indices
     // outputs
-    double* H;                  // [P, 9] (estimateAffine2D: [P, 6])
+    double* H;                  // [P, 9] (the affine methods: [P, 6])
     uint8_t* mask;              // [total]
     uint8_t* ransac_mask;       // [total] or NULL
     int32_t* found;             // [P]
@@ -156,7 +157,7 @@ struct RansacWork {
     // chunked sampler scratch (huge single rounds; NULL / 0 = not available)
     void* chunk_outs; int32_t* chunk_lists; int32_t* chunk_offsets; int* chunk_serial; int n_chunks;
     uint8_t* chunk_maps; int32_t* chunk_entries; int* chunk_serial_count;
-    int model_points;           // RANSAC modelPoints: 4 findHomography, 3 estimateAffine2D
+    int model_points;           // RANSAC modelPoints: 4 findHomography, 3 estimateAffine2D, 2 estimateAffinePartial2D
 };
 int64_t ransac_chunk_scratch_bytes(int n_sets, int n_chunks, size_t* outs, size_t* lists, size_t* offsets, size_t* serial,
                                    size_t* maps, size_t* entries);
@@ -175,9 +176,10 @@ int  launch_ransac_sample(const RansacWork& w, int rb, int len, cudaStream_t st)
 int  launch_ransac_hyp(const RansacWork& w, int hb, int hlen, cudaStream_t st, const cudaEvent_t* ev, bool* hyp_complete);
 int  launch_ransac_select(const RansacWork& w, int rb, int len, cudaStream_t st);   // serial scan of round [rb, rb + len)
 int  launch_ransac_finish(const RansacWork& w, bool hyp_complete, cudaStream_t st);
-// cv::estimateAffine2D(RANSAC) for every set of w (w.model_points == 3): the round-based sampler, one solve-and-score kernel
-// per round, the select scan, then the finish kernel (winner's mask, compaction, 6-parameter LM of refine_iters iterations,
-// none for 0).  M goes to w.H as 6 doubles per set.  Returns the number of kernel launches.
+// cv::estimateAffine2D(RANSAC) (w.model_points == 3) or cv::estimateAffinePartial2D(RANSAC) (2) for every set of w: the
+// round-based sampler, one solve-and-score kernel per round, the select scan, then the finish kernel (winner's mask,
+// compaction, 6- or 4-parameter LM of refine_iters iterations, none for 0).  M goes to w.H as 6 doubles per set.  Returns
+// the number of kernel launches.
 int  launch_affine(const RansacWork& w, int refine_iters, cudaStream_t st);
 
 // detect glue (ransac.cu)

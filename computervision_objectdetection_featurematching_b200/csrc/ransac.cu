@@ -75,12 +75,14 @@ __device__ __forceinline__ int draw_subset(const uint32_t* __restrict__ tab, int
 // (ceil(log2(SW/MP)) doubling rounds: an attempt of an MP-point model consumes >= MP draws, so a window holds
 // <= SW/MP chain nodes), ranked by a block prefix sum, and the accepted ones become the samples of consecutive
 // iterations — the same order, rejected attempts and 10000-attempt limit as the serial loop.
-// MP = 4: findHomography (checkSubset: collinearity + orientation); MP = 3: estimateAffine2D (collinearity only).
+// MP = 4: findHomography (checkSubset: collinearity + orientation); MP = 3: estimateAffine2D (collinearity only);
+// MP = 2: estimateAffinePartial2D (collinearity of two points: always accepted).
 constexpr int SW = 2048;                          // measured: 512 -> 2048 halves the sampler time per draw (fewer serial windows)
 constexpr int SW_ROUNDS = 9;                      // log2(SW / 4): the 4-point chunked sampler below
 template <int MP> __host__ __device__ constexpr int sw_rounds() { int r = 0; while ((MP << r) < SW) r++; return r; }
 static_assert(sw_rounds<4>() == SW_ROUNDS && (4 << SW_ROUNDS) == SW, "pointer-jumping rounds must cover SW / 4 chain nodes");
 static_assert(sw_rounds<3>() == 10 && (3 << sw_rounds<3>()) >= SW, "pointer-jumping rounds must cover SW / 3 chain nodes");
+static_assert(sw_rounds<2>() == 10 && (2 << sw_rounds<2>()) >= SW, "pointer-jumping rounds must cover SW / 2 chain nodes");
 constexpr int SW_TAIL = 64;                       // draws staged beyond the window for attempts that start near its end
 constexpr int SMP_THREADS = 512;                  // one window offset per thread
 constexpr int SW_PER_THREAD = SW / SMP_THREADS;
@@ -151,7 +153,7 @@ ransac_sample_kernel(RansacWork w, int round_base, int round_end, const int* __r
                 }
                 bool ok;
                 if constexpr (MP == 4) ok = check_subset4(ms1, ms2);
-                else ok = check_subset_affine(ms1, ms2);
+                else ok = check_subset_affine<MP>(ms1, ms2);
                 e = (uint16_t)(cons | (ok ? 0x8000 : 0));
             }
             info[o] = e;
@@ -953,7 +955,8 @@ __device__ int update_num_iters_checked(const RansacWork& w, int n, int good, in
     double denom; bool zero;
     if (found >= 0) { denom = w.nit_tab[found].denom_log; zero = w.nit_tab[found].zero != 0; }
     else {
-        const double d0 = 1. - (w.model_points == 4 ? pow(1. - ep, 4.0) : pow(1. - ep, 3.0));
+        const double d0 = 1. - (w.model_points == 4 ? pow(1. - ep, 4.0) : w.model_points == 3 ? pow(1. - ep, 3.0)
+                                                                                                 : pow(1. - ep, 2.0));
         zero = d0 < DBL_MIN;
         denom = zero ? -1. : log(d0);
     }
@@ -1869,26 +1872,76 @@ int launch_ransac(const RansacWork& w, cudaStream_t st, cudaEvent_t* hyp_events,
     return launches;
 }
 
-// ---- cv::estimateAffine2D(RANSAC): solve + score, finish -------------------------------------------
-// The affine path shares the sampler (ransac_sample_kernel<3>), the select scan and the niters verification with
-// findHomography.  Its minimal solve is a closed form of ~40 fp64 operations, so one kernel solves and scores: a CTA is
-// SCORE_THREADS consecutive iterations of one set x one slice of its correspondences (blockIdx.z), as in
-// ransac_score_kernel; every thread re-solves its hypothesis from the sample (cheaper than a round trip through HBM) and
-// adds its slice's count to counts[] (zeroed before the launch) with an integer atomicAdd.
+// ---- cv::estimateAffine2D / estimateAffinePartial2D (RANSAC): solve + score, finish -------------------
+// The two affine methods share the sampler (ransac_sample_kernel<MP>), the select scan and the niters verification with
+// findHomography, and one pair of kernels below, instantiated for each model description (AffineModel, PartialModel).
+// A minimal solve is a closed form of ~40 fp64 operations, so one kernel solves and scores: a CTA is SCORE_THREADS
+// consecutive iterations of one set x one slice of its correspondences (blockIdx.z), as in ransac_score_kernel; every
+// thread re-solves its hypothesis from the sample (cheaper than a round trip through HBM) and adds its slice's count to
+// counts[] (zeroed before the launch) with an integer atomicAdd.
+//
+// A model description gives the sample size MP and the closed-form solve (2x3 M from MP points), the N parameters LMSolver
+// refines and their map to and from M, and the refine callback's residuals and Jacobian entries for one correspondence
+// q = (Mx, My, X, Y): row 2i is the x residual, row 2i + 1 the y residual.
+struct AffineModel {            // estimateAffine2D: Affine2DEstimatorCallback, Affine2DRefineCallback; x = M
+    static constexpr int MP = 3, N = 6;
+    __device__ static void solve(const float* from, const float* to, double* M) { affine_solve(from, to, M); }
+    __device__ static void params(const double* M, double* x) { for (int i = 0; i < 6; i++) x[i] = M[i]; }
+    __device__ static void matrix(const double* x, double* M) { for (int i = 0; i < 6; i++) M[i] = x[i]; }
+    __device__ static void residuals(const double* h, const float4& q, double& r0, double& r1)
+    {
+        const double Mx = q.x, My = q.y;
+        r0 = h[0] * Mx + h[1] * My + h[2] - q.z;
+        r1 = h[3] * Mx + h[4] * My + h[5] - q.w;
+    }
+    // row 2i is (X, Y, 1, 0, 0, 0), row 2i + 1 is (0, 0, 0, X, Y, 1)
+    __device__ static double jac(int row, int j, const float4& q)
+    {
+        const int c = j - 3 * (row & 1);
+        return c == 0 ? (double)q.x : c == 1 ? (double)q.y : c == 2 ? 1.0 : 0.0;
+    }
+};
+
+struct PartialModel {           // estimateAffinePartial2D: AffinePartial2DEstimatorCallback, AffinePartial2DRefineCallback
+    static constexpr int MP = 2, N = 4;
+    __device__ static void solve(const float* from, const float* to, double* M) { affine_partial_solve(from, to, M); }
+    // x = (a, b, tx, ty) = (M00, M10, M02, M12); M = [a, -b, tx; b, a, ty] (the solve's M maps back to itself, bit for bit)
+    __device__ static void params(const double* M, double* x) { x[0] = M[0]; x[1] = M[3]; x[2] = M[2]; x[3] = M[5]; }
+    __device__ static void matrix(const double* x, double* M)
+    {
+        M[0] = x[0]; M[1] = -x[1]; M[2] = x[2]; M[3] = x[1]; M[4] = x[0]; M[5] = x[3];
+    }
+    __device__ static void residuals(const double* h, const float4& q, double& r0, double& r1)
+    {
+        const double Mx = q.x, My = q.y;
+        r0 = h[0] * Mx - h[1] * My + h[2] - q.z;
+        r1 = h[1] * Mx + h[0] * My + h[3] - q.w;
+    }
+    // row 2i is (X, -Y, 1, 0), row 2i + 1 is (Y, X, 0, 1)
+    __device__ static double jac(int row, int j, const float4& q)
+    {
+        if (row & 1) return j == 0 ? (double)q.y : j == 1 ? (double)q.x : j == 2 ? 0.0 : 1.0;
+        return j == 0 ? (double)q.x : j == 1 ? -(double)q.y : j == 2 ? 1.0 : 0.0;
+    }
+};
+
+template <class Model>
 __device__ __forceinline__ void affine_solve_sample(const RansacWork& w, const float4* __restrict__ pts, int n, int32_t pos,
                                                     double M[6])
 {
-    int idx[3];
-    draw_subset_g<3>(TabGet{ w.rng_tab, w.rng_len, (uint32_t)n }, pos, idx);
-    float ms1[6], ms2[6];
+    constexpr int MP = Model::MP;
+    int idx[MP];
+    draw_subset_g<MP>(TabGet{ w.rng_tab, w.rng_len, (uint32_t)n }, pos, idx);
+    float ms1[2 * MP], ms2[2 * MP];
     #pragma unroll
-    for (int i = 0; i < 3; i++) {
+    for (int i = 0; i < MP; i++) {
         const float4 q = pts[idx[i]];
         ms1[2 * i] = q.x; ms1[2 * i + 1] = q.y; ms2[2 * i] = q.z; ms2[2 * i + 1] = q.w;
     }
-    affine_solve(ms1, ms2, M);
+    Model::solve(ms1, ms2, M);
 }
 
+template <class Model>
 __global__ void __launch_bounds__(SCORE_THREADS)
 ransac_affine_hyp_kernel(RansacWork w, int round_base, int round_len, int n_slices, int tiles)
 {
@@ -1904,7 +1957,7 @@ ransac_affine_hyp_kernel(RansacWork w, int round_base, int round_len, int n_slic
     float F[6];
     {
         double M[6];
-        if (live) affine_solve_sample(w, ps, n, w.sample_pos[slot], M);
+        if (live) affine_solve_sample<Model>(w, ps, n, w.sample_pos[slot], M);
         #pragma unroll
         for (int i = 0; i < 6; i++) F[i] = live ? (float)M[i] : 0.f;
     }
@@ -1928,108 +1981,100 @@ ransac_affine_hyp_kernel(RansacWork w, int round_base, int round_len, int n_slic
     if (live && cnt) atomicAdd(&w.counts[slot], cnt);
 }
 
+// The refine's sums for N parameters: the upper triangle of J^T J (NT entries), J^T r (N), |r|^2 and (exact mode) max |r|
+template <int N>
 struct AffineShared {
-    double part[(RS_THREADS / 32) * 28];
-    double out[29];
-    LmStateN<6> lm;
-    double scratch_a[36], scratch_v[36];
+    static constexpr int NT = N * (N + 1) / 2;
+    double part[(RS_THREADS / 32) * (NT + N + 1)];
+    double out[NT + N + 2];
+    LmStateN<N> lm;
+    double scratch_a[N * N], scratch_v[N * N];
     double r[2 * EXACT_MAX_INLIERS];            // exact mode: residuals of the current evaluation
     int flag;
     int warp_cnt[RS_THREADS / 32];
     int base_cnt;
 };
 
-// Jacobian entry (row, j) of Affine2DRefineCallback: row 2i is (X, Y, 1, 0, 0, 0), row 2i + 1 is (0, 0, 0, X, Y, 1)
-__device__ __forceinline__ double affine_jac(int row, int j, const float4& q)
-{
-    const int c = j - 3 * (row & 1);
-    return c == 0 ? (double)q.x : c == 1 ? (double)q.y : c == 2 ? 1.0 : 0.0;
-}
-
-// At x (wantJ): S = |r|^2, max |r|, A = J^T J (6 x 6) and v = J^T r, left in st.  At xd: Sd = |r|^2 in sh.out[0].  Up to
+// At x (wantJ): S = |r|^2, max |r|, A = J^T J (N x N) and v = J^T r, left in st.  At xd: Sd = |r|^2 in sh.out[0].  Up to
 // EXACT_MAX_INLIERS inliers every sum is one thread's, in OpenCV's order (mulTransposed sequential over rows, gemm with
 // 4 interleaved accumulators below 100 rows, norm in the AVX2 pattern); above, per-thread partial sums and block_sum.
+template <class Model>
 __device__ void affine_lm_eval(const float4* __restrict__ pts, const int32_t* __restrict__ sel, int count, const double* h,
-                               bool wantJ, AffineShared& sh)
+                               bool wantJ, AffineShared<Model::N>& sh)
 {
+    constexpr int N = Model::N, NT = AffineShared<N>::NT;
     const int tid = threadIdx.x;
-    double S, rm, A[21], v[6];
+    double S, rm, A[NT], v[N];
     if (count <= EXACT_MAX_INLIERS) {
         const int rows = 2 * count;
-        for (int i = tid; i < count; i += (int)blockDim.x) {
-            const float4 q = pts[sel[i]];
-            const double Mx = q.x, My = q.y;
-            sh.r[2 * i] = h[0] * Mx + h[1] * My + h[2] - q.z;
-            sh.r[2 * i + 1] = h[3] * Mx + h[4] * My + h[5] - q.w;
-        }
+        for (int i = tid; i < count; i += (int)blockDim.x) Model::residuals(h, pts[sel[i]], sh.r[2 * i], sh.r[2 * i + 1]);
         __syncthreads();
-        if (wantJ && tid < 21) {                                 // upper triangle entry (j, k) of J^T J
+        if (wantJ && tid < NT) {                                 // upper triangle entry (j, k) of J^T J
             int j = 0, e = tid;
-            while (e >= 6 - j) { e -= 6 - j; j++; }
+            while (e >= N - j) { e -= N - j; j++; }
             const int k = j + e;
             double s = 0;
             for (int row = 0; row < rows; row++) {
                 const float4 q = pts[sel[row >> 1]];
-                s += affine_jac(row, j, q) * affine_jac(row, k, q);
+                s += Model::jac(row, j, q) * Model::jac(row, k, q);
             }
             sh.out[tid] = s;
-        } else if (wantJ && tid >= 21 && tid < 27) {             // J^T r entry
-            const int j = tid - 21;
+        } else if (wantJ && tid >= NT && tid < NT + N) {         // J^T r entry
+            const int j = tid - NT;
             double s;
             if (rows < 100) {
                 double s4[4] = { 0, 0, 0, 0 };
                 const int full = rows & ~3;
                 for (int row = 0; row < rows; row++)
-                    s4[row < full ? (row & 3) : 0] += affine_jac(row, j, pts[sel[row >> 1]]) * sh.r[row];
+                    s4[row < full ? (row & 3) : 0] += Model::jac(row, j, pts[sel[row >> 1]]) * sh.r[row];
                 s = ((s4[0] + s4[1]) + s4[2]) + s4[3];
             } else {
                 s = 0;
-                for (int row = 0; row < rows; row++) s += affine_jac(row, j, pts[sel[row >> 1]]) * sh.r[row];
+                for (int row = 0; row < rows; row++) s += Model::jac(row, j, pts[sel[row >> 1]]) * sh.r[row];
             }
-            sh.out[21 + j] = s;
-        } else if (tid == 27) {
+            sh.out[NT + j] = s;
+        } else if (tid == NT + N) {
             NormL2SqrAcc na; na.init();
             for (int row = 0; row < rows; row++) na.push(sh.r[row]);
-            sh.out[27] = na.finish();
-        } else if (tid == 28) {
+            sh.out[NT + N] = na.finish();
+        } else if (tid == NT + N + 1) {
             double m = 0;
             for (int row = 0; row < rows; row++) { const double q = fabs(sh.r[row]); if (q > m) m = q; }
-            sh.out[28] = m;
+            sh.out[NT + N + 1] = m;
         }
         __syncthreads();
-        S = sh.out[27]; rm = sh.out[28];
+        S = sh.out[NT + N]; rm = sh.out[NT + N + 1];
         if (wantJ) {
-            for (int e = 0; e < 21; e++) A[e] = sh.out[e];
-            for (int j = 0; j < 6; j++) v[j] = sh.out[21 + j];
+            for (int e = 0; e < NT; e++) A[e] = sh.out[e];
+            for (int j = 0; j < N; j++) v[j] = sh.out[NT + j];
         }
         __syncthreads();
     } else {
-        double acc[28];
+        double acc[NT + N + 1];
         #pragma unroll
-        for (int k = 0; k < 28; k++) acc[k] = 0;
+        for (int k = 0; k < NT + N + 1; k++) acc[k] = 0;
         rm = 0;
         // 64 partial sums whatever blockDim.x (64 or 128, chosen from the batch's largest set): threads 64.. add exact
         // zeros, so a set's M does not depend on the batch it came in
         for (int i = tid; tid < 64 && i < count; i += 64) {
             const float4 q = pts[sel[i]];
-            const double Mx = q.x, My = q.y;
-            const double r0 = h[0] * Mx + h[1] * My + h[2] - q.z;
-            const double r1 = h[3] * Mx + h[4] * My + h[5] - q.w;
-            acc[27] += r0 * r0; acc[27] += r1 * r1;
+            double r0, r1;
+            Model::residuals(h, q, r0, r1);
+            acc[NT + N] += r0 * r0; acc[NT + N] += r1 * r1;
             rm = fmax(rm, fmax(fabs(r0), fabs(r1)));
             if (wantJ) {
                 int e = 0;
                 #pragma unroll
-                for (int j = 0; j < 6; j++) {
+                for (int j = 0; j < N; j++) {
                     #pragma unroll
-                    for (int k = j; k < 6; k++) {
-                        acc[e] += affine_jac(0, j, q) * affine_jac(0, k, q); acc[e] += affine_jac(1, j, q) * affine_jac(1, k, q); e++;
+                    for (int k = j; k < N; k++) {
+                        acc[e] += Model::jac(0, j, q) * Model::jac(0, k, q); acc[e] += Model::jac(1, j, q) * Model::jac(1, k, q); e++;
                     }
-                    acc[21 + j] += affine_jac(0, j, q) * r0; acc[21 + j] += affine_jac(1, j, q) * r1;
+                    acc[NT + j] += Model::jac(0, j, q) * r0; acc[NT + j] += Model::jac(1, j, q) * r1;
                 }
             }
         }
-        block_sum<28>(acc, sh.part, sh.out);
+        block_sum<NT + N + 1>(acc, sh.part, sh.out);
         #pragma unroll
         for (int o = 16; o > 0; o >>= 1) rm = fmax(rm, shfl_down_d(rm, o));
         if ((tid & 31) == 0) sh.part[tid >> 5] = rm;
@@ -2037,16 +2082,16 @@ __device__ void affine_lm_eval(const float4* __restrict__ pts, const int32_t* __
         rm = sh.part[0];
         for (int q = 1; q < (int)(blockDim.x >> 5); q++) rm = fmax(rm, sh.part[q]);
         __syncthreads();
-        S = acc[27];
-        for (int e = 0; e < 21; e++) A[e] = acc[e];
-        for (int j = 0; j < 6; j++) v[j] = acc[21 + j];
+        S = acc[NT + N];
+        for (int e = 0; e < NT; e++) A[e] = acc[e];
+        for (int j = 0; j < N; j++) v[j] = acc[NT + j];
     }
     if (tid == 0) {
-        LmStateN<6>& st = sh.lm;
+        LmStateN<N>& st = sh.lm;
         if (wantJ) {
             int e = 0;
-            for (int j = 0; j < 6; j++) {
-                for (int k = j; k < 6; k++) { st.A[j * 6 + k] = A[e]; st.A[k * 6 + j] = A[e]; e++; }
+            for (int j = 0; j < N; j++) {
+                for (int k = j; k < N; k++) { st.A[j * N + k] = A[e]; st.A[k * N + j] = A[e]; e++; }
                 st.v[j] = v[j];
             }
             st.S = S; st.rmax = rm;
@@ -2058,10 +2103,12 @@ __device__ void affine_lm_eval(const float4* __restrict__ pts, const int32_t* __
 }
 
 // One CTA per set: the winner re-solved in fp64, the returned mask from (float)M (RANSAC stage: the refine moves M, not the
-// mask), the ordered compaction of its inliers and LMSolver with Affine2DRefineCallback for refine_iters iterations.
+// mask), the ordered compaction of its inliers and LMSolver with the model's refine callback for refine_iters iterations.
+template <class Model>
 __global__ void __launch_bounds__(RS_THREADS)
 ransac_affine_finish_kernel(RansacWork w, int refine_iters)
 {
+    constexpr int MP = Model::MP, N = Model::N;
     const int set = blockIdx.x;
     const int n = w.counts_n[set];
     const int64_t start = w.starts[set];
@@ -2069,35 +2116,41 @@ ransac_affine_finish_kernel(RansacWork w, int refine_iters)
     uint8_t* mask = w.mask + start;
     int32_t* sel = w.sel + start;
     double* Mout = w.H + (size_t)set * 6;
-    __shared__ AffineShared sh;
-    LmStateN<6>& st = sh.lm;
+    __shared__ AffineShared<N> sh;
+    LmStateN<N>& st = sh.lm;
     const int tid = threadIdx.x;
-    if (n < 3 || (n > 3 && w.best_iter[set] < 0)) {             // cv2 returns an empty matrix
+    if (n < MP || (n > MP && w.best_iter[set] < 0)) {           // cv2 returns an empty matrix
         for (int i = tid; i < n; i += (int)blockDim.x) mask[i] = 0;
         if (tid < 6) Mout[tid] = 0.0;
         if (tid == 0) w.found[set] = 0;
         return;
     }
-    if (n == 3) {                                                // count == modelPoints: the closed form, mask 1,1,1, no refine
+    if (n == MP) {                                               // count == modelPoints: the closed form, mask all 1, no refine
         if (tid == 0) {
-            float ms1[6], ms2[6];
-            for (int i = 0; i < 3; i++) { ms1[2 * i] = pts[i].x; ms1[2 * i + 1] = pts[i].y; ms2[2 * i] = pts[i].z; ms2[2 * i + 1] = pts[i].w; }
+            float ms1[2 * MP], ms2[2 * MP];
+            for (int i = 0; i < MP; i++) { ms1[2 * i] = pts[i].x; ms1[2 * i + 1] = pts[i].y; ms2[2 * i] = pts[i].z; ms2[2 * i + 1] = pts[i].w; }
             double M[6];
-            affine_solve(ms1, ms2, M);
+            Model::solve(ms1, ms2, M);
             for (int i = 0; i < 6; i++) Mout[i] = M[i];
             w.found[set] = 1;
         }
-        if (tid < 3) mask[tid] = 1;
+        if (tid < MP) mask[tid] = 1;
         return;
     }
     if (tid == 0) {
-        affine_solve_sample(w, pts, n, w.sample_pos[(size_t)set * w.max_iters + w.best_iter[set]], st.x);
+        double M[6];
+        affine_solve_sample<Model>(w, pts, n, w.sample_pos[(size_t)set * w.max_iters + w.best_iter[set]], M);
+        Model::params(M, st.x);
         sh.base_cnt = 0;
     }
     __syncthreads();
     float F[6];
-    #pragma unroll
-    for (int i = 0; i < 6; i++) F[i] = (float)st.x[i];
+    {
+        double M[6];
+        Model::matrix(st.x, M);
+        #pragma unroll
+        for (int i = 0; i < 6; i++) F[i] = (float)M[i];
+    }
     const int lane = tid & 31, wid = tid >> 5;
     for (int base = 0; base < n; base += (int)blockDim.x) {       // mask + ordered compaction of the inlier indices
         const int i = base + tid;
@@ -2119,48 +2172,59 @@ ransac_affine_finish_kernel(RansacWork w, int refine_iters)
     }
     const int n_inl = sh.base_cnt;
     if (refine_iters > 0 && n_inl > 0) {
-        affine_lm_eval(pts, sel, n_inl, st.x, true, sh);
+        affine_lm_eval<Model>(pts, sel, n_inl, st.x, true, sh);
         if (tid == 0) lm_begin(st);
         for (;;) {
             if (tid == 0) lm_step(st, sh.scratch_a, sh.scratch_v);
             __syncthreads();
-            affine_lm_eval(pts, sel, n_inl, st.xd, false, sh);
+            affine_lm_eval<Model>(pts, sel, n_inl, st.xd, false, sh);
             if (tid == 0) sh.flag = lm_update(st, sh.out[0], sh.scratch_a, sh.scratch_v) ? 1 : 0;
             __syncthreads();
             if (sh.flag) {                                       // accepted: x = xd, A, v, S, rmax at x
-                if (tid == 0) for (int i = 0; i < 6; i++) st.x[i] = st.xd[i];
+                if (tid == 0) for (int i = 0; i < N; i++) st.x[i] = st.xd[i];
                 __syncthreads();
-                affine_lm_eval(pts, sel, n_inl, st.x, true, sh);
+                affine_lm_eval<Model>(pts, sel, n_inl, st.x, true, sh);
             }
             if (tid == 0) sh.flag = lm_proceed(st, refine_iters) ? 1 : 0;
             __syncthreads();
             if (!sh.flag) break;
         }
     }
-    if (tid < 6) Mout[tid] = st.x[tid];
-    if (tid == 0) w.found[set] = 1;
+    if (tid == 0) {
+        double M[6];
+        Model::matrix(st.x, M);
+        for (int i = 0; i < 6; i++) Mout[i] = M[i];
+        w.found[set] = 1;
+    }
 }
 
-int launch_affine(const RansacWork& w, int refine_iters, cudaStream_t st)
+template <class Model>
+static int launch_affine_model(const RansacWork& w, int refine_iters, cudaStream_t st)
 {
-    if (w.n_sets <= 0) return 0;
     const int round_len = ransac_round_len(w);
     const int n_sms = w.n_sms > 0 ? w.n_sms : 148;
     int launches = 0;
     for (int rb = 0; rb < w.max_iters; rb += round_len) {
         const int len = w.max_iters - rb < round_len ? w.max_iters - rb : round_len;
-        ransac_sample_kernel<3><<<w.n_sets, SMP_THREADS, 0, st>>>(w, rb, rb + len, nullptr);
+        ransac_sample_kernel<Model::MP><<<w.n_sets, SMP_THREADS, 0, st>>>(w, rb, rb + len, nullptr);
         cudaMemset2DAsync(w.counts + rb, (size_t)w.max_iters * 4, 0, (size_t)len * 4, (size_t)w.n_sets, st);
         // slices of the correspondences so that the launch holds >= ~6 CTAs per SM (or one slice per 512 points)
         const int tiles = (len + SCORE_THREADS - 1) / SCORE_THREADS;
         const int64_t ctas = (int64_t)tiles * w.n_sets;
         int n_slices = (int)std::min<int64_t>(std::max<int64_t>(1, ((int64_t)n_sms * 6 + ctas - 1) / ctas), std::max(1, w.max_n / 512));
         n_slices = std::max(1, std::min(n_slices, 64));
-        ransac_affine_hyp_kernel<<<dim3((unsigned)ctas, 1, (unsigned)n_slices), SCORE_THREADS, 0, st>>>(w, rb, len, n_slices, tiles);
+        ransac_affine_hyp_kernel<Model><<<dim3((unsigned)ctas, 1, (unsigned)n_slices), SCORE_THREADS, 0, st>>>(w, rb, len, n_slices, tiles);
         launches += 2 + launch_ransac_select(w, rb, len, st);
     }
-    ransac_affine_finish_kernel<<<w.n_sets, w.max_n <= 512 ? 64 : RS_THREADS, 0, st>>>(w, refine_iters);
+    ransac_affine_finish_kernel<Model><<<w.n_sets, w.max_n <= 512 ? 64 : RS_THREADS, 0, st>>>(w, refine_iters);
     return launches + 1;
+}
+
+int launch_affine(const RansacWork& w, int refine_iters, cudaStream_t st)
+{
+    if (w.n_sets <= 0) return 0;
+    return w.model_points == 2 ? launch_affine_model<PartialModel>(w, refine_iters, st)
+                               : launch_affine_model<AffineModel>(w, refine_iters, st);
 }
 
 // ---- gates + inlier gather: reference src/TestsDetector.cpp:74-94 ---------------------------------

@@ -86,8 +86,8 @@ typedef struct cvg_ransac_params {
     int32_t reserved;
 } cvg_ransac_params;
 
-/* estimateAffine2D(..., RANSAC, threshold, maxIters, confidence, refineIters) — OpenCV's defaults are
- * 3.0, 2000, 0.99, 10 (cvg_affine_params_default).  flags: CVG_RANSAC_NO_EARLY_STOP or 0. */
+/* estimateAffine2D and estimateAffinePartial2D(..., RANSAC, threshold, maxIters, confidence, refineIters) — OpenCV's
+ * defaults are 3.0, 2000, 0.99, 10 (cvg_affine_params_default).  flags: CVG_RANSAC_NO_EARLY_STOP or 0. */
 typedef struct cvg_affine_params {
     uint32_t size;                  /* = sizeof(cvg_affine_params)                                   */
     uint32_t flags;
@@ -132,7 +132,8 @@ int  cvg_create(cvg_ctx** out, int device, unsigned flags);
  * collective; cvg_match_knn2_sharded is the train-tile sharded match with its one all-gather, and
  * cvg_find_homography_sharded splits the hypotheses of one RANSAC over the GPUs with one all-gather of counts per
  * round.  The other entry points (cvg_match_knn2, cvg_find_homography, cvg_find_homography_batch,
- * cvg_estimate_affine2d, cvg_estimate_affine2d_batch, cvg_detect_pairs, cvg_dev_*) run on the first listed GPU.
+ * cvg_estimate_affine2d, cvg_estimate_affine2d_batch, cvg_estimate_affine_partial2d, cvg_estimate_affine_partial2d_batch,
+ * cvg_detect_pairs, cvg_dev_*) run on the first listed GPU.
  * A device may be listed more than once (logical shards on one GPU, used by the single-GPU tests); NCCL refuses
  * such a communicator, so the exchange then runs as device-to-device copies (cvg_exchange_kind: "memcpy"). */
 int  cvg_create_multi(cvg_ctx** out, const int* devices, int n_devices, unsigned flags);
@@ -214,6 +215,24 @@ int  cvg_estimate_affine2d_batch(cvg_ctx* ctx, const float* src_xy, const float*
                                  const int64_t* offsets, int n_sets, const cvg_affine_params* p,
                                  double* M /*[P,6]*/, uint8_t* mask, int32_t* found /*[P]*/,
                                  int32_t* iters /*[P]*/);
+
+/* cv::estimateAffinePartial2D(src, dst, inliers, RANSAC, p->threshold, p->max_iters, p->confidence, p->refine_iters):
+ * the 4-DOF similarity (rotation, uniform scale, translation) of src onto dst, M = [a, -b, tx; b, a, ty], with the
+ * outputs, parameter checks and return codes of cvg_estimate_affine2d.  RANSAC draws 2 distinct points per attempt and
+ * accepts every pair (two points are never collinear, so sets that estimateAffine2D rejects as collinear find a model
+ * here; coincident source points give an all-NaN hypothesis, which no point scores).  The Levenberg-Marquardt refine
+ * optimises (a, b, tx, ty) on the inliers of the winning hypothesis; the mask stays that hypothesis's.  n = 2 returns the
+ * exact fit of the two points with mask 1,1 and no refine (all NaN, still found, when the two source points coincide);
+ * n = 1 returns found = 0 and a zero mask; n = 0 -> CVG_ERR_TOO_FEW_POINTS.  M[1] is -0.0 when b is +0, as in OpenCV. */
+int  cvg_estimate_affine_partial2d(cvg_ctx* ctx, const float* src_xy, const float* dst_xy, int n,
+                                   const cvg_affine_params* p, double M[6], uint8_t* mask, int* found);
+
+/* Batched form: P independent point sets, each with the semantics above (sets of fewer than 2 points report
+ * found = 0).  iters (may be NULL) [P] = RANSAC iterations. */
+int  cvg_estimate_affine_partial2d_batch(cvg_ctx* ctx, const float* src_xy, const float* dst_xy,
+                                         const int64_t* offsets, int n_sets, const cvg_affine_params* p,
+                                         double* M /*[P,6]*/, uint8_t* mask, int32_t* found /*[P]*/,
+                                         int32_t* iters /*[P]*/);
 
 /* ---- fused path: replaces the body of the view loop, src/TestsDetector.cpp:58-95 -------------
  * All views of the resident model set against one scene (descriptors [n_train,128] + keypoints
@@ -328,7 +347,7 @@ int  cvg_last_match_guard_rows(const cvg_ctx* ctx);
 /* Verify calls with CVG_RANSAC_NO_EARLY_STOP and max_iters >= 32768 cut every set's cv::RNG draw stream into
  * chunks walked by many CTAs (same samples as the serial walk).  Returns how many sets of the last such call
  * were handed back to the one-CTA-per-set sampler, or -1 if the last verify call did not use the chunked sampler
- * (estimateAffine2D calls never do). */
+ * (estimateAffine2D and estimateAffinePartial2D calls never do). */
 int  cvg_last_sampler_serial_sets(const cvg_ctx* ctx);
 /* The context's cudaStream_t (all of its GPU work is issued there); lets a harness record its own
  * CUDA events around calls. */
