@@ -19,7 +19,8 @@ class AffineParams(C.Structure):
 
 class DetectParams(C.Structure):
     _fields_ = [("size", C.c_uint32), ("ratio", C.c_float), ("min_inliers", C.c_int32), ("det_lo", C.c_float),
-                ("det_hi", C.c_float), ("reserved", C.c_int32), ("ransac", RansacParams)]
+                ("det_hi", C.c_float), ("reserved", C.c_int32), ("ransac", RansacParams),
+                ("method", C.c_int32), ("refine_iters", C.c_int32)]
 
 
 class PairResult(C.Structure):

@@ -97,6 +97,7 @@ void cvg_detect_params_default(cvg_detect_params* p)
     memset(p, 0, sizeof *p);
     p->size = sizeof *p; p->ratio = 0.9f; p->min_inliers = 4; p->det_lo = 0.1f; p->det_hi = 10.0f;
     cvg_ransac_params_default(&p->ransac);
+    p->method = CVG_VERIFY_HOMOGRAPHY; p->refine_iters = 10;
 }
 
 }  // extern "C"
@@ -1083,14 +1084,28 @@ static int detect_common(cvg_ctx* c, const cvg_models* m, cvg_scenes* cache, Tra
     if (c->timing) cudaEventRecord(c->ev[1], c->stream);
     int max_view = 0;
     for (int v = 0; v < V; v++) max_view = std::max(max_view, m->view_offsets[v + 1] - m->view_offsets[v]);
+    // the verify stage of p->method: RANSAC modelPoints 4 (findHomography), 3 (estimateAffine2D), 2 (estimateAffinePartial2D)
+    const int mp = p->method == CVG_VERIFY_AFFINE ? 3 : (p->method == CVG_VERIFY_AFFINE_PARTIAL ? 2 : 4);
     int flag = 0;
     for (int attempt = 0;; attempt++) {
-        rc = run_ransac(c, c->pts.as<float4>(), c->starts.as<int64_t>(), c->counts_n.as<int32_t>(), P, max_view,
-                        (int64_t)rows, &p->ransac, false);
+        if (mp == 4) {
+            rc = run_ransac(c, c->pts.as<float4>(), c->starts.as<int64_t>(), c->counts_n.as<int32_t>(), P, max_view,
+                            (int64_t)rows, &p->ransac, false);
+        } else {
+            RansacWork w;
+            rc = eng_ransac_work(c, c->pts.as<float4>(), c->starts.as<int64_t>(), c->counts_n.as<int32_t>(), P, max_view,
+                                 (int64_t)rows, &p->ransac, false, 0, &w, mp);
+            if (!rc) {
+                c->launches += launch_affine(w, p->refine_iters, c->stream);
+                c->hyp_rounds = 0;                                  // no solve / score events: the timing below reports 0
+                CU_CHECK(cudaGetLastError());
+            }
+        }
         if (rc) return rc;
         GateWork g;
         g.n_pairs = P; g.pts = c->pts.as<float4>(); g.starts = c->starts.as<int64_t>(); g.counts_n = c->counts_n.as<int32_t>();
         g.mask = c->mask.as<uint8_t>(); g.found = c->found.as<int32_t>(); g.H = c->H.as<double>();
+        g.model_points = mp; g.h_stride = mp == 4 ? 9 : 6;
         g.iters_run = c->iters_run.as<int32_t>(); g.pair_scale = d_scales;
         g.min_inliers = p->min_inliers; g.det_lo = p->det_lo; g.det_hi = p->det_hi;
         g.results = c->results.as<cvg_pair_result>();
@@ -1149,22 +1164,42 @@ static int detect_common(cvg_ctx* c, const cvg_models* m, cvg_scenes* cache, Tra
     return CVG_OK;
 }
 
-int check_detect_params(const cvg_detect_params* p)
+// The caller's struct in either layout (include/cvgraft.h) as a full, checked copy: every entry point works on `out` from
+// here on, so nothing reads past the caller's `size` bytes (the 56-byte layout ends before `method`: homography).
+int check_detect_params(const cvg_detect_params* p, cvg_detect_params* out)
 {
-    if (!p || p->size != sizeof(cvg_detect_params)) return set_err(CVG_ERR_INVALID, "cvg_detect_params: bad size field");
-    return check_params(&p->ransac);
+    constexpr uint32_t OLD_SIZE = offsetof(cvg_detect_params, method);
+    if (!p || (p->size != sizeof(cvg_detect_params) && p->size != OLD_SIZE))
+        return set_err(CVG_ERR_INVALID, "cvg_detect_params: bad size field");
+    cvg_detect_params q;
+    cvg_detect_params_default(&q);
+    memcpy(&q, p, p->size);
+    q.size = sizeof q;
+    if (q.method < CVG_VERIFY_HOMOGRAPHY || q.method > CVG_VERIFY_AFFINE_PARTIAL)
+        return set_err(CVG_ERR_INVALID, "cvg_detect_params: unknown method %d", q.method);
+    if (q.method != CVG_VERIFY_HOMOGRAPHY) {
+        if (q.ransac.flags & ~CVG_RANSAC_NO_EARLY_STOP)
+            return set_err(CVG_ERR_INVALID, "cvg_detect_params: flags 0x%x with an affine method", q.ransac.flags);
+        if (q.refine_iters < 0 || q.refine_iters > 1000) return set_err(CVG_ERR_LIMIT, "refine_iters out of range [0, 1000]");
+    }
+    const int rc = check_params(&q.ransac);
+    if (rc) return rc;
+    *out = q;
+    return CVG_OK;
 }
 
 extern "C" {
 
 int cvg_detect_pairs(cvg_ctx* c, const cvg_models* m, const float* scene_desc, const float* scene_kpt_xy, int n_train,
-                     float scale, const cvg_detect_params* p, cvg_pair_result* per_view, float* inlier_scene_xy,
+                     float scale, const cvg_detect_params* p_in, cvg_pair_result* per_view, float* inlier_scene_xy,
                      int32_t* inlier_offsets)
 {
     c = cvg_primary(c); m = cvg_models_on(m, c);
     if (!c || !m || !per_view) return set_err(CVG_ERR_INVALID, "cvg_detect_pairs: NULL argument");
-    int rc = check_detect_params(p);
+    cvg_detect_params params;
+    int rc = check_detect_params(p_in, &params);
     if (rc) return rc;
+    const cvg_detect_params* p = &params;
     if (n_train < 0 || (n_train > 0 && (!scene_desc || !scene_kpt_xy))) return set_err(CVG_ERR_INVALID, "bad scene arrays");
     CU_CHECK(cudaSetDevice(c->device));
     c->stage_used = 0; c->stage_fallback = false;

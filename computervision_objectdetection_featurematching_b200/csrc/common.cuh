@@ -187,6 +187,8 @@ struct GateWork {
     int n_pairs;
     const float4* pts; const int64_t* starts; const int32_t* counts_n;   // per pair correspondences
     const uint8_t* mask; const int32_t* found; const double* H; const int32_t* iters_run;
+    int model_points;                               // 4 homography, 3 / 2 the affine methods: fewer matches -> no model
+    int h_stride;                                   // doubles per pair in H: 9 (3x3), 6 (2x3 M, promoted to 3x3 here)
     const float* pair_scale;                        // [n_pairs] or NULL
     int min_inliers; float det_lo, det_hi;
     cvg_pair_result* results;                       // [n_pairs] device

@@ -228,7 +228,9 @@ int  eng_scenes_wait(cvg_ctx* c, cvg_scenes* sc);
 int  eng_detect_range(cvg_ctx* c, const cvg_models* m, cvg_scenes* sc, int s0, int s1, const float* scales,
                       const cvg_detect_params* p, cvg_pair_result* per_pair, std::vector<float>* pool,
                       std::vector<int32_t>* cnt);
-int  check_detect_params(const cvg_detect_params* p);
+// the caller's cvg_detect_params (either size, include/cvgraft.h) checked and copied in full into *out; every entry point
+// hands the copy on, never the caller's pointer
+int  check_detect_params(const cvg_detect_params* p, cvg_detect_params* out);
 int  check_params(const cvg_ransac_params* p);
 int  sync_and_check(cvg_ctx* c);                        // waits for the engine's stream; names the device on a fault
 // verify stage building blocks (the hypothesis-range sharded driver of multi.cu runs one engine per device through them)

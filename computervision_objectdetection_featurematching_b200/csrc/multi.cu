@@ -467,12 +467,14 @@ void cvg_scenes_free(cvg_ctx* c, cvg_scenes* sc)
 
 // ---- fused path over resident scene batches ---------------------------------------------------------------------
 int cvg_detect_scenes_submit(cvg_ctx* c, const cvg_models* m, const cvg_scenes* scenes, const float* scales,
-                             const cvg_detect_params* p, cvg_pair_result* per_pair, float* inlier_scene_xy,
+                             const cvg_detect_params* p_in, cvg_pair_result* per_pair, float* inlier_scene_xy,
                              int64_t* inlier_offsets, cvg_job** job)
 {
     if (!c || !m || !scenes || !per_pair || !job) return cvg_set_err(CVG_ERR_INVALID, "cvg_detect_scenes_submit: NULL argument");
-    const int rc = check_detect_params(p);
+    cvg_detect_params params;                          // the full layout: dev_submit copies it into the job
+    const int rc = check_detect_params(p_in, &params);
     if (rc) return rc;
+    const cvg_detect_params* p = &params;
     if (c->multi) return multi_submit(c, m, scenes, scales, p, per_pair, inlier_scene_xy, inlier_offsets, false, job);
     return dev_submit(c, m, const_cast<cvg_scenes*>(scenes), scales, p, per_pair, inlier_scene_xy, inlier_offsets, false, job);
 }
@@ -486,12 +488,14 @@ int cvg_job_wait(cvg_ctx* c, cvg_job* job)
 }
 
 int cvg_detect_scenes_inliers(cvg_ctx* c, const cvg_models* m, const cvg_scenes* scenes, const float* scales,
-                              const cvg_detect_params* p, cvg_pair_result* per_pair, float* inlier_scene_xy,
+                              const cvg_detect_params* p_in, cvg_pair_result* per_pair, float* inlier_scene_xy,
                               int64_t* inlier_offsets)
 {
     if (!c || !m || !scenes || !per_pair) return cvg_set_err(CVG_ERR_INVALID, "cvg_detect_scenes: NULL argument");
-    int rc = check_detect_params(p);
+    cvg_detect_params params;
+    int rc = check_detect_params(p_in, &params);
     if (rc) return rc;
+    const cvg_detect_params* p = &params;
     cvg_job* job = nullptr;
     if (c->multi) {
         rc = multi_submit(c, m, scenes, scales, p, per_pair, inlier_scene_xy, inlier_offsets, true, &job);

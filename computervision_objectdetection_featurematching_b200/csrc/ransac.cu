@@ -2237,15 +2237,23 @@ __global__ void gates_kernel(GateWork g)
     const int64_t start = g.starts[pair];
     const uint8_t* mask = g.mask + start;
     const float4* pts = g.pts + start;
-    const bool found = n >= 4 && g.found[pair] != 0;
+    const bool found = n >= g.model_points && g.found[pair] != 0;
     int cnt = 0;
     if (found)
         for (int i = lane; i < n; i += 32) cnt += mask[i] ? 1 : 0;
     #pragma unroll
     for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+    // a 2x3 affine M (stride 6) is promoted to [M; 0 0 1]: its det3 is the area scale M00*M11 - M01*M10
+    const double* Hs = g.H + (size_t)pair * g.h_stride;
     double H[9];
     #pragma unroll
-    for (int i = 0; i < 9; i++) H[i] = found ? g.H[(size_t)pair * 9 + i] : 0.0;
+    for (int i = 0; i < 6; i++) H[i] = found ? Hs[i] : 0.0;
+    if (g.h_stride == 9) {
+        #pragma unroll
+        for (int i = 6; i < 9; i++) H[i] = found ? Hs[i] : 0.0;
+    } else {
+        H[6] = 0.0; H[7] = 0.0; H[8] = found ? 1.0 : 0.0;
+    }
     const double det = found ? det3(H) : 0.0;
     int status;
     if (n < g.min_inliers) status = CVG_PAIR_LT4_MATCHES;                     // :74

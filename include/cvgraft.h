@@ -97,23 +97,45 @@ typedef struct cvg_affine_params {
     int32_t refine_iters;           /* LM iterations on the inliers, [0, 1000]; 0 = none             */
 } cvg_affine_params;
 
-/* constants of detectObjects() — src/TestsDetector.cpp:21-25 */
+/* cvg_detect_params.method: the geometric check of the fused path (the call at src/TestsDetector.cpp:77-78) */
+#define CVG_VERIFY_HOMOGRAPHY     0 /* findHomography(RANSAC) (default)                                              */
+#define CVG_VERIFY_AFFINE         1 /* estimateAffine2D(RANSAC, refineIters = refine_iters)                         */
+#define CVG_VERIFY_AFFINE_PARTIAL 2 /* estimateAffinePartial2D(RANSAC, refineIters = refine_iters)                  */
+
+/* constants of detectObjects() — src/TestsDetector.cpp:21-25.
+ * Size rule: `size` = sizeof(cvg_detect_params) is this layout.  `size` = offsetof(cvg_detect_params, method) (56) is
+ * the layout before `method` and `refine_iters` existed and means CVG_VERIFY_HOMOGRAPHY: the library reads no byte
+ * past it.  Any other size -> CVG_ERR_INVALID.  `reserved` is ignored whatever it holds.
+ * The affine methods use ransac.threshold, ransac.max_iters and ransac.confidence as given (as cvg_affine_params
+ * carries them; cvg_detect_params_default keeps findHomography's 5.0 / 2000 / 0.995, not OpenCV's affine defaults);
+ * ransac.flags may be 0 or CVG_RANSAC_NO_EARLY_STOP (CVG_RANSAC_NO_REFINE -> CVG_ERR_INVALID); refine_iters outside
+ * [0, 1000] -> CVG_ERR_LIMIT.  An unknown method -> CVG_ERR_INVALID.  The homography method ignores refine_iters. */
 typedef struct cvg_detect_params {
-    uint32_t size;                  /* = sizeof(cvg_detect_params)                                   */
+    uint32_t size;                  /* = sizeof(cvg_detect_params), or 56 (see above)                */
     float ratio;                    /* MATCH_RATIO_THRESHOLD = 0.9f                       :21        */
     int32_t min_inliers;            /* MIN_INLIERS = 4                                    :22        */
     float det_lo;                   /* HOMOGRAPHY_DET_THRESHOLD = 0.1f                    :24        */
     float det_hi;                   /* HOMOGRAPHY_DET_UPPER_THRESHOLD = 10.0f             :25        */
     int32_t reserved;
     cvg_ransac_params ransac;
+    int32_t method;                 /* CVG_VERIFY_*; default CVG_VERIFY_HOMOGRAPHY                    */
+    int32_t refine_iters;           /* LM iterations of the affine methods; default 10 (OpenCV's)    */
 } cvg_detect_params;
 
+/* Per pair of the fused path.  For the affine methods (M the 2x3 matrix cv2 returns):
+ *   H = M promoted to 3x3, [M00 M01 M02; M10 M11 M12; 0 0 1], and det = its 3x3 determinant (= M00*M11 - M01*M10, the
+ *   area scale), which the det_lo / det_hi gate tests as at :84 — a NaN det (the all-NaN M of a coincident 2-point
+ *   partial set) fails neither comparison and passes, as the reference's expression would;
+ *   n_inliers = countNonZero of the RANSAC-stage mask OpenCV returns, ransac_iters = the iters of the batch calls;
+ *   "H empty" (:79) = cv2 returns no matrix: fewer good matches than the model's points (3, 2), every triple collinear
+ *   (affine), or getSubset's 10 000 attempts exhausted.  Gate order :74 -> :79 -> :81 -> :84 for every method. */
 typedef struct cvg_pair_result {
     int32_t status;                 /* CVG_PAIR_*                                                    */
     int32_t n_good;                 /* matches that passed the ratio test                            */
     int32_t n_inliers;              /* countNonZero(inlierMask) (0 when no H)                        */
     int32_t ransac_iters;           /* RANSAC iterations the reference loop would have run           */
-    double H[9];                    /* row-major 3x3, H[8] == 1; zeros when status is LT4/H_EMPTY     */
+    double H[9];                    /* row-major 3x3, H[8] == 1 (homography: as returned); zeros when */
+                                    /* no model was found (H_EMPTY, or fewer matches than its points) */
     double det;                     /* determinant(H)                                                */
 } cvg_pair_result;
 
@@ -235,6 +257,9 @@ int  cvg_estimate_affine_partial2d_batch(cvg_ctx* ctx, const float* src_xy, cons
                                          int32_t* iters /*[P]*/);
 
 /* ---- fused path: replaces the body of the view loop, src/TestsDetector.cpp:58-95 -------------
+ * Every fused call (cvg_detect_pairs, cvg_detect_scenes*, cvg_detect_scenes_submit) verifies with p->method: the
+ * findHomography, estimateAffine2D or estimateAffinePartial2D stage of the calls above, on the same correspondences,
+ * through every path (lanes, jobs in flight, multi-device pair sharding).
  * All views of the resident model set against one scene (descriptors [n_train,128] + keypoints
  * [n_train,2]).  per_view [V]: status, counts, H, det.  inlier_scene_xy receives, view after view,
  * the scene points of the inliers of ACCEPTED views divided by `scale` when scale != 1.0f
@@ -361,7 +386,9 @@ int  cvg_set_timing(cvg_ctx* ctx, int enabled);
 int  cvg_last_timing(const cvg_ctx* ctx, float* match_ms, float* ransac_ms, float* total_ms);
 /* Verify-stage detail of the last fused call (timing enabled): summed device time of the hypothesis
  * kernel launches, their number, and the number of (hypothesis, correspondence) pairs they scored —
- * 16 bytes each is the algorithmic traffic of the scoring (SURVEY.md section 8d). */
+ * 16 bytes each is the algorithmic traffic of the scoring (SURVEY.md section 8d).  These cover the homography method
+ * only: after a fused call with an affine method (whose solve-and-score kernel is one fused launch) hyp_ms,
+ * hyp_launches, scored_points and cvg_last_score_ms are all 0; ransac_ms of cvg_last_timing covers its whole stage. */
 int  cvg_last_hyp_stats(const cvg_ctx* ctx, float* hyp_ms, int* hyp_launches, uint64_t* scored_points);
 /* hyp_ms above covers the solve kernel (4-point DLT, one launch per round); the inlier counting of those models runs in
  * ransac_score_kernel, one launch per round as well: its summed device time in the last fused call. */
