@@ -56,6 +56,8 @@ SYMBOLS = {
     "cvg_models_num_rows": (C.c_int, [_P]),
     "cvg_match_knn2": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_float, _P, _P, _P]),
     "cvg_match_knn2_raw": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_float, _P, _P, _P]),
+    "cvg_match_cross_check": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, _P]),
+    "cvg_match_cross_check_raw": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, _P]),
     "cvg_find_homography": (C.c_int, [_P, _P, _P, C.c_int, C.POINTER(RansacParams), _P, _P, C.POINTER(C.c_int), _P]),
     "cvg_find_homography_batch": (C.c_int, [_P, _P, _P, _P, C.c_int, C.POINTER(RansacParams), _P, _P, _P, _P, _P]),
     "cvg_estimate_affine2d": (C.c_int, [_P, _P, _P, C.c_int, C.POINTER(AffineParams), _P, _P, C.POINTER(C.c_int)]),

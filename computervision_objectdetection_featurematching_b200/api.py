@@ -2,6 +2,7 @@
 
     Context.match_knn2        <- cv::BFMatcher(NORM_L2).knnMatch(q, t, 2) + ratio test
                                  reference src/TestsDetector.cpp:59-72
+    Context.match_cross_check <- cv::BFMatcher(NORM_L2, crossCheck=true).match(q, t)
     Context.find_homography   <- cv::findHomography(src, dst, RANSAC, 5.0, mask)    :77-78
     Context.estimate_affine2d <- cv::estimateAffine2D(src, dst, inliers, RANSAC)    (the other geometric checks)
     Context.estimate_affine_partial2d <- cv::estimateAffinePartial2D(src, dst, inliers, RANSAC)
@@ -243,6 +244,23 @@ class Context:
         self._check(rc)
         return idx, dist, acc
 
+    def match_cross_check(self, query, train, view=-1):
+        """BFMatcher(NORM_L2, crossCheck=True).match.  query: Models (resident; one view, or view=-1 for every view, each
+        view its own query matrix) or an [nq,128] array.  -> idx[nq] (-1 = no match), dist[nq] (0 where idx is -1)."""
+        t = _f32(train, 128)
+        if isinstance(query, Models):
+            nq = query.n_rows if view < 0 else int(query.view_offsets[view + 1] - query.view_offsets[view])
+        else:
+            q = _f32(query, 128)
+            nq = q.shape[0]
+        idx = np.full(nq, -1, np.int32); dist = np.zeros(nq, np.float32)
+        if isinstance(query, Models):
+            rc = self.lib.cvg_match_cross_check(self.handle, query.handle, view, _ptr(t), t.shape[0], _ptr(idx), _ptr(dist))
+        else:
+            rc = self.lib.cvg_match_cross_check_raw(self.handle, _ptr(q), nq, _ptr(t), t.shape[0], _ptr(idx), _ptr(dist))
+        self._check(rc)
+        return idx, dist
+
     @property
     def last_match_path(self):
         return self.lib.cvg_last_match_path(self.handle)
@@ -254,7 +272,8 @@ class Context:
 
     @property
     def last_match_guard_rows(self):
-        """Rows of the last tensor-path call whose second distance reached 2048 and were redone exactly."""
+        """Rows of the last tensor-path call whose second distance reached 2048 and were redone exactly (cross-check calls:
+        query rows plus train columns whose nearest distance reached 2048)."""
         return int(self.lib.cvg_last_match_guard_rows(self.handle))
 
     @property

@@ -169,7 +169,7 @@ void eng_destroy(cvg_ctx* c)
     if (c->stream) cudaStreamSynchronize(c->stream);
     for (int i = 0; i < 3; i++) if (c->copy_stream[i]) cudaStreamSynchronize(c->copy_stream[i]);
     DevBuf* bufs[] = { &c->q_f32, &c->q_b, &c->q_blo, &c->q_aug, &c->q_norm, &c->t_f32, &c->t_b, &c->t_blo, &c->t_aug, &c->t_segtab, &c->t_kpt, &c->t_kptoff,
-                       &c->units, &c->dir, &c->parts, &c->parts4, &c->segdev, &c->fb, &c->plan_units, &c->plan_dir, &c->chunk, &c->hypH, &c->idx, &c->dist, &c->accept, &c->pts, &c->starts, &c->counts_n,
+                       &c->xc, &c->units, &c->dir, &c->parts, &c->parts4, &c->segdev, &c->fb, &c->plan_units, &c->plan_dir, &c->chunk, &c->hypH, &c->idx, &c->dist, &c->accept, &c->pts, &c->starts, &c->counts_n,
                        &c->sample_pos, &c->n_samples, &c->counts, &c->best_iter, &c->best_count, &c->iters_run, &c->niters_cur, &c->smp_state, &c->sel,
                        &c->H, &c->mask, &c->rmask, &c->found, &c->sflags, &c->results, &c->inl_xy, &c->inl_cnt,
                        &c->scales, &c->src, &c->dst, &c->nit, &c->nitreq };
@@ -386,6 +386,23 @@ struct QuerySide {
     int n_pad;                     // rows of the padded operand matrices
 };
 
+// Train tiles per unit for n_rb query row blocks against every segment: the length that minimises the estimated makespan
+// (tiles per CTA incl. an A-reload cost of 0.5 tile).
+static int plan_chunk_len(int64_t n_rb, const TrainSet& ts, int n_sms)
+{
+    int max_ct = 1;
+    for (const SegInfo& s : ts.segs) max_ct = std::max(max_ct, s.ct);
+    int best_ch = 1; double best_cost = 1e300;
+    for (int ch = 1; ch <= max_ct; ch++) {
+        int64_t n_units = 0;
+        for (const SegInfo& s : ts.segs) n_units += n_rb * ((s.ct + ch - 1) / ch);
+        const double waves = ceil((double)n_units / n_sms);
+        const double cost = waves * (ch + 0.5);
+        if (cost < best_cost - 1e-9) { best_cost = cost; best_ch = ch; }
+    }
+    return best_ch;
+}
+
 // Build the unit list for query rows [row_begin,row_end) x all segments.  Returns units sorted by size
 // (largest first) and the merge directory [seg][rowblock].
 static void build_plan(const QuerySide& q, const TrainSet& ts, int n_sms, std::vector<MatchUnit>& units,
@@ -393,18 +410,7 @@ static void build_plan(const QuerySide& q, const TrainSet& ts, int n_sms, std::v
 {
     const int nq = q.row_end - q.row_begin;
     n_rb = (nq + TILE_M - 1) / TILE_M;
-    int64_t total_tiles = 0;
-    int max_ct = 1;
-    for (const SegInfo& s : ts.segs) { total_tiles += (int64_t)n_rb * s.ct; max_ct = std::max(max_ct, s.ct); }
-    // chunk length: minimise the estimated makespan (tiles per CTA incl. an A-reload cost of 0.5 tile)
-    int best_ch = 1; double best_cost = 1e300;
-    for (int ch = 1; ch <= max_ct; ch++) {
-        int64_t n_units = 0;
-        for (const SegInfo& s : ts.segs) n_units += (int64_t)n_rb * ((s.ct + ch - 1) / ch);
-        const double waves = ceil((double)n_units / n_sms);
-        const double cost = waves * (ch + 0.5);
-        if (cost < best_cost - 1e-9) { best_cost = cost; best_ch = ch; }
-    }
+    const int best_ch = plan_chunk_len(n_rb, ts, n_sms);
     units.clear(); dir.assign((size_t)ts.n_segs * n_rb, MergeEntry{ 0, 0 });
     // With an even number of row blocks the list is made of PAIRS: units (2p, 2p + 1) are row blocks (2i, 2i + 1) against
     // the same train tiles — what the cta_group::2 form of the match kernel needs (launch_match_tc, paired); any other
@@ -443,6 +449,36 @@ static void build_plan(const QuerySide& q, const TrainSet& ts, int n_sms, std::v
     std::vector<MatchUnit> sorted; sorted.reserve(units.size());
     for (int gi : order) for (int k = 0; k < group; k++) sorted.push_back(units[(size_t)gi * group + k]);
     units.swap(sorted);
+}
+
+// Cross-check plan (one train segment): 128-row blocks of each view, starting at the view's first row — the padded query
+// operand holds such a tile (DESIGN.md 2) — against runs of train tiles.  A unit carries its view slot and how many of
+// its rows belong to the view (MatchUnit::pad1); the row side needs no merge directory (atomicMin keys).  Largest first.
+static void build_xc_plan(const std::vector<SegDev>& views, const TrainSet& ts, int n_sms, std::vector<MatchUnit>& units)
+{
+    units.clear();
+    const SegInfo& g = ts.segs[0];
+    if (g.rows == 0) return;
+    int64_t n_rb = 0;
+    for (const SegDev& v : views) n_rb += (v.rows + TILE_M - 1) / TILE_M;
+    const int ch = plan_chunk_len(n_rb, ts, n_sms);
+    const int n_chunks = (g.ct + ch - 1) / ch;
+    for (size_t s = 0; s < views.size(); s++)
+        for (int rb = 0; rb * TILE_M < views[s].rows; rb++)
+            for (int ck = 0; ck < n_chunks; ck++) {
+                const int t0 = (int)((int64_t)g.ct * ck / n_chunks), t1 = (int)((int64_t)g.ct * (ck + 1) / n_chunks);
+                MatchUnit u;
+                u.q_row0 = (int32_t)views[s].f32_row0 + rb * TILE_M;
+                u.t_row0 = t0 * TILE_N;
+                u.n_tiles = t1 - t0;
+                u.t_local0 = t0 * TILE_N;
+                u.part_slot = 0;
+                u.seg_cols = g.rows;
+                u.t_row0_f32 = t0 * TILE_N;
+                u.pad1 = (int32_t)(s << 8) | std::min(TILE_M, views[s].rows - rb * TILE_M);
+                units.push_back(u);
+            }
+    std::stable_sort(units.begin(), units.end(), [](const MatchUnit& a, const MatchUnit& b) { return a.n_tiles > b.n_tiles; });
 }
 
 // Match paths.  Host-side hints / cvg_last_match_path: 1 = tensor cores, exact (integer descriptors), 2 = exact fp32
@@ -841,14 +877,11 @@ int cvg_match_knn2(cvg_ctx* c, const cvg_models* m, int view, const float* train
     return match_host_train(c, q, m->nonint, train, n_train, ratio, idx, dist, accept);
 }
 
-int cvg_match_knn2_raw(cvg_ctx* c, const float* query, int n_query, const float* train, int n_train, float ratio,
-                       int32_t* idx, float* dist, uint8_t* accept)
+}  // extern "C"
+
+// a host query matrix [n_query,128] to the context's raw-query buffers (prepared operands); *qflag = its row kinds
+static int upload_raw_query(cvg_ctx* c, const float* query, int n_query, QuerySide* q, int* qflag)
 {
-    c = cvg_primary(c);
-    if (!c) return set_err(CVG_ERR_INVALID, "cvg_match_knn2_raw: NULL context");
-    if (n_query < 0 || (n_query > 0 && !query)) return set_err(CVG_ERR_INVALID, "bad query matrix");
-    if (n_query == 0) return CVG_OK;
-    CU_CHECK(cudaSetDevice(c->device));
     const int n_pad = round_up(n_query, TILE_M);
     CU_CHECK(c->q_f32.ensure((size_t)n_pad * DIM * 4)); CU_CHECK(c->q_b.ensure((size_t)n_pad * DIM * 2));
     CU_CHECK(c->q_blo.ensure((size_t)n_pad * DIM * 2));
@@ -858,12 +891,145 @@ int cvg_match_knn2_raw(cvg_ctx* c, const float* query, int n_query, const float*
     launch_prep_rows(c->q_f32.as<float>(), n_query, n_pad, 0, c->q_b.as<__nv_bfloat16>(), c->q_blo.as<__nv_bfloat16>(),
                      c->q_aug.as<__nv_bfloat16>(), c->q_norm.as<float>(), c->d_flags + 3, nullptr, c->stream);
     c->launches++;
-    int qflag = 0;
-    CU_CHECK(cudaMemcpyAsync(&qflag, c->d_flags + 3, 4, cudaMemcpyDeviceToHost, c->stream));
+    CU_CHECK(cudaMemcpyAsync(qflag, c->d_flags + 3, 4, cudaMemcpyDeviceToHost, c->stream));
     CU_CHECK(cudaStreamSynchronize(c->stream));
-    QuerySide q{ c->q_f32.as<float>(), c->q_b.as<__nv_bfloat16>(), c->q_blo.as<__nv_bfloat16>(), c->q_aug.as<__nv_bfloat16>(),
-                 c->q_norm.as<float>(), 0, n_query, n_pad };
+    *q = QuerySide{ c->q_f32.as<float>(), c->q_b.as<__nv_bfloat16>(), c->q_blo.as<__nv_bfloat16>(), c->q_aug.as<__nv_bfloat16>(),
+                    c->q_norm.as<float>(), 0, n_query, n_pad };
+    return CVG_OK;
+}
+
+extern "C" {
+
+int cvg_match_knn2_raw(cvg_ctx* c, const float* query, int n_query, const float* train, int n_train, float ratio,
+                       int32_t* idx, float* dist, uint8_t* accept)
+{
+    c = cvg_primary(c);
+    if (!c) return set_err(CVG_ERR_INVALID, "cvg_match_knn2_raw: NULL context");
+    if (n_query < 0 || (n_query > 0 && !query)) return set_err(CVG_ERR_INVALID, "bad query matrix");
+    if (n_query == 0) return CVG_OK;
+    CU_CHECK(cudaSetDevice(c->device));
+    QuerySide q; int qflag = 0;
+    const int rc = upload_raw_query(c, query, n_query, &q, &qflag);
+    if (rc) return rc;
     return match_host_train(c, q, qflag, train, n_train, ratio, idx, dist, accept);
+}
+
+}  // extern "C"
+
+// BFMatcher(NORM_L2, crossCheck = true).match of every view slot's query rows against a host train matrix; results to host.
+// The tensor-core instance (integer rows) and the exact SIMT kernel are both enqueued and gate themselves on the path word.
+static int match_cross_check(cvg_ctx* c, const QuerySide& q, const std::vector<SegDev>& views, int q_nonint, const float* train,
+                             int n_train, int32_t* idx, float* dist)
+{
+    const int nq = q.row_end - q.row_begin;
+    if (nq <= 0) return CVG_OK;
+    if (n_train < 0 || (n_train > 0 && !train)) return set_err(CVG_ERR_INVALID, "bad train matrix");
+    if (!idx || !dist) return set_err(CVG_ERR_INVALID, "idx/dist must not be NULL");
+    TrainSet ts;
+    const int64_t offs[2] = { 0, n_train };
+    layout_segments(ts, offs, 1);
+    CU_CHECK(c->t_f32.ensure((size_t)std::max(n_train, 1) * DIM * 4));
+    ts.d_f32 = c->t_f32.as<float>();
+    if (n_train > 0) CU_CHECK(cudaMemcpyAsync(ts.d_f32, train, (size_t)n_train * DIM * 4, cudaMemcpyHostToDevice, c->stream));
+    CU_CHECK(cudaMemsetAsync(c->d_flags, 0, 4, c->stream));
+    int rc = prep_train(c, ts, c->t_b, c->t_blo, c->t_aug, c->t_segtab, 0);
+    if (rc) return rc;
+    CU_CHECK(cudaMemcpyAsync(c->d_flags + 1, &q_nonint, 4, cudaMemcpyHostToDevice, c->stream));
+    combine_flags_kernel<<<1, 1, 0, c->stream>>>(c->d_flags, c->d_flags, (c->flags & CVG_FORCE_EXACT_MATCH) ? 4 : 0);
+    c->launches++;
+    std::vector<MatchUnit> units;
+    build_xc_plan(views, ts, c->n_sms, units);
+    const int V = (int)views.size(), n_units = (int)units.size();
+    int max_view_rows = 0;
+    for (const SegDev& v : views) max_view_rows = std::max(max_view_rows, v.rows);
+    const size_t n_cols_all = (size_t)V * n_train;
+    CU_CHECK(c->units.ensure(std::max<size_t>(units.size(), 1) * sizeof(MatchUnit)));
+    CU_CHECK(c->xc.ensure(64 + ((size_t)q.row_end + n_cols_all) * 8));            // XcOut, row keys (absolute rows), column keys
+    CU_CHECK(c->segdev.ensure((size_t)(V + 1) * sizeof(SegDev)));
+    CU_CHECK(c->fb.ensure(((size_t)nq + n_cols_all) * (sizeof(int2) + 16)));      // guard lists + their key pairs
+    CU_CHECK(c->idx.ensure((size_t)nq * 4)); CU_CHECK(c->dist.ensure((size_t)nq * 4));
+    XcOut xo;
+    xo.rowkey = reinterpret_cast<unsigned long long*>(c->xc.as<uint8_t>() + 64);
+    xo.colkey = xo.rowkey + q.row_end;
+    std::vector<SegDev> sd(views);
+    sd.push_back(SegDev{ 0, n_train, 0 });
+    CU_CHECK(cudaMemcpyAsync(c->xc.p, &xo, sizeof xo, cudaMemcpyHostToDevice, c->stream));
+    CU_CHECK(cudaMemcpyAsync(c->segdev.p, sd.data(), sd.size() * sizeof(SegDev), cudaMemcpyHostToDevice, c->stream));
+    if (n_units > 0)
+        CU_CHECK(cudaMemcpyAsync(c->units.p, units.data(), units.size() * sizeof(MatchUnit), cudaMemcpyHostToDevice, c->stream));
+    CU_CHECK(cudaMemsetAsync(xo.rowkey, 0xFF, ((size_t)q.row_end + n_cols_all) * 8, c->stream));
+    CU_CHECK(cudaMemsetAsync(c->d_flags + 20, 0, 8, c->stream));
+    // the candidate path (non-integer rows, tensor cores) has no cross-check form: those calls take the SIMT kernel
+    const bool want_tc = path_from_kinds(c->flags, q_nonint, -1) == 0;
+    TcOperands op{ q.d_b, q.d_aug, q.d_norm, q.n_pad, ts.d_b, ts.d_aug, (int)ts.rows_pad_total, q.d_blo, ts.d_blo };
+    TcMapsOpaque maps;
+    char err[256];
+    if (n_units > 0 && want_tc && tc_encode_maps(op, 1, &maps, err, sizeof err)) return set_err(CVG_ERR_CUDA, "%s", err);
+    const MatchUnit* d_units = c->units.as<MatchUnit>();
+    if (c->timing) cudaEventRecord(c->ev[3], c->stream);
+    if (n_units > 0) {
+        if (want_tc) {
+            if (launch_match_tc(op, &maps, d_units, n_units, c->xc.p, 1, c->d_flags + 2, 0, c->d_flags + 8, c->n_sms, c->stream, err, sizeof err))
+                return set_err(CVG_ERR_CUDA, "%s", err);
+            c->launches++;
+        }
+        launch_match_exact_xc(q.d_f32, ts.d_f32, d_units, n_units, xo, c->d_flags + 2, c->stream);
+        c->launches++;
+    }
+    if (c->timing) cudaEventRecord(c->ev[4], c->stream);
+    int2* lists = c->fb.as<int2>();
+    XcFinish w;
+    w.keys = xo; w.row_begin = q.row_begin; w.row_end = q.row_end;
+    w.n_views = V; w.n_train = n_train; w.max_view_rows = max_view_rows;
+    w.views = c->segdev.as<SegDev>(); w.train_seg = c->segdev.as<SegDev>() + V;
+    w.Q = q.d_f32; w.T = ts.d_f32;
+    w.guard_counts = c->d_flags + 20; w.guard_total = c->d_flags + 7;
+    w.row_list = lists; w.col_list = lists + nq;
+    w.row_g = reinterpret_cast<unsigned long long*>(lists + nq + n_cols_all); w.col_g = w.row_g + 2 * (size_t)nq;
+    w.gate_flag = c->d_flags + 2;
+    w.idx = c->idx.as<int32_t>(); w.dist = c->dist.as<float>();
+    w.n_sms = c->n_sms;
+    c->launches += launch_xc_finish(w, c->stream);
+    CU_CHECK(cudaGetLastError());
+    int flag = 0;
+    CU_CHECK(cudaMemcpyAsync(idx, c->idx.p, (size_t)nq * 4, cudaMemcpyDeviceToHost, c->stream));
+    CU_CHECK(cudaMemcpyAsync(dist, c->dist.p, (size_t)nq * 4, cudaMemcpyDeviceToHost, c->stream));
+    CU_CHECK(cudaMemcpyAsync(&flag, c->d_flags + 2, 4, cudaMemcpyDeviceToHost, c->stream));
+    rc = sync_and_check(c);
+    if (rc) return rc;
+    c->last_match_path = flag == 0 ? 1 : 2;
+    if (c->timing) { cudaEventElapsedTime(&c->t_match, c->ev[3], c->ev[4]); c->t_ransac = 0; c->t_total = c->t_match; }
+    return CVG_OK;
+}
+
+extern "C" {
+
+int cvg_match_cross_check(cvg_ctx* c, const cvg_models* m, int view, const float* train, int n_train, int32_t* idx, float* dist)
+{
+    c = cvg_primary(c); m = cvg_models_on(m, c);
+    if (!c || !m) return set_err(CVG_ERR_INVALID, "cvg_match_cross_check: NULL context/models");
+    if (view < -1 || view >= m->n_views) return set_err(CVG_ERR_INVALID, "cvg_match_cross_check: view %d of %d", view, m->n_views);
+    CU_CHECK(cudaSetDevice(c->device));
+    QuerySide q{ m->d_f32, m->d_b, m->d_blo, m->d_aug, m->d_norm, 0, m->n_rows, m->n_pad };
+    std::vector<SegDev> views;
+    for (int v = view < 0 ? 0 : view; v < (view < 0 ? m->n_views : view + 1); v++)
+        views.push_back(SegDev{ m->view_offsets[v], m->view_offsets[v + 1] - m->view_offsets[v], 0 });
+    if (view >= 0) { q.row_begin = m->view_offsets[view]; q.row_end = m->view_offsets[view + 1]; }
+    return match_cross_check(c, q, views, m->nonint, train, n_train, idx, dist);
+}
+
+int cvg_match_cross_check_raw(cvg_ctx* c, const float* query, int n_query, const float* train, int n_train, int32_t* idx,
+                              float* dist)
+{
+    c = cvg_primary(c);
+    if (!c) return set_err(CVG_ERR_INVALID, "cvg_match_cross_check_raw: NULL context");
+    if (n_query < 0 || (n_query > 0 && !query)) return set_err(CVG_ERR_INVALID, "bad query matrix");
+    if (n_query == 0) return CVG_OK;
+    CU_CHECK(cudaSetDevice(c->device));
+    QuerySide q; int qflag = 0;
+    const int rc = upload_raw_query(c, query, n_query, &q, &qflag);
+    if (rc) return rc;
+    return match_cross_check(c, q, std::vector<SegDev>{ SegDev{ 0, n_query, 0 } }, qflag, train, n_train, idx, dist);
 }
 
 // ---- verify stage ---------------------------------------------------------------------------------

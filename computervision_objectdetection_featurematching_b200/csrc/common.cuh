@@ -24,7 +24,7 @@ struct MatchUnit {
     int32_t part_slot;       // partial record block: parts[part_slot * TILE_M + row]
     int32_t seg_cols;        // valid train rows of the segment (for masking the padded tail)
     int32_t t_row0_f32;      // first train row in the unpadded fp32 train matrix (exact kernel)
-    int32_t pad1;
+    int32_t pad1;            // knn2 plan: 0.  Cross-check plan: view slot << 8 | query rows of the unit in its view (1..128)
 };
 
 // Partial / final top-2 record of one query row.
@@ -67,6 +67,32 @@ void launch_match_exact(const float* Q, int n_query, const float* T, const Match
                         Top2* parts, const int* gate_flag /*device flag: run only if *flag == gate_want, or NULL*/,
                         int gate_want, cudaStream_t st);
 
+// Cross-check (BFMatcher(NORM_L2, crossCheck = true)): the match kernels leave, per query row, the (key << 32 | train index)
+// of its nearest train row and, per (view slot, train column), the (key << 32 | absolute query row) of the column's nearest
+// query row of that view, both reduced with atomicMin (~0 = none).  key = d^2 (tensor-core kernel, integer rows) or the
+// float bits of cv2's distance (exact SIMT kernel); xc_finish turns d^2 into distance bits.
+struct XcOut { unsigned long long* rowkey; unsigned long long* colkey; };
+void launch_match_exact_xc(const float* Q, const float* T, const MatchUnit* units, int n_units, XcOut out,
+                           const int* gate_flag /*skipped if *flag == 0 (the tensor-core kernel serves the call), or NULL*/,
+                           cudaStream_t st);
+struct XcFinish {
+    XcOut keys;
+    int row_begin, row_end;                         // query rows of the call (rowkey is indexed by absolute row)
+    int n_views, n_train, max_view_rows;
+    const SegDev* views;                            // [n_views] query rows of each view slot (f32_row0 = first row)
+    const SegDev* train_seg;                        // [1] {0, n_train}
+    const float* Q; const float* T;                 // fp32 rows
+    int* guard_counts;                              // [2] rows / columns redone by the d >= 2048 guard (zeroed by the caller)
+    int* guard_total;                               // receives their sum
+    int2* row_list; unsigned long long* row_g;      // [nq], [2 * nq]
+    int2* col_list; unsigned long long* col_g;      // [n_views * n_train], [2 * n_views * n_train]
+    const int* gate_flag;                           // the d^2 -> distance step runs only if *gate_flag == 0 (tensor-core path)
+    int32_t* idx; float* dist;                      // [nq]
+    int n_sms;
+};
+// d^2 keys -> distance keys (the d >= 2048 rows and columns redone exactly), then the mutual test; returns the launch count
+int launch_xc_finish(const XcFinish& w, cudaStream_t st);
+
 // match_tc.cu — tcgen05 / TMEM / TMA kernel
 struct TcOperands {
     const __nv_bfloat16* Qb; const __nv_bfloat16* Qaug; const float* qnorm; int nq_pad;
@@ -76,7 +102,8 @@ struct TcOperands {
 int  tc_init(char* err, size_t errlen);     // resolves cuTensorMapEncodeTiled; 0 = ok
 int  tc_set_device_attrs(char* err, size_t errlen);       // dynamic shared memory opt-in on the CURRENT device
 int  ransac_set_device_attrs(char* err, size_t errlen);   // same for the verify kernels
-// candidates = 2: exact top-2 (Top2 parts[n_units][128]); 4: candidate records (Top4 parts[n_units][4][128]).
+// candidates = 2: exact top-2 (Top2 parts[n_units][128]); 4: candidate records (Top4 parts[n_units][4][128]);
+// 1: cross-check keys (parts = device XcOut, units of build_xc_plan).
 // gate_flag (device, may be NULL): the kernel runs only if *gate_flag == gate_want.
 // paired: the unit list is made of pairs (2p, 2p + 1) with the same train tiles (build_plan with an even number of row
 // blocks): the exact form then runs as clusters of two CTAs with cta_group::2 MMAs.

@@ -143,7 +143,8 @@ struct cvg_ctx {
     int* d_flags = nullptr;            // [0] train row kinds, [1] query row kinds, [2] match path (0 tensor exact, 1 tensor
                                        // candidates + re-rank, 2 exact SIMT), [3] raw-query kinds, [4] RNG table short,
                                        // [5] max ||t||^2 bits, [6] fallback row count, [7] rows the d >= 2048 guard redid, [8..16) kernel debug words,
-                                       // [17] sets the chunked sampler handed to the serial one, [18] max ||q||^2 bits (models upload), [19] niters entries to verify
+                                       // [17] sets the chunked sampler handed to the serial one, [18] max ||q||^2 bits (models upload), [19] niters entries to verify,
+                                       // [20..22) rows / columns the cross-check guard redid
     uint32_t* d_rng = nullptr; int64_t rng_len = 0;
     int last_match_path = 0; int64_t launches = 0;
     int timing = 0; float t_match = 0, t_ransac = 0, t_total = 0;
@@ -159,6 +160,7 @@ struct cvg_ctx {
     DevBuf hypH;                                       // fp32 models of the current round(s), read by ransac_score_kernel
     DevBuf chunk;                                      // chunked sampler scratch (huge no-early-stop rounds)
     DevBuf plan_units, plan_dir;                       // match plan of the fused path, cached by (model set, scene shapes)
+    DevBuf xc;                                         // cross-check: XcOut, row keys, column keys
     bool last_chunked = false;                         // the last verify call used the chunked sampler (d_flags[17] = sets it handed back)
     uint64_t plan_models_uid = 0; std::vector<int> plan_shape; int plan_units_n = 0;   // keyed on cvg_models::uid: addresses get reused
     DevBuf pts, starts, counts_n, sample_pos, n_samples, counts, best_iter, best_count, iters_run, niters_cur, smp_state, sel;

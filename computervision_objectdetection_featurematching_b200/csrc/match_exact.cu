@@ -7,6 +7,7 @@
 // It serves calls whose descriptors are not integer-valued; integer (SIFT) data takes match_tc.cu.
 #include "common.cuh"
 #include <float.h>
+#include <algorithm>
 
 namespace cvg {
 
@@ -81,6 +82,88 @@ void launch_match_exact(const float* Q, int n_query, const float* T, const Match
 {
     if (n_units <= 0) return;
     match_exact_kernel<<<n_units, EX_THREADS, 0, st>>>(Q, n_query, T, units, parts, gate_flag, gate_want);
+}
+
+// Cross-check form (BFMatcher(NORM_L2, crossCheck = true)) of the kernel above, for the units of build_xc_plan: the same
+// distances, each row's nearest column (strict <, ascending columns), and per train column its nearest query row of the
+// unit's view — the minimum over the CTA's rows of (distance bits, absolute row), non-negative floats ordering like their
+// bits — merged per column with one global atomicMin per unit.  NaN and inf enter neither side.
+__global__ void __launch_bounds__(EX_THREADS)
+match_exact_xc_kernel(const float* __restrict__ Q, const float* __restrict__ T, const MatchUnit* __restrict__ units,
+                      XcOut out, const int* __restrict__ gate_flag)
+{
+    if (gate_flag && *gate_flag == 0) return;                  // the tensor-core kernel serves the call
+    __shared__ float4 tile[EX_TROWS][DIM / 4];
+    __shared__ unsigned long long s_col[EX_TROWS];
+    const MatchUnit u = units[blockIdx.x];
+    const int qrow = u.q_row0 + threadIdx.x, lane = threadIdx.x & 31;
+    const bool qvalid = (int)threadIdx.x < (u.pad1 & 255);
+    float4 q[DIM / 4];
+    {
+        const float4* qp = reinterpret_cast<const float4*>(Q + (size_t)(qvalid ? qrow : u.q_row0) * DIM);
+        #pragma unroll
+        for (int j = 0; j < DIM / 4; j++) q[j] = qp[j];
+    }
+    unsigned long long* ck = out.colkey + (size_t)(u.pad1 >> 8) * u.seg_cols;
+    int n_cols = u.n_tiles * TILE_N;
+    if (n_cols > u.seg_cols - u.t_local0) n_cols = u.seg_cols - u.t_local0;
+    if (threadIdx.x < EX_TROWS) s_col[threadIdx.x] = ~0ull;
+    float bd = FLT_MAX;
+    int bi = -1;
+    for (int c0 = 0; c0 < n_cols; c0 += EX_TROWS) {
+        const int nr = min(EX_TROWS, n_cols - c0);
+        __syncthreads();
+        for (int e = threadIdx.x; e < nr * (DIM / 4); e += EX_THREADS) {
+            const int r = e / (DIM / 4), k = e % (DIM / 4);
+            tile[r][k] = reinterpret_cast<const float4*>(T + (size_t)(u.t_row0_f32 + c0 + r) * DIM)[k];
+        }
+        __syncthreads();
+        for (int r = 0; r < nr; r++) {
+            float acc[4][4];
+            #pragma unroll
+            for (int a = 0; a < 4; a++)
+                #pragma unroll
+                for (int l = 0; l < 4; l++) acc[a][l] = 0.f;
+            #pragma unroll
+            for (int j4 = 0; j4 < DIM / 4; j4++) {              // the order of match_exact_kernel (SURVEY App. A.3)
+                const float4 t = tile[r][j4];
+                const int a = j4 & 3;
+                float d;
+                d = __fsub_rn(q[j4].x, t.x); acc[a][0] = __fadd_rn(acc[a][0], __fmul_rn(d, d));
+                d = __fsub_rn(q[j4].y, t.y); acc[a][1] = __fadd_rn(acc[a][1], __fmul_rn(d, d));
+                d = __fsub_rn(q[j4].z, t.z); acc[a][2] = __fadd_rn(acc[a][2], __fmul_rn(d, d));
+                d = __fsub_rn(q[j4].w, t.w); acc[a][3] = __fadd_rn(acc[a][3], __fmul_rn(d, d));
+            }
+            float v[4];
+            #pragma unroll
+            for (int l = 0; l < 4; l++)
+                v[l] = __fadd_rn(__fadd_rn(__fadd_rn(acc[0][l], acc[1][l]), acc[2][l]), acc[3][l]);
+            const float dist = sqrtf(__fadd_rn(__fadd_rn(v[0], v[2]), __fadd_rn(v[1], v[3])));
+            const bool ok = qvalid && dist < FLT_MAX;
+            if (ok && dist < bd) { bd = dist; bi = u.t_local0 + c0 + r; }
+            unsigned long long key = ok ? ((unsigned long long)__float_as_uint(dist) << 32) | (unsigned int)qrow : ~0ull;
+            #pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                const unsigned long long other = __shfl_xor_sync(0xffffffffu, key, o);
+                key = other < key ? other : key;
+            }
+            if (lane == 0 && key != ~0ull) atomicMin(&s_col[r], key);
+        }
+        __syncthreads();
+        if ((int)threadIdx.x < nr) {
+            const unsigned long long k = s_col[threadIdx.x];
+            s_col[threadIdx.x] = ~0ull;
+            if (k != ~0ull) atomicMin(&ck[u.t_local0 + c0 + threadIdx.x], k);
+        }
+    }
+    if (bi >= 0) atomicMin(&out.rowkey[qrow], ((unsigned long long)__float_as_uint(bd) << 32) | (unsigned int)bi);
+}
+
+void launch_match_exact_xc(const float* Q, const float* T, const MatchUnit* units, int n_units, XcOut out,
+                           const int* gate_flag, cudaStream_t st)
+{
+    if (n_units <= 0) return;
+    match_exact_xc_kernel<<<n_units, EX_THREADS, 0, st>>>(Q, T, units, out, gate_flag);
 }
 
 // ---- merge: lexicographic (distance, train index), the order that reproduces OpenCV's tie rule ----
@@ -372,6 +455,102 @@ void launch_fallback_exact(const int* fb_count, const int2* fb_list, unsigned lo
     fallback_emit_kernel<<<n_sms, 256, 0, st>>>(fb_count, fb_list, n_query, ratio, g1, g2, idx, dist, accept, gate_flag, gate_want);
 }
 
+
+// ---- cross-check: distances, the d >= 2048 guard, the mutual test -------------------------------------
+constexpr unsigned long long XC_NONE = ~0ull;
+constexpr uint32_t XC_GUARD_D2 = 1u << 22;                 // d = 2048: from here on distinct d^2 can share a float distance
+
+// Tensor-core path only: the keys hold d^2.  Below 2^22 the order by (d^2, index) is cv2's order by (sqrtf(d^2), index) — every
+// d^2 < 2^22 keeps its own float distance, and every larger d^2 has a distance >= 2048 — so the key becomes (distance bits,
+// index).  A row or column whose best d^2 reaches 2^22 is listed for the exact scan instead.
+__global__ void xc_distance_kernel(XcOut k, int row_begin, int n_rows, int64_t n_cols_all, int n_train, int* __restrict__ counts,
+                                   int2* __restrict__ row_list, int2* __restrict__ col_list, const int* __restrict__ gate_flag)
+{
+    if (gate_flag && *gate_flag != 0) return;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < (int64_t)n_rows + n_cols_all; e += (int64_t)gridDim.x * blockDim.x) {
+        const bool is_row = e < n_rows;
+        unsigned long long* p = is_row ? &k.rowkey[row_begin + e] : &k.colkey[e - n_rows];
+        const unsigned long long v = *p;
+        if (v == XC_NONE) continue;
+        const uint32_t d2 = (uint32_t)(v >> 32);
+        if (d2 >= XC_GUARD_D2) {
+            if (is_row) row_list[atomicAdd(&counts[0], 1)] = make_int2(0, row_begin + (int)e);
+            else { const int64_t c = e - n_rows; col_list[atomicAdd(&counts[1], 1)] = make_int2((int)(c / n_train), (int)(c % n_train)); }
+        } else {
+            *p = ((unsigned long long)__float_as_uint(sqrtf((float)d2)) << 32) | (v & 0xFFFFFFFFull);
+        }
+    }
+}
+
+// the exact scans' results into the key arrays (a column's scan ran over its view's rows: local row -> absolute row)
+__global__ void xc_apply_kernel(XcOut k, int n_train, const SegDev* __restrict__ views, const int* __restrict__ counts,
+                                const int2* __restrict__ row_list, const unsigned long long* __restrict__ row_g,
+                                const int2* __restrict__ col_list, const unsigned long long* __restrict__ col_g, int* __restrict__ guard_total)
+{
+    const int nr = counts[0], nc = counts[1];
+    if (blockIdx.x == 0 && threadIdx.x == 0) *guard_total = nr + nc;
+    for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < nr + nc; e += gridDim.x * blockDim.x) {
+        if (e < nr) { k.rowkey[row_list[e].y] = row_g[e]; continue; }
+        const int2 vc = col_list[e - nr];
+        const unsigned long long g = col_g[e - nr];
+        k.colkey[(size_t)vc.x * n_train + vc.y] =
+            g == XC_NONE ? XC_NONE : (g & 0xFFFFFFFF00000000ull) | (unsigned int)(views[vc.x].f32_row0 + (int)(unsigned int)g);
+    }
+}
+
+// row i of view slot v, nearest column j: a match iff column j's nearest row in view v is i
+__global__ void xc_emit_kernel(XcOut k, int row_begin, int n_views, int n_train, const SegDev* __restrict__ views,
+                               int32_t* __restrict__ idx, float* __restrict__ dist)
+{
+    const int x = blockIdx.x * blockDim.x + threadIdx.x;
+    for (int v = blockIdx.y; v < n_views; v += gridDim.y) {
+        const SegDev vw = views[v];
+        if (x >= vw.rows) continue;
+        const int row = (int)vw.f32_row0 + x;
+        const unsigned long long rk = k.rowkey[row];
+        int j = -1;
+        float d = 0.f;
+        if (rk != XC_NONE) {
+            const int c = (int)(unsigned int)rk;
+            if ((unsigned int)k.colkey[(size_t)v * n_train + c] == (unsigned int)row) { j = c; d = __uint_as_float((unsigned int)(rk >> 32)); }
+        }
+        idx[row - row_begin] = j;
+        dist[row - row_begin] = d;
+    }
+}
+
+int launch_xc_finish(const XcFinish& w, cudaStream_t st)
+{
+    const int nq = w.row_end - w.row_begin;
+    const int64_t n_cols_all = (int64_t)w.n_views * w.n_train;
+    if (nq <= 0) return 0;
+    int launches = 0;
+    if (n_cols_all > 0) {
+        const int64_t n = nq + n_cols_all;
+        xc_distance_kernel<<<(unsigned)std::min<int64_t>((n + 255) / 256, (int64_t)w.n_sms * 8), 256, 0, st>>>(
+            w.keys, w.row_begin, nq, n_cols_all, w.n_train, w.guard_counts, w.row_list, w.col_list, w.gate_flag);
+        // exact scans of the listed rows (over the train rows) and columns (over their view's rows, roles swapped); empty
+        // loops when nothing is listed
+        unsigned long long* rg1 = w.row_g; unsigned long long* rg2 = w.row_g + nq;
+        unsigned long long* cg1 = w.col_g; unsigned long long* cg2 = w.col_g + n_cols_all;
+        fallback_init_kernel<<<w.n_sms, 256, 0, st>>>(&w.guard_counts[0], rg1, rg2, nullptr, 0);
+        fallback_init_kernel<<<w.n_sms, 256, 0, st>>>(&w.guard_counts[1], cg1, cg2, nullptr, 0);
+        fallback_scan_kernel<<<w.n_sms * 8, FB_THREADS, 0, st>>>(&w.guard_counts[0], w.row_list, w.train_seg,
+                                                                 (w.n_train + FB_CHUNK - 1) / FB_CHUNK, w.Q, 0, w.T, rg1, rg2, 1, nullptr, 0);
+        fallback_scan_kernel<<<w.n_sms * 8, FB_THREADS, 0, st>>>(&w.guard_counts[1], w.col_list, w.views,
+                                                                 (w.max_view_rows + FB_CHUNK - 1) / FB_CHUNK, w.T, 0, w.Q, cg1, cg2, 1, nullptr, 0);
+        xc_apply_kernel<<<w.n_sms, 256, 0, st>>>(w.keys, w.n_train, w.views, w.guard_counts, w.row_list, rg1, w.col_list, cg1,
+                                                   w.guard_total);
+        launches += 6;
+    }
+    // rows outside every view (models whose first view starts after row 0) keep no match
+    cudaMemsetAsync(w.idx, 0xFF, (size_t)nq * 4, st);
+    cudaMemsetAsync(w.dist, 0, (size_t)nq * 4, st);
+    if (w.max_view_rows <= 0 || w.n_views <= 0) return launches;
+    xc_emit_kernel<<<dim3((unsigned)((w.max_view_rows + 255) / 256), (unsigned)std::min(w.n_views, 65535)), 256, 0, st>>>(
+        w.keys, w.row_begin, w.n_views, w.n_train, w.views, w.idx, w.dist);
+    return launches + 1;
+}
 
 // merge of n_parts partial results laid out [n_parts][n_query][2] (multi-GPU train-tile shards)
 __global__ void merge_parts_kernel(const float* __restrict__ dparts, const int32_t* __restrict__ iparts,

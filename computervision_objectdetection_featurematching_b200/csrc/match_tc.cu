@@ -20,6 +20,11 @@
 // issues: inside an `if (lane == 0)` region ptxas wraps each tcgen05.mma / commit / TMA instruction in an election loop
 // and moves every descriptor through R2UR, ~250 instructions per tile instead of ~60 (DESIGN.md 4.1: 1.11 -> 0.96 ms).
 //
+// Cross-check form (KP = 1, BFMatcher(NORM_L2, crossCheck = true)): the same producer, MMA issuer and accumulator; the
+// epilogue keeps each query row's nearest column and, per tile, reduces each train column to its nearest query row of the
+// unit's view (redux.sync per warp, shared atomicMin over the four TMEM lane quarters, one global atomicMin per column and
+// unit).  DESIGN.md 4.5.
+//
 // Pair mode (template PAIR, opt-in: CVG_MATCH_PAIR_MODE): the same kernel as clusters of two CTAs around
 // tcgen05.mma.cta_group::2 (M256 N256 K16): each CTA holds its own query tile and half of every train stage, TMA loads
 // are counted on the leader CTA's barriers, the leader issues the MMAs and multicasts its commits to both CTAs, both
@@ -62,6 +67,10 @@ constexpr uint32_t SCRATCH_BYTES = 3 * TILE_M * 16;                 // partial t
 constexpr uint32_t OFF_SHARE = OFF_SCRATCH + SCRATCH_BYTES;         // running (best, second best) of every column part, per row
 constexpr uint32_t SHARE_BYTES = 4 * TILE_M * 8;                    //                              4 KB
 constexpr uint32_t OFF_BAR = OFF_SHARE + SHARE_BYTES;
+// cross-check form: the row merge (3 parts x 128 rows x 8 B) and the 16 tile counters live in the scratch area, the column
+// keys of four tiles (4 x 256 x 4 B) in the share area
+constexpr uint32_t XC_MERGE_BYTES = 3 * TILE_M * 8;
+static_assert(XC_MERGE_BYTES + 16 * 4 <= SCRATCH_BYTES && 4 * TILE_N * 4 <= SHARE_BYTES, "cross-check shared memory");
 constexpr uint32_t TC_SMEM_SLACK = 512;                           // the dynamic window is 1024-aligned in practice; checked in the kernel
 constexpr uint32_t TC_SMEM_BYTES = OFF_BAR + 512 + TC_SMEM_SLACK;
 static_assert(TC_SMEM_BYTES <= 232448, "shared memory budget of one CTA (227 KB)");
@@ -392,8 +401,38 @@ __device__ __forceinline__ void top4_scan32(const uint32_t* r, int c0, float (&b
     }
 }
 
+// ---- cross-check epilogue (KP = 1) ----
+// Nearest column of a row over 32 more columns: larger acc' wins, ties keep the lower column (the ascending scan's strict >).
+__device__ __forceinline__ void xc_row_scan32(const uint32_t* r, int c0, float& b1, int& i1)
+{
+    float m = __uint_as_float(r[0]);
+    #pragma unroll
+    for (int k = 1; k < 32; k++) m = fmaxf(m, __uint_as_float(r[k]));
+    if (m > b1) {
+        int j = 31;
+        #pragma unroll
+        for (int k = 30; k >= 0; k--) j = (__uint_as_float(r[k]) == m) ? k : j;
+        b1 = m; i1 = c0 + j;
+    }
+}
+// Column keys of 32 columns for this warp's 32 rows, reduced over the warp and merged into the tile's shared slots.
+// qbias = ||q||^2 + 2^23 (exact: ||q||^2 < 2^23 for rows of 0..255), so qbias - acc' = d^2 + 2^23 exactly and its float
+// bits are 0x4B000000 + d^2: shifted left by 7 (the constant part wraps to 0x80000000) and or-ed with the row in the tile,
+// the key orders by (d^2, row) and stays <= 0xBFFFFFFF.  Rows outside the unit's view have qbias = inf: key 0xC00000xx.
+constexpr uint32_t XC_KEY_ABSENT = 0xC0000000u;
+__device__ __forceinline__ void xc_col_keys32(const uint32_t* r, float qbias, uint32_t row, uint32_t* slots, int lane)
+{
+    #pragma unroll
+    for (int k = 0; k < 32; k++) {
+        const uint32_t key = (__float_as_uint(__fsub_rn(qbias, __uint_as_float(r[k]))) << 7) | row;
+        const uint32_t m = __reduce_min_sync(0xffffffffu, key);
+        if (lane == 0) atomicMin(&slots[k], m);
+    }
+}
+
 struct TcMaps { CUtensorMap q, qaug, t, taug, qlo, tlo, th, taugh; };   // th / taugh: 128-row boxes of the train operand (pair mode)
 
+// KP = 1: cross-check keys (integer descriptors), parts_out = XcOut; units of build_xc_plan.
 // KP = 2: exact top-2 per row (integer descriptors), partial records Top2 with distances.
 // KP = 4: four candidates per row and column part (non-integer descriptors), partial records Top4 with raw
 //         accumulator values, slot (part_slot * 4 + column part).
@@ -653,7 +692,13 @@ match_tc_kernel(const __grid_constant__ TcMaps maps, const float* __restrict__ q
         uint32_t t_full_r = t_full, t_empty_r = t_empty;
         uint32_t tmem_q = tmem_base + ((uint32_t)(quarter * 32) << 16);      // this warp's TMEM lane quarter (same treatment)
         asm volatile("" : "+r"(t_full_r), "+r"(t_empty_r), "+r"(tmem_q));
-        share_store(my_share, -INFINITY, -INFINITY);
+        if constexpr (KP == 1) {
+            // the share area holds the column keys of four tiles, the scratch area the row merge and the tiles' counters
+            reinterpret_cast<uint2*>(smem + OFF_SHARE)[ew * 32 + lane] = make_uint2(0xFFFFFFFFu, 0xFFFFFFFFu);
+            if (ew == 0 && lane < 16) reinterpret_cast<int*>(smem + OFF_SCRATCH + XC_MERGE_BYTES)[lane] = 0;
+        } else {
+            share_store(my_share, -INFINITY, -INFINITY);
+        }
         asm volatile("bar.sync 1, %0;" :: "n"(32 * TC_EPI_WARPS) : "memory");
         if constexpr (KP == 2) {
             uint32_t tc = 0;
@@ -819,7 +864,7 @@ match_tc_kernel(const __grid_constant__ TcMaps maps, const float* __restrict__ q
                 o[0] = (int)c_tiles; o[1] = (int)(c_wait / 64); o[2] = (int)(c_share / 64); o[3] = (int)(c_ld / 64); o[4] = (int)(c_scan / 64);
                 o[5] = (int)(c_flush / 64); o[6] = (int)(c_unit / 64); o[7] = (int)((clock64() - t_start) / 64);
             }
-        } else {
+        } else if constexpr (KP == 4) {
             uint32_t tc = 0;
             for (int e = worker; e < n_entries; e += n_workers) {
                 const MatchUnit un = units[unit_of(e)];
@@ -864,6 +909,78 @@ match_tc_kernel(const __grid_constant__ TcMaps maps, const float* __restrict__ q
                 reinterpret_cast<Top4*>(parts_out)[((size_t)un.part_slot * 4 + part) * TILE_M + row_in_tile] = out;
                 asm volatile("bar.sync 1, %0;" :: "n"(32 * TC_EPI_WARPS) : "memory");     // all share slots reset before the next unit
             }
+        } else {
+            // Cross-check.  Column keys: tile tc's 256 columns have slots in buffer tc & 3; the four warps of a column part
+            // (one per TMEM lane quarter) merge into them with atomicMin, and the last of the four to count itself in flushes
+            // the 64 columns to global memory and resets the slots.  No per-tile barrier: a warp is at most two tiles ahead of
+            // the slowest (the accumulator of tile T + 2 needs every warp's release of tile T), and the flusher of tile T
+            // finishes it before it releases tile T + 1, so buffer tc & 3 is free again when tile tc + 4 arrives.
+            uint32_t* colkeys = reinterpret_cast<uint32_t*>(smem + OFF_SHARE);                 // [4 tiles][256 columns]
+            float2* rmerge = reinterpret_cast<float2*>(smem + OFF_SCRATCH);                    // [3 column parts][128 rows]
+            int* colcnt = reinterpret_cast<int*>(smem + OFF_SCRATCH + XC_MERGE_BYTES);         // [4 tiles][4 column parts]
+            const XcOut xo = *reinterpret_cast<const XcOut*>(parts_out);
+            uint32_t tc = 0;
+            for (int e = worker; e < n_entries; e += n_workers) {
+                const MatchUnit un = units[unit_of(e)];
+                const bool row_ok = row_in_tile < (un.pad1 & 255);
+                const float qbias = row_ok ? __fadd_rn(qnorm[un.q_row0 + row_in_tile], 8388608.f) : INFINITY;
+                unsigned long long* ck = xo.colkey + (size_t)(un.pad1 >> 8) * un.seg_cols;
+                float b1 = -INFINITY;
+                int i1 = -1;
+                for (int t = 0; t < un.n_tiles; t++, tc++) {
+                    const uint32_t acc = tc & 1;
+                    mbar_wait(t_full_r + 8 * acc, (tc >> 1) & 1, dbg, 6);
+                    tc_fence_after();
+                    const uint32_t tbase = tmem_q + acc * TILE_N + part * 64;
+                    const int col_base = un.t_local0 + t * TILE_N + part * 64;
+                    uint32_t ra[32], rb[32];
+                    tc_ld32(tbase, ra);
+                    tc_ld32(tbase + 32, rb);
+                    tc_wait_ld();
+                    tc_fence_before();
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive(t_empty_r + 8 * acc);
+                    xc_row_scan32(ra, col_base, b1, i1);
+                    xc_row_scan32(rb, col_base + 32, b1, i1);
+                    uint32_t* slots = colkeys + (tc & 3) * TILE_N + part * 64;
+                    xc_col_keys32(ra, qbias, (uint32_t)row_in_tile, slots, lane);
+                    xc_col_keys32(rb, qbias, (uint32_t)row_in_tile, slots + 32, lane);
+                    __syncwarp();
+                    int last = 0;
+                    if (lane == 0) {
+                        __threadfence_block();
+                        last = atomicAdd(&colcnt[(tc & 3) * 4 + part], 1) == 3;
+                    }
+                    if (__shfl_sync(0xffffffffu, last, 0)) {
+                        __threadfence_block();
+                        #pragma unroll
+                        for (int h = 0; h < 2; h++) {
+                            const uint32_t k = atomicExch(&slots[h * 32 + lane], 0xFFFFFFFFu);
+                            const int col = col_base + h * 32 + lane;
+                            if (k < XC_KEY_ABSENT && col < un.seg_cols)
+                                atomicMin(&ck[col], ((unsigned long long)((k >> 7) & 0x7FFFFFu) << 32) | (uint32_t)(un.q_row0 + (int)(k & 127u)));
+                        }
+                        if (lane == 0) colcnt[(tc & 3) * 4 + part] = 0;
+                    }
+                }
+                // ---- unit flush: merge the four column parts (larger acc', then lower column), one key per row ----
+                if (b1 < ABSENT_BELOW) i1 = -1;
+                if (part > 0) rmerge[(part - 1) * TILE_M + row_in_tile] = make_float2(b1, __int_as_float(i1));
+                asm volatile("bar.sync 1, %0;" :: "n"(32 * TC_EPI_WARPS) : "memory");
+                if (part == 0) {
+                    #pragma unroll
+                    for (int pp = 0; pp < 3; pp++) {
+                        const float2 o = rmerge[pp * TILE_M + row_in_tile];
+                        const int i = __float_as_int(o.y);
+                        if (i >= 0 && (i1 < 0 || o.x > b1 || (o.x == b1 && i < i1))) { b1 = o.x; i1 = i; }
+                    }
+                    if (row_ok && i1 >= 0) {
+                        const uint32_t d2 = __float_as_uint(__fsub_rn(qbias, b1)) - 0x4B000000u;
+                        atomicMin(&xo.rowkey[un.q_row0 + row_in_tile], ((unsigned long long)d2 << 32) | (uint32_t)i1);
+                    }
+                }
+                asm volatile("bar.sync 1, %0;" :: "n"(32 * TC_EPI_WARPS) : "memory");
+            }
         }
     }
     tc_fence_before();
@@ -902,11 +1019,12 @@ int tc_init(char* err, size_t errlen)
 // context is created on (api.cu, under its own mutex), with that device current.
 int tc_set_device_attrs(char* err, size_t errlen)
 {
-    const void* fns[6] = { (const void*)match_tc_kernel<2, false, false>, (const void*)match_tc_kernel<2, false, true>,
+    const void* fns[7] = { (const void*)match_tc_kernel<2, false, false>, (const void*)match_tc_kernel<2, false, true>,
                            (const void*)match_tc_kernel<4, false, false>, (const void*)match_tc_kernel<4, false, true>,
-                           (const void*)match_tc_kernel<2, true, false>, (const void*)match_tc_kernel<2, true, true> };
+                           (const void*)match_tc_kernel<2, true, false>, (const void*)match_tc_kernel<2, true, true>,
+                           (const void*)match_tc_kernel<1, false, false> };
     cudaError_t e = cudaSuccess;
-    for (int i = 0; i < 6 && e == cudaSuccess; i++)
+    for (int i = 0; i < 7 && e == cudaSuccess; i++)
         e = cudaFuncSetAttribute(fns[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_BYTES);
     if (e != cudaSuccess) {
         snprintf(err, errlen, "cudaFuncSetAttribute(match_tc_kernel): %s", cudaGetErrorString(e));
@@ -972,7 +1090,9 @@ int launch_match_tc(const TcOperands& op, const TcMapsOpaque* encoded, const Mat
     const int grid = n_units < n_sms ? n_units : n_sms;
     static int exp_mode = -1;
     if (exp_mode < 0) { const char* e = getenv("CVG_TC_EXP"); exp_mode = e ? atoi(e) : 0; }
-    if (candidates == 4) {
+    if (candidates == 1)
+        match_tc_kernel<1, false, false><<<grid, TC_THREADS, TC_SMEM_BYTES, st>>>(maps, op.qnorm, units, n_units, parts, gate_flag, gate_want, dbg, 0);
+    else if (candidates == 4) {
         if (exp_mode) match_tc_kernel<4, false, true><<<grid, TC_THREADS, TC_SMEM_BYTES, st>>>(maps, op.qnorm, units, n_units, parts, gate_flag, gate_want, dbg, exp_mode);
         else match_tc_kernel<4, false, false><<<grid, TC_THREADS, TC_SMEM_BYTES, st>>>(maps, op.qnorm, units, n_units, parts, gate_flag, gate_want, dbg, 0);
     }

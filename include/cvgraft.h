@@ -205,6 +205,26 @@ int  cvg_match_knn2_raw(cvg_ctx* ctx, const float* query, int n_query,
                         const float* train, int n_train, float ratio,
                         int32_t* idx, float* dist, uint8_t* accept);
 
+/* BFMatcher(NORM_L2, crossCheck = true).match(query, train): src/TestsDetector.cpp:36,59-60 with crossCheck on, the usual
+ * alternative to the ratio test.  Query row i is matched to train row j exactly when j is i's nearest train row (ties ->
+ * lower train index) and i is j's nearest query row (ties -> lower query row); there is no ratio test and no second choice.
+ * Outputs, per query row i in order:
+ *   idx[i]   the matched train index, or -1
+ *   dist[i]  its L2 distance (fp32, as DMatch.distance), 0 when idx[i] = -1
+ * view >= 0: the rows of that view are the query matrix.  view == -1: every view, view after view, is its OWN query
+ * matrix — a train row's nearest query row is looked for among the rows of one view — which is what a loop over the views
+ * returns (the reference's loop), not the result of one call on the concatenated rows.  n_train == 0 gives idx = -1
+ * everywhere (cv2 fails an assertion).  NaN/inf distances are never returned.  Integer descriptors 0..255 (SIFT) take
+ * the tcgen05 tensor-core kernel (cvg_last_match_path 1; rows or columns at d >= 2048 are redone exactly,
+ * cvg_last_match_guard_rows); any other rows, and CVG_FORCE_EXACT_MATCH, take the exact fp32 SIMT kernel (path 2),
+ * which is slow: it is meant for correctness, not throughput.  On a multi-device context the call runs on the first GPU.
+ * cvg_last_timing reports the match kernel's time as match_ms. */
+int  cvg_match_cross_check(cvg_ctx* ctx, const cvg_models* models, int view, const float* train, int n_train,
+                           int32_t* idx, float* dist);
+/* Same for an arbitrary query matrix [n_query,128] in host memory (one query matrix). */
+int  cvg_match_cross_check_raw(cvg_ctx* ctx, const float* query, int n_query, const float* train, int n_train,
+                               int32_t* idx, float* dist);
+
 /* ---- verify stage: replaces src/TestsDetector.cpp:77-79 --------------------------------------
  * findHomography(src, dst, RANSAC, p->threshold, mask, p->max_iters, p->confidence).
  * H gets the 3x3 CV_64F result (zeros if none), mask [n] the returned inlier mask, *found = 0 iff
@@ -359,7 +379,7 @@ int  cvg_dev_merge_top2(cvg_ctx* ctx, void* stream, const float* dist_parts_dev,
  * descriptors, what SIFT emits); 3 = tcgen05 kernel on hi/lo split bf16 operands keeping four candidates per row,
  * then an fp32 re-rank in cv::batchDistance's summation order that proves the answer with an error bound
  * (non-integer descriptors; unproven rows are redone exactly); 2 = exact fp32 SIMT kernel (CVG_FORCE_EXACT_MATCH,
- * non-finite values); 0 = none yet.  Results are cv2's bit for bit on every path. */
+ * non-finite values); 0 = none yet.  Results are cv2's bit for bit on every path.  Cross-check calls report 1 or 2. */
 int  cvg_last_match_path(const cvg_ctx* ctx);
 /* Rows of the last path-3 call that the re-rank could not prove and the exact fallback kernel redid. */
 int  cvg_last_match_fallback_rows(const cvg_ctx* ctx);
@@ -367,7 +387,8 @@ int  cvg_last_match_fallback_rows(const cvg_ctx* ctx);
  * neighbouring integer d^2 round to one float (u8 rows reach d = 2885; SIFT rows, norm 512, stay below 1024).
  * Rows whose second distance reaches 2048 are redone by the exact kernels, which compare rounded distances:
  * how many rows of the last path-1 call that was.  When the norms of both sides are known on the host and
- * ||q|| + ||t|| < 2047 the guard is not even enqueued. */
+ * ||q|| + ||t|| < 2047 the guard is not even enqueued.  After cvg_match_cross_check(_raw): the query rows whose nearest
+ * distance, plus the train columns whose nearest distance in a view, reached 2048 and were redone exactly. */
 int  cvg_last_match_guard_rows(const cvg_ctx* ctx);
 /* Verify calls with CVG_RANSAC_NO_EARLY_STOP and max_iters >= 32768 cut every set's cv::RNG draw stream into
  * chunks walked by many CTAs (same samples as the serial walk).  Returns how many sets of the last such call
