@@ -8,7 +8,8 @@
     Context.estimate_affine_partial2d <- cv::estimateAffinePartial2D(src, dst, inliers, RANSAC)
     Context.detect_pairs      <- body of the view loop of detectAtScale             :58-95
                                  (detect_params(method=...): findHomography, estimateAffine2D or
-                                 estimateAffinePartial2D as its geometric check)
+                                 estimateAffinePartial2D as its geometric check; detect_params(cross_check=True):
+                                 BFMatcher(NORM_L2, crossCheck=true).match instead of knnMatch + ratio test)
     Models                    <- ObjectModel descriptors resident in HBM            include/objectModel.hpp:11-16
 
 Error behaviour follows OpenCV where the reference relies on it: find_homography raises for n < 4.
@@ -28,7 +29,8 @@ FORCE_EXACT_MATCH = 1
 MATCH_PAIR_MODE = 2
 NITERS_ALL_ON_HOST = 4
 PATH_TENSOR, PATH_EXACT, PATH_TENSOR_RERANK = 1, 2, 3   # cvg_last_match_path
-VERIFY_HOMOGRAPHY, VERIFY_AFFINE, VERIFY_AFFINE_PARTIAL = range(3)   # cvg_detect_params.method
+VERIFY_HOMOGRAPHY, VERIFY_AFFINE, VERIFY_AFFINE_PARTIAL = range(3)   # cvg_detect_params.method & 0xFF
+MATCH_CROSS_CHECK = 0x100                                             # cvg_detect_params.method flag (CVG_MATCH_CROSS_CHECK)
 
 PAIR_DTYPE = np.dtype([("status", "<i4"), ("n_good", "<i4"), ("n_inliers", "<i4"), ("ransac_iters", "<i4"),
                        ("H", "<f8", (9,)), ("det", "<f8")])
@@ -68,17 +70,18 @@ def affine_params(threshold=3.0, max_iters=2000, confidence=0.99, refine_iters=1
 
 
 def detect_params(ratio=0.9, min_inliers=4, det_lo=0.1, det_hi=10.0, ransac=None, method=VERIFY_HOMOGRAPHY,
-                  refine_iters=10):
+                  refine_iters=10, cross_check=False):
     """Constants of the fused path.  method picks its geometric check: VERIFY_HOMOGRAPHY (findHomography), VERIFY_AFFINE
     (estimateAffine2D) or VERIFY_AFFINE_PARTIAL (estimateAffinePartial2D, refineIters = refine_iters).  The affine methods
     read ransac's threshold, max_iters and confidence as given: pass ransac_params(3.0, 2000, 0.99) for OpenCV's affine
-    defaults."""
+    defaults.  cross_check=True sets MATCH_CROSS_CHECK in method: the correspondences are the mutual nearest neighbours of
+    BFMatcher(NORM_L2, crossCheck=true).match (each view its own query matrix) and ratio is ignored."""
     p = DetectParams()
     _lib.load().cvg_detect_params_default(C.byref(p))
     p.ratio = ratio; p.min_inliers = min_inliers; p.det_lo = det_lo; p.det_hi = det_hi
     if ransac is not None:
         p.ransac = ransac
-    p.method = method; p.refine_iters = refine_iters
+    p.method = method | (MATCH_CROSS_CHECK if cross_check else 0); p.refine_iters = refine_iters
     return p
 
 

@@ -451,33 +451,36 @@ static void build_plan(const QuerySide& q, const TrainSet& ts, int n_sms, std::v
     units.swap(sorted);
 }
 
-// Cross-check plan (one train segment): 128-row blocks of each view, starting at the view's first row — the padded query
-// operand holds such a tile (DESIGN.md 2) — against runs of train tiles.  A unit carries its view slot and how many of
-// its rows belong to the view (MatchUnit::pad1); the row side needs no merge directory (atomicMin keys).  Largest first.
+// Cross-check plan: 128-row blocks of each view, starting at the view's first row — the padded query operand holds such a
+// tile (DESIGN.md 2) — against runs of train tiles of each segment, the run length of build_plan.  A unit carries its
+// segment (MatchUnit::part_slot), its view slot and how many of its rows belong to the view (MatchUnit::pad1); the row
+// side needs no merge directory (atomicMin keys).  Largest first.
 static void build_xc_plan(const std::vector<SegDev>& views, const TrainSet& ts, int n_sms, std::vector<MatchUnit>& units)
 {
     units.clear();
-    const SegInfo& g = ts.segs[0];
-    if (g.rows == 0) return;
     int64_t n_rb = 0;
     for (const SegDev& v : views) n_rb += (v.rows + TILE_M - 1) / TILE_M;
     const int ch = plan_chunk_len(n_rb, ts, n_sms);
-    const int n_chunks = (g.ct + ch - 1) / ch;
-    for (size_t s = 0; s < views.size(); s++)
-        for (int rb = 0; rb * TILE_M < views[s].rows; rb++)
-            for (int ck = 0; ck < n_chunks; ck++) {
-                const int t0 = (int)((int64_t)g.ct * ck / n_chunks), t1 = (int)((int64_t)g.ct * (ck + 1) / n_chunks);
-                MatchUnit u;
-                u.q_row0 = (int32_t)views[s].f32_row0 + rb * TILE_M;
-                u.t_row0 = t0 * TILE_N;
-                u.n_tiles = t1 - t0;
-                u.t_local0 = t0 * TILE_N;
-                u.part_slot = 0;
-                u.seg_cols = g.rows;
-                u.t_row0_f32 = t0 * TILE_N;
-                u.pad1 = (int32_t)(s << 8) | std::min(TILE_M, views[s].rows - rb * TILE_M);
-                units.push_back(u);
-            }
+    for (int sg = 0; sg < ts.n_segs; sg++) {
+        const SegInfo& g = ts.segs[(size_t)sg];
+        if (g.rows == 0) continue;
+        const int n_chunks = (g.ct + ch - 1) / ch;
+        for (size_t s = 0; s < views.size(); s++)
+            for (int rb = 0; rb * TILE_M < views[s].rows; rb++)
+                for (int ck = 0; ck < n_chunks; ck++) {
+                    const int t0 = (int)((int64_t)g.ct * ck / n_chunks), t1 = (int)((int64_t)g.ct * (ck + 1) / n_chunks);
+                    MatchUnit u;
+                    u.q_row0 = (int32_t)views[s].f32_row0 + rb * TILE_M;
+                    u.t_row0 = (int32_t)(g.pad_row0 + (int64_t)t0 * TILE_N);
+                    u.n_tiles = t1 - t0;
+                    u.t_local0 = t0 * TILE_N;
+                    u.part_slot = sg;
+                    u.seg_cols = g.rows;
+                    u.t_row0_f32 = (int32_t)(g.f32_row0 + (int64_t)t0 * TILE_N);
+                    u.pad1 = (int32_t)(s << 8) | std::min(TILE_M, views[s].rows - rb * TILE_M);
+                    units.push_back(u);
+                }
+    }
     std::stable_sort(units.begin(), units.end(), [](const MatchUnit& a, const MatchUnit& b) { return a.n_tiles > b.n_tiles; });
 }
 
@@ -916,6 +919,81 @@ int cvg_match_knn2_raw(cvg_ctx* c, const float* query, int n_query, const float*
 
 }  // extern "C"
 
+// BFMatcher(NORM_L2, crossCheck = true).match of every view slot's query rows against every segment of a prepared train
+// set, on the device: the plan, the key arrays, the tensor-core instance (want_tc) and the exact SIMT kernel — both gated on
+// the path word d_flags[2], which the caller has set — and the finish into idx / dist, or, with accept, into the knn2
+// layout the fused path compacts (XcFinish).  staged: the small host -> device copies go through the engine's page-locked
+// staging (the fused path), else they are plain copies.
+static int enqueue_cross_check(cvg_ctx* c, const QuerySide& q, const std::vector<SegDev>& views, const TrainSet& ts, bool want_tc,
+                               bool staged, int32_t* idx, float* dist, uint8_t* accept)
+{
+    const int nq = q.row_end - q.row_begin, S = ts.n_segs, V = (int)views.size();
+    XcOut xo;
+    xo.row_stride = q.row_end;
+    xo.t_base = S > 0 ? ts.segs[0].f32_row0 : 0;
+    xo.t_total = S > 0 ? ts.segs[(size_t)S - 1].f32_row0 + ts.segs[(size_t)S - 1].rows - xo.t_base : 0;
+    const int64_t n_rows_all = (int64_t)S * nq, n_cols_all = (int64_t)V * xo.t_total;
+    // the guard lists and their counters are 32-bit (include/cvgraft.h: CVG_MATCH_CROSS_CHECK)
+    if (n_rows_all + n_cols_all > INT32_MAX)
+        return set_err(CVG_ERR_LIMIT, "cross-check: %lld scene x query rows + %lld view x train rows exceed 2^31 - 1",
+                       (long long)n_rows_all, (long long)n_cols_all);
+    std::vector<MatchUnit> units;
+    build_xc_plan(views, ts, c->n_sms, units);
+    const int n_units = (int)units.size();
+    int max_view_rows = 0, max_seg_rows = 0;
+    for (const SegDev& v : views) max_view_rows = std::max(max_view_rows, v.rows);
+    for (const SegInfo& g : ts.segs) max_seg_rows = std::max(max_seg_rows, g.rows);
+    const size_t n_keys = (size_t)S * xo.row_stride + (size_t)n_cols_all;
+    CU_CHECK(c->units.ensure(std::max<size_t>(units.size(), 1) * sizeof(MatchUnit) + 16));
+    CU_CHECK(c->xc.ensure(64 + n_keys * 8));                                                   // XcOut, row keys, column keys
+    CU_CHECK(c->segdev.ensure((size_t)(V + S) * sizeof(SegDev) + 16));
+    CU_CHECK(c->fb.ensure((size_t)(n_rows_all + n_cols_all) * (sizeof(int2) + 16)));         // guard lists + their key pairs
+    xo.rowkey = reinterpret_cast<unsigned long long*>(c->xc.as<uint8_t>() + 64);
+    xo.colkey = xo.rowkey + (size_t)S * xo.row_stride;
+    std::vector<SegDev> sd(views);                                                             // views, then segments
+    for (const SegInfo& g : ts.segs) sd.push_back(SegDev{ g.f32_row0, g.rows, 0 });
+    auto h2d = [&](void* dst, const void* src, size_t bytes) {
+        return staged ? h2d_small(c, dst, src, bytes) : cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, c->stream);
+    };
+    CU_CHECK(h2d(c->xc.p, &xo, sizeof xo));
+    CU_CHECK(h2d(c->segdev.p, sd.data(), sd.size() * sizeof(SegDev)));
+    if (n_units > 0) CU_CHECK(h2d(c->units.p, units.data(), units.size() * sizeof(MatchUnit)));
+    if (staged && c->stage_fallback) CU_CHECK(cudaStreamSynchronize(c->stream));    // memcpy fallback: host sources go out of scope
+    CU_CHECK(cudaMemsetAsync(xo.rowkey, 0xFF, n_keys * 8, c->stream));
+    CU_CHECK(cudaMemsetAsync(c->d_flags + 20, 0, 8, c->stream));
+    TcOperands op{ q.d_b, q.d_aug, q.d_norm, q.n_pad, ts.d_b, ts.d_aug, (int)ts.rows_pad_total, q.d_blo, ts.d_blo };
+    TcMapsOpaque maps;
+    char err[256];
+    if (n_units > 0 && want_tc && tc_encode_maps(op, 1, &maps, err, sizeof err)) return set_err(CVG_ERR_CUDA, "%s", err);
+    const MatchUnit* d_units = c->units.as<MatchUnit>();
+    if (c->timing) cudaEventRecord(c->ev[3], c->stream);
+    if (n_units > 0) {
+        if (want_tc) {
+            if (launch_match_tc(op, &maps, d_units, n_units, c->xc.p, 1, c->d_flags + 2, 0, c->d_flags + 8, c->n_sms, c->stream, err, sizeof err))
+                return set_err(CVG_ERR_CUDA, "%s", err);
+            c->launches++;
+        }
+        launch_match_exact_xc(q.d_f32, ts.d_f32, d_units, n_units, xo, c->d_flags + 2, c->stream);
+        c->launches++;
+    }
+    if (c->timing) cudaEventRecord(c->ev[4], c->stream);
+    int2* lists = c->fb.as<int2>();
+    XcFinish w;
+    w.keys = xo; w.row_begin = q.row_begin; w.row_end = q.row_end;
+    w.n_segs = S; w.n_views = V; w.max_view_rows = max_view_rows; w.max_seg_rows = max_seg_rows;
+    w.views = c->segdev.as<SegDev>(); w.segs = c->segdev.as<SegDev>() + V;
+    w.Q = q.d_f32; w.T = ts.d_f32;
+    w.guard_counts = c->d_flags + 20; w.guard_total = c->d_flags + 7;
+    w.row_list = lists; w.col_list = lists + n_rows_all;
+    w.row_g = reinterpret_cast<unsigned long long*>(lists + n_rows_all + n_cols_all); w.col_g = w.row_g + 2 * n_rows_all;
+    w.gate_flag = c->d_flags + 2;
+    w.idx = idx; w.dist = dist; w.accept = accept;
+    w.n_sms = c->n_sms;
+    c->launches += launch_xc_finish(w, c->stream);
+    CU_CHECK(cudaGetLastError());
+    return CVG_OK;
+}
+
 // BFMatcher(NORM_L2, crossCheck = true).match of every view slot's query rows against a host train matrix; results to host.
 // The tensor-core instance (integer rows) and the exact SIMT kernel are both enqueued and gate themselves on the path word.
 static int match_cross_check(cvg_ctx* c, const QuerySide& q, const std::vector<SegDev>& views, int q_nonint, const float* train,
@@ -937,60 +1015,11 @@ static int match_cross_check(cvg_ctx* c, const QuerySide& q, const std::vector<S
     CU_CHECK(cudaMemcpyAsync(c->d_flags + 1, &q_nonint, 4, cudaMemcpyHostToDevice, c->stream));
     combine_flags_kernel<<<1, 1, 0, c->stream>>>(c->d_flags, c->d_flags, (c->flags & CVG_FORCE_EXACT_MATCH) ? 4 : 0);
     c->launches++;
-    std::vector<MatchUnit> units;
-    build_xc_plan(views, ts, c->n_sms, units);
-    const int V = (int)views.size(), n_units = (int)units.size();
-    int max_view_rows = 0;
-    for (const SegDev& v : views) max_view_rows = std::max(max_view_rows, v.rows);
-    const size_t n_cols_all = (size_t)V * n_train;
-    CU_CHECK(c->units.ensure(std::max<size_t>(units.size(), 1) * sizeof(MatchUnit)));
-    CU_CHECK(c->xc.ensure(64 + ((size_t)q.row_end + n_cols_all) * 8));            // XcOut, row keys (absolute rows), column keys
-    CU_CHECK(c->segdev.ensure((size_t)(V + 1) * sizeof(SegDev)));
-    CU_CHECK(c->fb.ensure(((size_t)nq + n_cols_all) * (sizeof(int2) + 16)));      // guard lists + their key pairs
     CU_CHECK(c->idx.ensure((size_t)nq * 4)); CU_CHECK(c->dist.ensure((size_t)nq * 4));
-    XcOut xo;
-    xo.rowkey = reinterpret_cast<unsigned long long*>(c->xc.as<uint8_t>() + 64);
-    xo.colkey = xo.rowkey + q.row_end;
-    std::vector<SegDev> sd(views);
-    sd.push_back(SegDev{ 0, n_train, 0 });
-    CU_CHECK(cudaMemcpyAsync(c->xc.p, &xo, sizeof xo, cudaMemcpyHostToDevice, c->stream));
-    CU_CHECK(cudaMemcpyAsync(c->segdev.p, sd.data(), sd.size() * sizeof(SegDev), cudaMemcpyHostToDevice, c->stream));
-    if (n_units > 0)
-        CU_CHECK(cudaMemcpyAsync(c->units.p, units.data(), units.size() * sizeof(MatchUnit), cudaMemcpyHostToDevice, c->stream));
-    CU_CHECK(cudaMemsetAsync(xo.rowkey, 0xFF, ((size_t)q.row_end + n_cols_all) * 8, c->stream));
-    CU_CHECK(cudaMemsetAsync(c->d_flags + 20, 0, 8, c->stream));
     // the candidate path (non-integer rows, tensor cores) has no cross-check form: those calls take the SIMT kernel
     const bool want_tc = path_from_kinds(c->flags, q_nonint, -1) == 0;
-    TcOperands op{ q.d_b, q.d_aug, q.d_norm, q.n_pad, ts.d_b, ts.d_aug, (int)ts.rows_pad_total, q.d_blo, ts.d_blo };
-    TcMapsOpaque maps;
-    char err[256];
-    if (n_units > 0 && want_tc && tc_encode_maps(op, 1, &maps, err, sizeof err)) return set_err(CVG_ERR_CUDA, "%s", err);
-    const MatchUnit* d_units = c->units.as<MatchUnit>();
-    if (c->timing) cudaEventRecord(c->ev[3], c->stream);
-    if (n_units > 0) {
-        if (want_tc) {
-            if (launch_match_tc(op, &maps, d_units, n_units, c->xc.p, 1, c->d_flags + 2, 0, c->d_flags + 8, c->n_sms, c->stream, err, sizeof err))
-                return set_err(CVG_ERR_CUDA, "%s", err);
-            c->launches++;
-        }
-        launch_match_exact_xc(q.d_f32, ts.d_f32, d_units, n_units, xo, c->d_flags + 2, c->stream);
-        c->launches++;
-    }
-    if (c->timing) cudaEventRecord(c->ev[4], c->stream);
-    int2* lists = c->fb.as<int2>();
-    XcFinish w;
-    w.keys = xo; w.row_begin = q.row_begin; w.row_end = q.row_end;
-    w.n_views = V; w.n_train = n_train; w.max_view_rows = max_view_rows;
-    w.views = c->segdev.as<SegDev>(); w.train_seg = c->segdev.as<SegDev>() + V;
-    w.Q = q.d_f32; w.T = ts.d_f32;
-    w.guard_counts = c->d_flags + 20; w.guard_total = c->d_flags + 7;
-    w.row_list = lists; w.col_list = lists + nq;
-    w.row_g = reinterpret_cast<unsigned long long*>(lists + nq + n_cols_all); w.col_g = w.row_g + 2 * (size_t)nq;
-    w.gate_flag = c->d_flags + 2;
-    w.idx = c->idx.as<int32_t>(); w.dist = c->dist.as<float>();
-    w.n_sms = c->n_sms;
-    c->launches += launch_xc_finish(w, c->stream);
-    CU_CHECK(cudaGetLastError());
+    rc = enqueue_cross_check(c, q, views, ts, want_tc, false, c->idx.as<int32_t>(), c->dist.as<float>(), nullptr);
+    if (rc) return rc;
     int flag = 0;
     CU_CHECK(cudaMemcpyAsync(idx, c->idx.p, (size_t)nq * 4, cudaMemcpyDeviceToHost, c->stream));
     CU_CHECK(cudaMemcpyAsync(dist, c->dist.p, (size_t)nq * 4, cudaMemcpyDeviceToHost, c->stream));
@@ -1195,26 +1224,31 @@ static int detect_common(cvg_ctx* c, const cvg_models* m, cvg_scenes* cache, Tra
     const int P = S * V;
     if (P == 0) return CVG_OK;
     QuerySide q{ m->d_f32, m->d_b, m->d_blo, m->d_aug, m->d_norm, 0, nq, m->n_pad };
+    // CVG_MATCH_CROSS_CHECK: BFMatcher(crossCheck = true).match instead of knnMatch(k = 2) + ratio test.  Its plan is built
+    // per call (enqueue_cross_check) and never enters the cached knn2 plan below.
+    const bool xc = (p->method & CVG_MATCH_CROSS_CHECK) != 0;
     int n_units = 0, n_rb = 0;
-    const MatchUnit* d_units; const MergeEntry* d_dir;
+    const MatchUnit* d_units = nullptr; const MergeEntry* d_dir = nullptr;
     // The match plan depends only on the model set and on the row counts of the scenes: a streaming caller whose
     // batches have the same shape (same number of descriptors per scene) reuses the plan already on the device.
-    std::vector<int> shape((size_t)S);
-    for (int i = 0; i < S; i++) shape[(size_t)i] = ts.segs[(size_t)i].rows;
-    if (c->plan_models_uid == m->uid && c->plan_shape == shape && c->plan_units_n > 0) {
-        n_units = c->plan_units_n; n_rb = (nq + TILE_M - 1) / TILE_M;
-        d_units = c->plan_units.as<MatchUnit>(); d_dir = c->plan_dir.as<MergeEntry>();
-    } else {
-        std::vector<MatchUnit> units; std::vector<MergeEntry> dir;
-        build_plan(q, ts, c->n_sms, units, dir, n_rb);
-        CU_CHECK(c->plan_units.ensure(std::max<size_t>(units.size(), 1) * sizeof(MatchUnit) + 16));
-        CU_CHECK(c->plan_dir.ensure(std::max<size_t>(dir.size(), 1) * sizeof(MergeEntry) + 16));
-        if (!units.empty()) CU_CHECK(h2d_small(c, c->plan_units.p, units.data(), units.size() * sizeof(MatchUnit)));
-        if (!dir.empty()) CU_CHECK(h2d_small(c, c->plan_dir.p, dir.data(), dir.size() * sizeof(MergeEntry)));
-        if (c->stage_fallback) CU_CHECK(cudaStreamSynchronize(c->stream));    // memcpy fallback: host vectors go out of scope
-        n_units = (int)units.size();
-        d_units = c->plan_units.as<MatchUnit>(); d_dir = c->plan_dir.as<MergeEntry>();
-        c->plan_models_uid = m->uid; c->plan_shape = shape; c->plan_units_n = n_units;
+    if (!xc) {
+        std::vector<int> shape((size_t)S);
+        for (int i = 0; i < S; i++) shape[(size_t)i] = ts.segs[(size_t)i].rows;
+        if (c->plan_models_uid == m->uid && c->plan_shape == shape && c->plan_units_n > 0) {
+            n_units = c->plan_units_n; n_rb = (nq + TILE_M - 1) / TILE_M;
+            d_units = c->plan_units.as<MatchUnit>(); d_dir = c->plan_dir.as<MergeEntry>();
+        } else {
+            std::vector<MatchUnit> units; std::vector<MergeEntry> dir;
+            build_plan(q, ts, c->n_sms, units, dir, n_rb);
+            CU_CHECK(c->plan_units.ensure(std::max<size_t>(units.size(), 1) * sizeof(MatchUnit) + 16));
+            CU_CHECK(c->plan_dir.ensure(std::max<size_t>(dir.size(), 1) * sizeof(MergeEntry) + 16));
+            if (!units.empty()) CU_CHECK(h2d_small(c, c->plan_units.p, units.data(), units.size() * sizeof(MatchUnit)));
+            if (!dir.empty()) CU_CHECK(h2d_small(c, c->plan_dir.p, dir.data(), dir.size() * sizeof(MergeEntry)));
+            if (c->stage_fallback) CU_CHECK(cudaStreamSynchronize(c->stream));    // memcpy fallback: host vectors go out of scope
+            n_units = (int)units.size();
+            d_units = c->plan_units.as<MatchUnit>(); d_dir = c->plan_dir.as<MergeEntry>();
+            c->plan_models_uid = m->uid; c->plan_shape = shape; c->plan_units_n = n_units;
+        }
     }
     const size_t rows = (size_t)S * std::max(nq, 1);
     CU_CHECK(c->parts.ensure(std::max<size_t>(n_units, 1) * TILE_M * sizeof(Top2)));
@@ -1232,12 +1266,24 @@ static int detect_common(cvg_ctx* c, const cvg_models* m, cvg_scenes* cache, Tra
     const int did = det_id.fetch_add(1);
     cvg_trace_mark(c->stream, "det_begin", did);
     const int path = path_from_kinds(c->flags, m->nonint, ts.nonint);
-    if (path == 0) {
-        combine_flags_kernel<<<1, 1, 0, c->stream>>>(c->d_flags, (cache && cache->d_flag) ? cache->d_flag : c->d_flags, m->nonint, 1);
+    int rc;
+    if (xc) {
+        // the path word from the row kinds of both sides, as cvg_match_cross_check sets it: 0 = tensor cores (integer rows),
+        // anything else (non-integer rows, CVG_FORCE_EXACT_MATCH) = the exact SIMT kernel
+        combine_flags_kernel<<<1, 1, 0, c->stream>>>(c->d_flags, (cache && cache->d_flag) ? cache->d_flag : c->d_flags,
+                                                     m->nonint | ((c->flags & CVG_FORCE_EXACT_MATCH) ? 4 : 0), 1);
         c->launches++;
-    }
-    int rc = launch_match(c, q, ts, d_units, n_units, d_dir, n_rb, p->ratio, path, c->parts.as<Top2>(),
+        std::vector<SegDev> views((size_t)V);
+        for (int v = 0; v < V; v++) views[(size_t)v] = SegDev{ m->view_offsets[v], m->view_offsets[v + 1] - m->view_offsets[v], 0 };
+        rc = enqueue_cross_check(c, q, views, ts, path == 0 || path == 1, true, c->idx.as<int32_t>(), nullptr, c->accept.as<uint8_t>());
+    } else {
+        if (path == 0) {
+            combine_flags_kernel<<<1, 1, 0, c->stream>>>(c->d_flags, (cache && cache->d_flag) ? cache->d_flag : c->d_flags, m->nonint, 1);
+            c->launches++;
+        }
+        rc = launch_match(c, q, ts, d_units, n_units, d_dir, n_rb, p->ratio, path, c->parts.as<Top2>(),
                           c->idx.as<int32_t>(), c->dist.as<float>(), c->accept.as<uint8_t>(), guard);
+    }
     if (rc) return rc;
     CompactWork cw;
     cw.n_segments = S; cw.n_views = V; cw.n_query = nq; cw.view_offsets = m->d_view_offsets;
@@ -1251,7 +1297,8 @@ static int detect_common(cvg_ctx* c, const cvg_models* m, cvg_scenes* cache, Tra
     int max_view = 0;
     for (int v = 0; v < V; v++) max_view = std::max(max_view, m->view_offsets[v + 1] - m->view_offsets[v]);
     // the verify stage of p->method: RANSAC modelPoints 4 (findHomography), 3 (estimateAffine2D), 2 (estimateAffinePartial2D)
-    const int mp = p->method == CVG_VERIFY_AFFINE ? 3 : (p->method == CVG_VERIFY_AFFINE_PARTIAL ? 2 : 4);
+    const int vm = p->method & CVG_VERIFY_METHOD_MASK;
+    const int mp = vm == CVG_VERIFY_AFFINE ? 3 : (vm == CVG_VERIFY_AFFINE_PARTIAL ? 2 : 4);
     int flag = 0;
     for (int attempt = 0;; attempt++) {
         if (mp == 4) {
@@ -1296,7 +1343,7 @@ static int detect_common(cvg_ctx* c, const cvg_models* m, cvg_scenes* cache, Tra
             CU_CHECK(cudaMemcpyAsync(c->inl_h.p, c->inl_xy.p, rows * 8, cudaMemcpyDeviceToHost, c->stream));
         }
         CU_CHECK(cudaMemcpyAsync(&words_h[0], c->d_flags + 4, 4, cudaMemcpyDeviceToHost, c->stream));
-        if (path == 0) CU_CHECK(cudaMemcpyAsync(&words_h[1], c->d_flags + 2, 4, cudaMemcpyDeviceToHost, c->stream));
+        if (path == 0 || xc) CU_CHECK(cudaMemcpyAsync(&words_h[1], c->d_flags + 2, 4, cudaMemcpyDeviceToHost, c->stream));
         rc = sync_and_check(c);
         if (rc) return rc;
         memcpy(per_pair, c->res_h.p, res_bytes);
@@ -1314,7 +1361,7 @@ static int detect_common(cvg_ctx* c, const cvg_models* m, cvg_scenes* cache, Tra
         rc = ensure_rng(c, p->ransac.max_iters, c->rng_len * 4);   // more draws, then the verify stage again
         if (rc) return rc;
     }
-    c->last_match_path = path == 0 ? path_from_device_word(flag) : path;
+    c->last_match_path = xc ? (flag == 0 ? 1 : 2) : (path == 0 ? path_from_device_word(flag) : path);
     if (c->timing) {
         c->t_hyp = 0; c->t_score = 0;
         for (int r = 0; r < c->hyp_rounds; r++) {
@@ -1341,9 +1388,10 @@ int check_detect_params(const cvg_detect_params* p, cvg_detect_params* out)
     cvg_detect_params_default(&q);
     memcpy(&q, p, p->size);
     q.size = sizeof q;
-    if (q.method < CVG_VERIFY_HOMOGRAPHY || q.method > CVG_VERIFY_AFFINE_PARTIAL)
-        return set_err(CVG_ERR_INVALID, "cvg_detect_params: unknown method %d", q.method);
-    if (q.method != CVG_VERIFY_HOMOGRAPHY) {
+    const int vm = q.method & CVG_VERIFY_METHOD_MASK;
+    if ((q.method & ~(CVG_VERIFY_METHOD_MASK | CVG_MATCH_CROSS_CHECK)) || vm > CVG_VERIFY_AFFINE_PARTIAL)
+        return set_err(CVG_ERR_INVALID, "cvg_detect_params: unknown method 0x%x", (unsigned)q.method);
+    if (vm != CVG_VERIFY_HOMOGRAPHY) {
         if (q.ransac.flags & ~CVG_RANSAC_NO_EARLY_STOP)
             return set_err(CVG_ERR_INVALID, "cvg_detect_params: flags 0x%x with an affine method", q.ransac.flags);
         if (q.refine_iters < 0 || q.refine_iters > 1000) return set_err(CVG_ERR_LIMIT, "refine_iters out of range [0, 1000]");

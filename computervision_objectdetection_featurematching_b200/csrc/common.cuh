@@ -21,7 +21,7 @@ struct MatchUnit {
     int32_t t_row0;          // first train row in the concatenated, padded train matrix
     int32_t n_tiles;         // number of TILE_N-wide train tiles
     int32_t t_local0;        // index of t_row0 inside its segment (train index reported = local)
-    int32_t part_slot;       // partial record block: parts[part_slot * TILE_M + row]
+    int32_t part_slot;       // partial record block: parts[part_slot * TILE_M + row].  Cross-check plan: the segment index
     int32_t seg_cols;        // valid train rows of the segment (for masking the padded tail)
     int32_t t_row0_f32;      // first train row in the unpadded fp32 train matrix (exact kernel)
     int32_t pad1;            // knn2 plan: 0.  Cross-check plan: view slot << 8 | query rows of the unit in its view (1..128)
@@ -67,27 +67,37 @@ void launch_match_exact(const float* Q, int n_query, const float* T, const Match
                         Top2* parts, const int* gate_flag /*device flag: run only if *flag == gate_want, or NULL*/,
                         int gate_want, cudaStream_t st);
 
-// Cross-check (BFMatcher(NORM_L2, crossCheck = true)): the match kernels leave, per query row, the (key << 32 | train index)
-// of its nearest train row and, per (view slot, train column), the (key << 32 | absolute query row) of the column's nearest
-// query row of that view, both reduced with atomicMin (~0 = none).  key = d^2 (tensor-core kernel, integer rows) or the
-// float bits of cv2's distance (exact SIMT kernel); xc_finish turns d^2 into distance bits.
-struct XcOut { unsigned long long* rowkey; unsigned long long* colkey; };
+// Cross-check (BFMatcher(NORM_L2, crossCheck = true)): the match kernels leave, per (segment, query row), the
+// (key << 32 | train index in the segment) of the row's nearest train row of that segment and, per (view slot, train
+// column), the (key << 32 | absolute query row) of the column's nearest query row of that view, both reduced with atomicMin
+// (~0 = none).  key = d^2 (tensor-core kernel, integer rows) or the float bits of cv2's distance (exact SIMT kernel);
+// xc_finish turns d^2 into distance bits.  Layout (DESIGN.md 4.5): rowkey[seg * row_stride + absolute query row],
+// colkey[view * t_total + fp32 train row - t_base]; the segment travels in MatchUnit::part_slot.  One train matrix is
+// the case seg = 0, t_base = 0.
+struct XcOut {
+    unsigned long long* rowkey; unsigned long long* colkey;
+    int64_t row_stride;                             // rows per segment block of rowkey
+    int64_t t_total;                                // train rows of the call (the segments' rows, contiguous from t_base)
+    int64_t t_base;                                 // fp32 row of the call's first train row
+};
 void launch_match_exact_xc(const float* Q, const float* T, const MatchUnit* units, int n_units, XcOut out,
                            const int* gate_flag /*skipped if *flag == 0 (the tensor-core kernel serves the call), or NULL*/,
                            cudaStream_t st);
 struct XcFinish {
     XcOut keys;
-    int row_begin, row_end;                         // query rows of the call (rowkey is indexed by absolute row)
-    int n_views, n_train, max_view_rows;
+    int row_begin, row_end;                         // query rows of the call (absolute)
+    int n_segs, n_views, max_view_rows, max_seg_rows;
     const SegDev* views;                            // [n_views] query rows of each view slot (f32_row0 = first row)
-    const SegDev* train_seg;                        // [1] {0, n_train}
+    const SegDev* segs;                             // [n_segs] train rows of each segment (f32_row0 = first fp32 row)
     const float* Q; const float* T;                 // fp32 rows
     int* guard_counts;                              // [2] rows / columns redone by the d >= 2048 guard (zeroed by the caller)
     int* guard_total;                               // receives their sum
-    int2* row_list; unsigned long long* row_g;      // [nq], [2 * nq]
-    int2* col_list; unsigned long long* col_g;      // [n_views * n_train], [2 * n_views * n_train]
+    int2* row_list; unsigned long long* row_g;      // [n_segs * nq], [2 * n_segs * nq]
+    int2* col_list; unsigned long long* col_g;      // [n_views * t_total], [2 * n_views * t_total]
     const int* gate_flag;                           // the d^2 -> distance step runs only if *gate_flag == 0 (tensor-core path)
-    int32_t* idx; float* dist;                      // [nq]
+    // outputs.  accept == NULL: idx / dist [nq] of the one segment (cvg_match_cross_check).  Otherwise the knn2 layout the
+    // fused path compacts: idx[2 * (seg * nq + i)] = train index, accept[seg * nq + i] = matched (dist unused)
+    int32_t* idx; float* dist; uint8_t* accept;
     int n_sms;
 };
 // d^2 keys -> distance keys (the d >= 2048 rows and columns redone exactly), then the mutual test; returns the launch count

@@ -104,7 +104,7 @@ match_exact_xc_kernel(const float* __restrict__ Q, const float* __restrict__ T, 
         #pragma unroll
         for (int j = 0; j < DIM / 4; j++) q[j] = qp[j];
     }
-    unsigned long long* ck = out.colkey + (size_t)(u.pad1 >> 8) * u.seg_cols;
+    unsigned long long* ck = out.colkey + (u.pad1 >> 8) * out.t_total + (u.t_row0_f32 - u.t_local0 - out.t_base);
     int n_cols = u.n_tiles * TILE_N;
     if (n_cols > u.seg_cols - u.t_local0) n_cols = u.seg_cols - u.t_local0;
     if (threadIdx.x < EX_TROWS) s_col[threadIdx.x] = ~0ull;
@@ -156,7 +156,7 @@ match_exact_xc_kernel(const float* __restrict__ Q, const float* __restrict__ T, 
             if (k != ~0ull) atomicMin(&ck[u.t_local0 + c0 + threadIdx.x], k);
         }
     }
-    if (bi >= 0) atomicMin(&out.rowkey[qrow], ((unsigned long long)__float_as_uint(bd) << 32) | (unsigned int)bi);
+    if (bi >= 0) atomicMin(&out.rowkey[u.part_slot * out.row_stride + qrow], ((unsigned long long)__float_as_uint(bd) << 32) | (unsigned int)bi);
 }
 
 void launch_match_exact_xc(const float* Q, const float* T, const MatchUnit* units, int n_units, XcOut out,
@@ -462,20 +462,22 @@ constexpr uint32_t XC_GUARD_D2 = 1u << 22;                 // d = 2048: from her
 
 // Tensor-core path only: the keys hold d^2.  Below 2^22 the order by (d^2, index) is cv2's order by (sqrtf(d^2), index) — every
 // d^2 < 2^22 keeps its own float distance, and every larger d^2 has a distance >= 2048 — so the key becomes (distance bits,
-// index).  A row or column whose best d^2 reaches 2^22 is listed for the exact scan instead.
-__global__ void xc_distance_kernel(XcOut k, int row_begin, int n_rows, int64_t n_cols_all, int n_train, int* __restrict__ counts,
+// index).  A row or column whose best d^2 reaches 2^22 is listed for the exact scan instead: rows as (segment, absolute
+// row), columns as (view slot, train row - t_base).
+__global__ void xc_distance_kernel(XcOut k, int row_begin, int n_rows, int64_t n_rows_all, int64_t n_cols_all, int* __restrict__ counts,
                                    int2* __restrict__ row_list, int2* __restrict__ col_list, const int* __restrict__ gate_flag)
 {
     if (gate_flag && *gate_flag != 0) return;
-    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < (int64_t)n_rows + n_cols_all; e += (int64_t)gridDim.x * blockDim.x) {
-        const bool is_row = e < n_rows;
-        unsigned long long* p = is_row ? &k.rowkey[row_begin + e] : &k.colkey[e - n_rows];
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n_rows_all + n_cols_all; e += (int64_t)gridDim.x * blockDim.x) {
+        const bool is_row = e < n_rows_all;
+        const int seg = is_row ? (int)(e / n_rows) : 0, row = is_row ? row_begin + (int)(e % n_rows) : 0;
+        unsigned long long* p = is_row ? &k.rowkey[seg * k.row_stride + row] : &k.colkey[e - n_rows_all];
         const unsigned long long v = *p;
         if (v == XC_NONE) continue;
         const uint32_t d2 = (uint32_t)(v >> 32);
         if (d2 >= XC_GUARD_D2) {
-            if (is_row) row_list[atomicAdd(&counts[0], 1)] = make_int2(0, row_begin + (int)e);
-            else { const int64_t c = e - n_rows; col_list[atomicAdd(&counts[1], 1)] = make_int2((int)(c / n_train), (int)(c % n_train)); }
+            if (is_row) row_list[atomicAdd(&counts[0], 1)] = make_int2(seg, row);
+            else { const int64_t c = e - n_rows_all; col_list[atomicAdd(&counts[1], 1)] = make_int2((int)(c / k.t_total), (int)(c % k.t_total)); }
         } else {
             *p = ((unsigned long long)__float_as_uint(sqrtf((float)d2)) << 32) | (v & 0xFFFFFFFFull);
         }
@@ -483,72 +485,86 @@ __global__ void xc_distance_kernel(XcOut k, int row_begin, int n_rows, int64_t n
 }
 
 // the exact scans' results into the key arrays (a column's scan ran over its view's rows: local row -> absolute row)
-__global__ void xc_apply_kernel(XcOut k, int n_train, const SegDev* __restrict__ views, const int* __restrict__ counts,
+__global__ void xc_apply_kernel(XcOut k, const SegDev* __restrict__ views, const int* __restrict__ counts,
                                 const int2* __restrict__ row_list, const unsigned long long* __restrict__ row_g,
                                 const int2* __restrict__ col_list, const unsigned long long* __restrict__ col_g, int* __restrict__ guard_total)
 {
     const int nr = counts[0], nc = counts[1];
     if (blockIdx.x == 0 && threadIdx.x == 0) *guard_total = nr + nc;
     for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < nr + nc; e += gridDim.x * blockDim.x) {
-        if (e < nr) { k.rowkey[row_list[e].y] = row_g[e]; continue; }
+        if (e < nr) { k.rowkey[row_list[e].x * k.row_stride + row_list[e].y] = row_g[e]; continue; }
         const int2 vc = col_list[e - nr];
         const unsigned long long g = col_g[e - nr];
-        k.colkey[(size_t)vc.x * n_train + vc.y] =
+        k.colkey[vc.x * k.t_total + vc.y] =
             g == XC_NONE ? XC_NONE : (g & 0xFFFFFFFF00000000ull) | (unsigned int)(views[vc.x].f32_row0 + (int)(unsigned int)g);
     }
 }
 
-// row i of view slot v, nearest column j: a match iff column j's nearest row in view v is i
-__global__ void xc_emit_kernel(XcOut k, int row_begin, int n_views, int n_train, const SegDev* __restrict__ views,
-                               int32_t* __restrict__ idx, float* __restrict__ dist)
+// row i of view slot v against segment s, nearest column j: a match iff column j's nearest row in view v is i
+__global__ void xc_emit_kernel(XcOut k, int row_begin, int n_query, int n_segs, int n_views, const SegDev* __restrict__ views,
+                               const SegDev* __restrict__ segs, int32_t* __restrict__ idx, float* __restrict__ dist,
+                               uint8_t* __restrict__ accept)
 {
     const int x = blockIdx.x * blockDim.x + threadIdx.x;
-    for (int v = blockIdx.y; v < n_views; v += gridDim.y) {
+    for (int64_t pv = blockIdx.y; pv < (int64_t)n_segs * n_views; pv += gridDim.y) {
+        const int s = (int)(pv / n_views), v = (int)(pv % n_views);
         const SegDev vw = views[v];
         if (x >= vw.rows) continue;
         const int row = (int)vw.f32_row0 + x;
-        const unsigned long long rk = k.rowkey[row];
+        const unsigned long long rk = k.rowkey[s * k.row_stride + row];
         int j = -1;
         float d = 0.f;
         if (rk != XC_NONE) {
             const int c = (int)(unsigned int)rk;
-            if ((unsigned int)k.colkey[(size_t)v * n_train + c] == (unsigned int)row) { j = c; d = __uint_as_float((unsigned int)(rk >> 32)); }
+            if ((unsigned int)k.colkey[v * k.t_total + (segs[s].f32_row0 - k.t_base) + c] == (unsigned int)row) {
+                j = c; d = __uint_as_float((unsigned int)(rk >> 32));
+            }
         }
-        idx[row - row_begin] = j;
-        dist[row - row_begin] = d;
+        if (accept) {
+            const size_t o = (size_t)s * n_query + (row - row_begin);
+            idx[2 * o] = j;
+            accept[o] = j >= 0;
+        } else {
+            idx[row - row_begin] = j;
+            dist[row - row_begin] = d;
+        }
     }
 }
 
 int launch_xc_finish(const XcFinish& w, cudaStream_t st)
 {
     const int nq = w.row_end - w.row_begin;
-    const int64_t n_cols_all = (int64_t)w.n_views * w.n_train;
-    if (nq <= 0) return 0;
+    const int64_t n_rows_all = (int64_t)w.n_segs * nq, n_cols_all = (int64_t)w.n_views * w.keys.t_total;
+    if (nq <= 0 || w.n_segs <= 0) return 0;
     int launches = 0;
     if (n_cols_all > 0) {
-        const int64_t n = nq + n_cols_all;
+        const int64_t n = n_rows_all + n_cols_all;
         xc_distance_kernel<<<(unsigned)std::min<int64_t>((n + 255) / 256, (int64_t)w.n_sms * 8), 256, 0, st>>>(
-            w.keys, w.row_begin, nq, n_cols_all, w.n_train, w.guard_counts, w.row_list, w.col_list, w.gate_flag);
-        // exact scans of the listed rows (over the train rows) and columns (over their view's rows, roles swapped); empty
-        // loops when nothing is listed
-        unsigned long long* rg1 = w.row_g; unsigned long long* rg2 = w.row_g + nq;
+            w.keys, w.row_begin, nq, n_rows_all, n_cols_all, w.guard_counts, w.row_list, w.col_list, w.gate_flag);
+        // exact scans of the listed rows (over their segment's train rows) and columns (over their view's rows, roles
+        // swapped); empty loops when nothing is listed
+        unsigned long long* rg1 = w.row_g; unsigned long long* rg2 = w.row_g + n_rows_all;
         unsigned long long* cg1 = w.col_g; unsigned long long* cg2 = w.col_g + n_cols_all;
         fallback_init_kernel<<<w.n_sms, 256, 0, st>>>(&w.guard_counts[0], rg1, rg2, nullptr, 0);
         fallback_init_kernel<<<w.n_sms, 256, 0, st>>>(&w.guard_counts[1], cg1, cg2, nullptr, 0);
-        fallback_scan_kernel<<<w.n_sms * 8, FB_THREADS, 0, st>>>(&w.guard_counts[0], w.row_list, w.train_seg,
-                                                                 (w.n_train + FB_CHUNK - 1) / FB_CHUNK, w.Q, 0, w.T, rg1, rg2, 1, nullptr, 0);
+        fallback_scan_kernel<<<w.n_sms * 8, FB_THREADS, 0, st>>>(&w.guard_counts[0], w.row_list, w.segs,
+                                                                 (w.max_seg_rows + FB_CHUNK - 1) / FB_CHUNK, w.Q, 0, w.T, rg1, rg2, 1, nullptr, 0);
         fallback_scan_kernel<<<w.n_sms * 8, FB_THREADS, 0, st>>>(&w.guard_counts[1], w.col_list, w.views,
-                                                                 (w.max_view_rows + FB_CHUNK - 1) / FB_CHUNK, w.T, 0, w.Q, cg1, cg2, 1, nullptr, 0);
-        xc_apply_kernel<<<w.n_sms, 256, 0, st>>>(w.keys, w.n_train, w.views, w.guard_counts, w.row_list, rg1, w.col_list, cg1,
-                                                   w.guard_total);
+                                                                 (w.max_view_rows + FB_CHUNK - 1) / FB_CHUNK, w.T, (int)w.keys.t_base, w.Q,
+                                                                 cg1, cg2, 1, nullptr, 0);
+        xc_apply_kernel<<<w.n_sms, 256, 0, st>>>(w.keys, w.views, w.guard_counts, w.row_list, rg1, w.col_list, cg1, w.guard_total);
         launches += 6;
     }
     // rows outside every view (models whose first view starts after row 0) keep no match
-    cudaMemsetAsync(w.idx, 0xFF, (size_t)nq * 4, st);
-    cudaMemsetAsync(w.dist, 0, (size_t)nq * 4, st);
+    if (w.accept) {
+        cudaMemsetAsync(w.accept, 0, (size_t)n_rows_all, st);
+    } else {
+        cudaMemsetAsync(w.idx, 0xFF, (size_t)nq * 4, st);
+        cudaMemsetAsync(w.dist, 0, (size_t)nq * 4, st);
+    }
     if (w.max_view_rows <= 0 || w.n_views <= 0) return launches;
-    xc_emit_kernel<<<dim3((unsigned)((w.max_view_rows + 255) / 256), (unsigned)std::min(w.n_views, 65535)), 256, 0, st>>>(
-        w.keys, w.row_begin, w.n_views, w.n_train, w.views, w.idx, w.dist);
+    xc_emit_kernel<<<dim3((unsigned)((w.max_view_rows + 255) / 256), (unsigned)std::min<int64_t>((int64_t)w.n_segs * w.n_views, 65535)), 256, 0, st>>>(
+        w.keys, w.row_begin, nq, w.n_segs, w.n_views, w.views, w.segs, w.idx, w.dist, w.accept);
     return launches + 1;
 }
 

@@ -432,7 +432,7 @@ __device__ __forceinline__ void xc_col_keys32(const uint32_t* r, float qbias, ui
 
 struct TcMaps { CUtensorMap q, qaug, t, taug, qlo, tlo, th, taugh; };   // th / taugh: 128-row boxes of the train operand (pair mode)
 
-// KP = 1: cross-check keys (integer descriptors), parts_out = XcOut; units of build_xc_plan.
+// KP = 1: cross-check keys (integer descriptors), parts_out = XcOut (common.cuh: key layout); units of build_xc_plan.
 // KP = 2: exact top-2 per row (integer descriptors), partial records Top2 with distances.
 // KP = 4: four candidates per row and column part (non-integer descriptors), partial records Top4 with raw
 //         accumulator values, slot (part_slot * 4 + column part).
@@ -924,7 +924,8 @@ match_tc_kernel(const __grid_constant__ TcMaps maps, const float* __restrict__ q
                 const MatchUnit un = units[unit_of(e)];
                 const bool row_ok = row_in_tile < (un.pad1 & 255);
                 const float qbias = row_ok ? __fadd_rn(qnorm[un.q_row0 + row_in_tile], 8388608.f) : INFINITY;
-                unsigned long long* ck = xo.colkey + (size_t)(un.pad1 >> 8) * un.seg_cols;
+                // this unit's view slot and segment: column keys from the segment's first train row, row keys of the segment
+                unsigned long long* ck = xo.colkey + (un.pad1 >> 8) * xo.t_total + (un.t_row0_f32 - un.t_local0 - xo.t_base);
                 float b1 = -INFINITY;
                 int i1 = -1;
                 for (int t = 0; t < un.n_tiles; t++, tc++) {
@@ -976,7 +977,7 @@ match_tc_kernel(const __grid_constant__ TcMaps maps, const float* __restrict__ q
                     }
                     if (row_ok && i1 >= 0) {
                         const uint32_t d2 = __float_as_uint(__fsub_rn(qbias, b1)) - 0x4B000000u;
-                        atomicMin(&xo.rowkey[un.q_row0 + row_in_tile], ((unsigned long long)d2 << 32) | (uint32_t)i1);
+                        atomicMin(&xo.rowkey[un.part_slot * xo.row_stride + un.q_row0 + row_in_tile], ((unsigned long long)d2 << 32) | (uint32_t)i1);
                     }
                 }
                 asm volatile("bar.sync 1, %0;" :: "n"(32 * TC_EPI_WARPS) : "memory");

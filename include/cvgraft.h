@@ -101,6 +101,22 @@ typedef struct cvg_affine_params {
 #define CVG_VERIFY_HOMOGRAPHY     0 /* findHomography(RANSAC) (default)                                              */
 #define CVG_VERIFY_AFFINE         1 /* estimateAffine2D(RANSAC, refineIters = refine_iters)                         */
 #define CVG_VERIFY_AFFINE_PARTIAL 2 /* estimateAffinePartial2D(RANSAC, refineIters = refine_iters)                  */
+#define CVG_VERIFY_METHOD_MASK 0xFF /* method & CVG_VERIFY_METHOD_MASK is the CVG_VERIFY_* value                    */
+/* Flag in the upper bits of cvg_detect_params.method: the correspondences come from BFMatcher(NORM_L2, crossCheck = true)
+ * .match — src/TestsDetector.cpp:36,59-60 with crossCheck on — instead of knnMatch(k = 2) + the ratio test (:59-72):
+ *   - each view is its own query matrix against each scene, exactly as cvg_match_cross_check(view = v) matches it;
+ *   - the correspondences of a pair are its mutual matches in query-row order (cv2's order); n_good is their count;
+ *   - ratio is ignored;
+ *   - the verify stage of method & CVG_VERIFY_METHOD_MASK, the gates, H, det, n_inliers, ransac_iters and the inlier
+ *     gather are those of the ratio-test form, on these correspondences.
+ * Paths: integer rows (SIFT) take the tcgen05 kernel (cvg_last_match_path 1; rows and columns at d >= 2048 are redone
+ * exactly and counted by cvg_last_match_guard_rows); non-integer rows and CVG_FORCE_EXACT_MATCH take the exact fp32 SIMT
+ * kernel (path 2), which is slow.  cvg_last_timing's match_ms covers the cross-check match kernels.
+ * Limit: (scenes x model rows) + (views x scene rows) of one call — of one lane sub-batch or one GPU's share on a
+ * multi-device context — must stay below 2^31, else CVG_ERR_LIMIT.  Scratch: 32 bytes per such entry.
+ * Any other bit of method, or a verify method above CVG_VERIFY_AFFINE_PARTIAL, -> CVG_ERR_INVALID.  The 56-byte layout
+ * has no method field and always means homography + ratio test. */
+#define CVG_MATCH_CROSS_CHECK 0x100
 
 /* constants of detectObjects() — src/TestsDetector.cpp:21-25.
  * Size rule: `size` = sizeof(cvg_detect_params) is this layout.  `size` = offsetof(cvg_detect_params, method) (56) is
@@ -118,7 +134,7 @@ typedef struct cvg_detect_params {
     float det_hi;                   /* HOMOGRAPHY_DET_UPPER_THRESHOLD = 10.0f             :25        */
     int32_t reserved;
     cvg_ransac_params ransac;
-    int32_t method;                 /* CVG_VERIFY_*; default CVG_VERIFY_HOMOGRAPHY                    */
+    int32_t method;                 /* CVG_VERIFY_* [| CVG_MATCH_CROSS_CHECK]; default homography    */
     int32_t refine_iters;           /* LM iterations of the affine methods; default 10 (OpenCV's)    */
 } cvg_detect_params;
 
@@ -131,7 +147,8 @@ typedef struct cvg_detect_params {
  *   (affine), or getSubset's 10 000 attempts exhausted.  Gate order :74 -> :79 -> :81 -> :84 for every method. */
 typedef struct cvg_pair_result {
     int32_t status;                 /* CVG_PAIR_*                                                    */
-    int32_t n_good;                 /* matches that passed the ratio test                            */
+    int32_t n_good;                 /* matches that passed the ratio test (CVG_MATCH_CROSS_CHECK:     */
+                                    /* the pair's mutual matches)                                    */
     int32_t n_inliers;              /* countNonZero(inlierMask) (0 when no H)                        */
     int32_t ransac_iters;           /* RANSAC iterations the reference loop would have run           */
     double H[9];                    /* row-major 3x3, H[8] == 1 (homography: as returned); zeros when */
@@ -387,8 +404,9 @@ int  cvg_last_match_fallback_rows(const cvg_ctx* ctx);
  * neighbouring integer d^2 round to one float (u8 rows reach d = 2885; SIFT rows, norm 512, stay below 1024).
  * Rows whose second distance reaches 2048 are redone by the exact kernels, which compare rounded distances:
  * how many rows of the last path-1 call that was.  When the norms of both sides are known on the host and
- * ||q|| + ||t|| < 2047 the guard is not even enqueued.  After cvg_match_cross_check(_raw): the query rows whose nearest
- * distance, plus the train columns whose nearest distance in a view, reached 2048 and were redone exactly. */
+ * ||q|| + ||t|| < 2047 the guard is not even enqueued.  After cvg_match_cross_check(_raw), or a fused call with
+ * CVG_MATCH_CROSS_CHECK on the context's own engine: the query rows whose nearest distance, plus the train columns whose
+ * nearest distance in a view, reached 2048 and were redone exactly. */
 int  cvg_last_match_guard_rows(const cvg_ctx* ctx);
 /* Verify calls with CVG_RANSAC_NO_EARLY_STOP and max_iters >= 32768 cut every set's cv::RNG draw stream into
  * chunks walked by many CTAs (same samples as the serial walk).  Returns how many sets of the last such call
